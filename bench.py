@@ -23,6 +23,10 @@ c4s web-scale-shaped pg k=64 (1/10 scale in users, items and non-zeros), c5s bat
 
 --impl reference times only the reference's CPU implementation on the same arrays, sweeps 1..K of one fit
 (rank 0; other ranks exit).
+
+--dump-outputs DIR writes what the timed path returned after its last step (A and B after sweep K; for c5s the
+ranked ids and scores) as DIR/<name>.npy, so that two builds can be compared output for output on the same
+seeded inputs.  Outputs larger than DUMP_BYTES in all are cut to the same seeded sample of rows on every run.
 """
 from __future__ import annotations
 
@@ -65,6 +69,21 @@ CONFIGS = {
 }
 TOPN = dict(users=32_768, items=1_000_000, k=64, top_n=100, excl=200,
             label="batched topN: 32k users x 1M items, k=64, top-100, ~200 excluded items per user")
+
+
+DUMP_BYTES = 60 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> float32/float64 array.  Every array keeps the same fraction of its rows (sorted, drawn with
+    a fixed seed) so that together they fit in DUMP_BYTES."""
+    os.makedirs(out_dir, exist_ok=True)
+    frac = min(1.0, DUMP_BYTES / sum(a.nbytes for a in arrays.values()))
+    for name, a in arrays.items():
+        if frac < 1.0:
+            rows = np.random.default_rng(0).choice(a.shape[0], int(a.shape[0] * frac), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def make_problem(cfg, dtype=np.float32):
@@ -143,7 +162,7 @@ class ClockSampler:
 def run_reference(cfg, problem, sweeps, warmup_sweeps=0):
     """The reference's own CPU path (oracle/_ref, -O3 OpenMP build of /root/reference/src) on the SAME arrays
     as the device arm: sweeps 1..`sweeps` of ONE fit from the initial factors (what the device arm times).
-    Returns (ms per sweep, info)."""
+    Returns (ms per sweep, info, (A, B) after the last sweep)."""
     from oracle.oracle import Ref, Restatement
     csr, csc, A0, B0 = problem
     nnz = int(csr[0].shape[0])
@@ -165,7 +184,7 @@ def run_reference(cfg, problem, sweeps, warmup_sweeps=0):
     info = {"value": nnz / (ms / 1e3), "unit": "nnz/s per sweep", "cores": cores, "kind": kind, "same_config": True,
             "sample": f"the full workload ({cfg['label']}: {nnz} stored nnz), sweeps 1..{sweeps} of one fit from the "
                       f"initial factors ({build})"}
-    return ms, info
+    return ms, info, (A, B)
 
 
 def topn_problem():
@@ -232,15 +251,21 @@ def bench_topn(args, rank, world, local_rank):
     else:
         fit = be.fit
 
+    last = []
+
     def one_resident():
         t0 = time.perf_counter()
-        fit.topN(users=users, excl_ptr=lptr, excl_ix=leix, top_n=t["top_n"], output_score=True)
+        last[:] = fit.topN(users=users, excl_ptr=lptr, excl_ix=leix, top_n=t["top_n"], output_score=True)
         return time.perf_counter() - t0
     for _ in range(max(args.warmup, 1)):
         one_resident()
     if dist is not None:
         dist.barrier()
     ms = 1e3 * float(np.mean([one_resident() for _ in range(args.steps)]))
+    if args.dump_outputs:      # this rank's users; ids are exact in float64
+        ids, scores = last
+        dump_outputs(os.path.join(args.dump_outputs, f"rank{rank}") if world > 1 else args.dump_outputs,
+                     {"topn_ids": ids.astype(np.float64), "topn_scores": scores})
     if dist is not None:
         tt = torch.tensor([ms, ms_e2e], device="cuda", dtype=torch.float64)
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -292,6 +317,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (at most 60 MiB in all: "
+                         "larger outputs as a fixed seeded sample of their rows)")
     ap.add_argument("--flags", type=int, default=0)
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "p2p-host", "nccl"],
                     help="N>1: refresh replicas by peer-memory stores from the row kernels, completion signalled on the "
@@ -321,7 +349,9 @@ def main():
         if rank != 0:
             return 0
         problem = make_problem(cfg)
-        ms, info = run_reference(cfg, problem, args.steps, warmup_sweeps=min(args.warmup, 1))
+        ms, info, (A, B) = run_reference(cfg, problem, args.steps, warmup_sweeps=min(args.warmup, 1))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"A": A, "B": B})
         line = {"impl": "reference", "metric": metric, "value": info["value"],
                 "unit": "nnz/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
                 "ms_per_step": ms, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
@@ -394,6 +424,10 @@ def main():
     barrier()
     ms_total = ev0.elapsed_time(ev1)
     launches = L.pmf_b200_kernel_launches() - launches0
+    if args.dump_outputs:
+        out = fit.get_factors() if world == 1 else be.factors(root=0)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"A": out[0], "B": out[1]})
     # second pass over the same K sweeps with per-launch CUDA events (bins run one after the
     # other on the launching stream here; in the timed pass above they overlap on side streams)
     reset()
@@ -602,7 +636,7 @@ def main():
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         try:
-            _, cpu = run_reference(cfg, problem, 3)
+            _, cpu, _ = run_reference(cfg, problem, 3)
         except Exception as e:  # the oracle is optional infrastructure for this leg
             cpu = {"value": None, "unit": "nnz/s per sweep", "cores": 0, "kind": "unavailable", "sample": str(e)}
 

@@ -2,7 +2,7 @@
 
   * `Ref(dtype, fast=False)`  : the reference's own C sources compiled by
     oracle/Makefile into oracle/_ref/ (prebuilt .so travels to the GPU box).
-  * `Restatement(dtype)`      : this repo's plain-C restatement (oracle/poismf_oracle.c).
+  * `Restatement(dtype, fast=False)` : this repo's plain-C restatement (oracle/poismf_oracle.c).
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference
 legs may import this module.  The product package (poismf_b200) never does.
@@ -134,11 +134,13 @@ class Ref(_Base):
 
 
 class Restatement(_Base):
-    """This repo's restatement of the same algorithm (oracle/poismf_oracle.c)."""
+    """This repo's restatement of the same algorithm (oracle/poismf_oracle.c); `fast=True` loads
+    it compiled with the reference's fast flags (-O3, FMA contraction)."""
 
-    def __init__(self, dtype):
+    def __init__(self, dtype, fast=False):
         _, name = _real(dtype)
-        super().__init__(os.path.join(HERE, "libpoismf_oracle_" + name + ".so"), dtype)
+        stem = "libpoismf_oraclefast_" if fast else "libpoismf_oracle_"
+        super().__init__(os.path.join(HERE, stem + name + ".so"), dtype)
 
     def run_poismf(self, A, B, csr, csc, method, l2_reg, l1_reg=0.0, w_mult=1.0, step_size=1e-7,
                    limit_step=False, numiter=1, maxupd=1, early_stop=False, reuse_prev=False,

@@ -26,6 +26,14 @@ def _built():
     yield
 
 
+def golden():
+    """Committed outputs of the reference (tests/golden/make_golden.py), stored one file per dtype."""
+    out = {}
+    for name in ("float64", "float32"):
+        out.update(np.load(os.path.join(ROOT, "tests", "golden", f"reference_outputs_{name}.npz")))
+    return out
+
+
 def has_gpu():
     try:
         from poismf_b200 import _lib

@@ -1,15 +1,13 @@
 """CPU tests of the checkers: the plain-C restatement against (a) the reference itself
 (oracle/_ref, when it has been built here) and (b) the committed golden outputs of the
 reference (always).  Bit-exact: both are compiled -O2 -ffp-contract=off with sequential BLAS."""
-import os
-
 import numpy as np
 import pytest
 
-from conftest import CASES, FM_CASES, FS_CASES, FS_ROWS, fm_hyper, fm_problem, fs_row, hyper, problem
+from conftest import CASES, FM_CASES, FS_CASES, FS_ROWS, fm_hyper, fm_problem, fs_row, golden, hyper, problem
 from oracle.oracle import Ref, Restatement
 
-GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_outputs.npz"))
+GOLD = golden()
 DTYPES = [np.float64, np.float32]
 
 
