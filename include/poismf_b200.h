@@ -205,6 +205,23 @@ int pmf_b200_topN_fitted(pmf_b200_handle* h, int index_bytes, const void* user_i
                          const void* excl_ptr, const void* excl_ix,
                          void* outp_ix, void* outp_score, size_t n_top);
 
+/* Batched top-N where user u ranks ONLY the items incl_ix[incl_ptr[u] .. incl_ptr[u+1]) (any order; duplicates are
+ * ranked as given, like src/topN.c).  Users are selected by user_ix, or rows 0..n_users-1 when NULL.  Scores are
+ * the exact sequential, unfused dots <a_u, B_j> (the bits of the reference's strict build); the ranking is
+ * descending score, ties by ascending item id.  Output [n_users x n_top] item ids and optionally scores.
+ * Returns 2, before any result is written, when n_top == 0, a user id is >= dimA, incl_ptr is not monotone,
+ * a list is longer than n or shorter than n_top, or a listed id is >= n; 1 on a CUDA failure.  No reference
+ * equivalent: the reference loops topN(include) per user. */
+int pmf_b200_topN_batch_include(int dtype, int index_bytes, const void* A, const void* B, int k,
+                                const void* user_ix, size_t n_users, size_t dimA,
+                                const void* incl_ptr, const void* incl_ix,
+                                void* outp_ix, void* outp_score, size_t n_top, size_t n);
+
+/* The same against the factors resident in a fit handle (waits like pmf_b200_topN_fitted). */
+int pmf_b200_topN_fitted_include(pmf_b200_handle* h, int index_bytes, const void* user_ix, size_t n_users,
+                                 const void* incl_ptr, const void* incl_ix,
+                                 void* outp_ix, void* outp_score, size_t n_top);
+
 /* Counters of the calling thread's topN calls: users scored by the tensor-core candidate scorer,
  * and how many of those had to be redone by the exact scorer because the TF32 error bound could
  * not prove their candidate set complete. */

@@ -26,6 +26,7 @@ SYMBOLS = [
     "pmf_b200_set_stream", "pmf_b200_sweeps", "pmf_b200_half_sweep", "pmf_b200_sync",
     "pmf_b200_set_profiling", "pmf_b200_get_profile", "pmf_b200_ipc_export", "pmf_b200_ipc_import",
     "pmf_b200_run_poismf", "pmf_b200_factors_multiple", "pmf_b200_factors_single", "pmf_b200_predict_multiple", "pmf_b200_topN", "pmf_b200_topN_batch", "pmf_b200_topN_fitted", "pmf_b200_topN_stats",
+    "pmf_b200_topN_batch_include", "pmf_b200_topN_fitted_include",
     "pmf_b200_release_cache", "pmf_b200_fit_coo", "pmf_b200_coo_to_csr_csc",
 ]
 
@@ -85,6 +86,8 @@ def lib():
     L.pmf_b200_topN.argtypes = [i, i, vp, vp, i, vp, sz, vp, sz, vp, vp, sz, sz]
     L.pmf_b200_topN_batch.argtypes = [i, i, vp, vp, i, vp, sz, sz, vp, vp, vp, vp, sz, sz]
     L.pmf_b200_topN_fitted.argtypes = [vp, i, vp, sz, vp, vp, vp, vp, sz]
+    L.pmf_b200_topN_batch_include.argtypes = [i, i, vp, vp, i, vp, sz, sz, vp, vp, vp, vp, sz, sz]
+    L.pmf_b200_topN_fitted_include.argtypes = [vp, i, vp, sz, vp, vp, vp, vp, sz]
     L.pmf_b200_topN_stats.argtypes = [C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong), i]
     L.pmf_b200_topN_stats.restype = None
     L.pmf_b200_fit_coo.argtypes = [i, i] + [vp] * 5 + [sz, sz, sz, sz, d, d, d, d, i, i, sz, sz, i, i, i]

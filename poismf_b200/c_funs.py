@@ -118,16 +118,46 @@ def _call_topN(a_vec, B, include_ix, exclude_ix, top_n=10, output_score=False, n
     return outp_ix, outp_score
 
 
-def _topN_batch(A, B, users=None, excl_ptr=None, excl_ix=None, top_n=10, output_score=False):
-    """Batched top-N for many users at once (no reference equivalent; include/poismf_b200.h)."""
+def _include_lists(incl_ptr, incl_ix, excl_ptr, excl_ix, n_users):
+    """(incl_ptr, incl_ix) as uint64 arrays, or None without include lists.  Include and exclude lists together
+    are invalid, as in the reference (src/topN.c:124-128), and so are offsets that do not cover n_users lists
+    inside incl_ix."""
+    if incl_ptr is None and incl_ix is None:
+        return None
+    if incl_ptr is None or incl_ix is None:
+        raise ValueError("topN: incl_ptr and incl_ix go together")
+    if excl_ptr is not None or excl_ix is not None:
+        raise ValueError("topN: include and exclude lists cannot be combined")
+    ptr = np.ascontiguousarray(incl_ptr, dtype=np.uint64)
+    ix = np.ascontiguousarray(incl_ix, dtype=np.uint64)
+    if ptr.ndim != 1 or ptr.shape[0] != n_users + 1 or int(ptr.max()) > ix.shape[0]:
+        raise ValueError("topN: incl_ptr must hold n_users + 1 offsets into incl_ix")
+    return ptr, ix
+
+
+def _topN_batch(A, B, users=None, excl_ptr=None, excl_ix=None, top_n=10, output_score=False, incl_ptr=None,
+                incl_ix=None):
+    """Batched top-N for many users at once (no reference equivalent; include/poismf_b200.h).  With
+    `incl_ptr` / `incl_ix` user u ranks only the items incl_ix[incl_ptr[u]:incl_ptr[u+1]]."""
     _lib.require_gpu()
     ixdt = np.uint64
     u = None if users is None else np.ascontiguousarray(users, dtype=ixdt)
     n_users = A.shape[0] if u is None else u.shape[0]
-    ep = None if excl_ptr is None else np.ascontiguousarray(excl_ptr, dtype=ixdt)
-    ei = None if excl_ix is None else np.ascontiguousarray(excl_ix, dtype=ixdt)
+    include = _include_lists(incl_ptr, incl_ix, excl_ptr, excl_ix, n_users)
     outp_ix = np.empty((n_users, top_n), dtype=ixdt)
     outp_score = np.empty((n_users, top_n) if output_score else (0, 0), dtype=B.dtype)
+    if include is not None:
+        rc = _lib.lib().pmf_b200_topN_batch_include(
+            _lib.dtype_code(B.dtype), 8, _lib.ptr(A), _lib.ptr(B), B.shape[1], _lib.ptr(u), n_users, A.shape[0],
+            _lib.ptr(include[0]), _lib.ptr(include[1]), _lib.ptr(outp_ix),
+            _lib.ptr(outp_score) if output_score else None, top_n, B.shape[0])
+        if rc == 1:
+            raise MemoryError(_lib.last_error())
+        if rc == 2:
+            raise ValueError("topN_batch: invalid arguments")
+        return outp_ix, outp_score
+    ep = None if excl_ptr is None else np.ascontiguousarray(excl_ptr, dtype=ixdt)
+    ei = None if excl_ix is None else np.ascontiguousarray(excl_ix, dtype=ixdt)
     rc = _lib.lib().pmf_b200_topN_batch(
         _lib.dtype_code(B.dtype), 8, _lib.ptr(A), _lib.ptr(B), B.shape[1], _lib.ptr(u), n_users, A.shape[0],
         _lib.ptr(ep), _lib.ptr(ei), _lib.ptr(outp_ix), _lib.ptr(outp_score) if output_score else None,

@@ -34,6 +34,7 @@
 #include "dense_rows.cuh"
 #include "launch.h"
 #include "topn_tc.cuh"
+#include "topn_include.cuh"
 
 using namespace pmf;
 
@@ -2219,6 +2220,199 @@ static int topn_batch_impl(const real* A, const real* B, int k, const IX* user_i
     return rc;
 }
 
+// Batched top-N over per-user candidate lists (topn_include.cuh).  Lists up to `cap` items are ranked in
+// shared memory, one CTA per user; longer ones go through CUB's segmented radix sort.  The path follows
+// from each list's length.
+template <class real, class IX>
+static int topn_include_impl(const real* A, const real* B, int k, const IX* user_ix, size_t n_users, size_t dimA,
+                             const IX* incl_ptr, const IX* incl_ix, IX* outp_ix, real* outp_score, size_t n_top,
+                             size_t n, const ResidentFactors* rf = nullptr)
+{
+    using K = typename incl::OrderKey<real>::T;
+    CK(cudaSetDevice(rf ? rf->device : env_device()));
+    // argument checks of src/topN.c:121-128 per user, and the existing include rule n_top <= list length;
+    // the item ids are range-checked on the device once uploaded, before any result is written
+    if (n_top == 0 || !incl_ptr || !incl_ix) return 2;
+    if (std::is_signed<IX>::value && (long long)incl_ptr[0] < 0) return 2;     // 4-byte (R) offsets are signed
+    if (!user_ix && n_users > dimA) return 2;
+    if (user_ix)
+        for (size_t u = 0; u < n_users; u++)
+            if ((size_t)user_ix[u] >= dimA) return 2;
+    for (size_t u = 0; u < n_users; u++) {
+        if (incl_ptr[u + 1] < incl_ptr[u]) return 2;
+        const size_t len = (size_t)(incl_ptr[u + 1] - incl_ptr[u]);
+        if (len > n || len < n_top) return 2;
+    }
+    if (n_users == 0) return 0;
+    if (n >= 0xffffffffull) return fail("topN_include: item ids must fit 32 bits");
+    const int V = RealTraits<real>::V, ldf = round_up(k, V);
+    const size_t pitch = (size_t)ldf * sizeof(real), rowb = incl::row_bytes(ldf, sizeof(real));
+    const size_t entry = sizeof(K) + sizeof(uint32_t);
+    if (rowb + entry > SMEM_CTA_MAX) return fail("topN_include: k = %d leaves no shared memory to rank in", k);
+    // shared-memory capacity: 16 K candidates in f32, 8 K in f64 (a power of two)
+    int cap = std::is_same<real, float>::value ? 16384 : 8192;
+    while (cap > 1 && rowb + (size_t)cap * entry > SMEM_CTA_MAX) cap >>= 1;
+    auto len_of = [&](size_t u) { return (size_t)(incl_ptr[u + 1] - incl_ptr[u]); };
+
+    // users per chunk: at most 32 768, and the chunk's lists and work arrays within a quarter of the free
+    // device memory (at most 32 GB)
+    size_t mem_free = 0, mem_total = 0;
+    CK(cudaMemGetInfo(&mem_free, &mem_total));
+    const size_t budget = std::max<size_t>((size_t)1 << 30, std::min<size_t>(mem_free / 4, (size_t)32 << 30));
+    const size_t per_user = pitch + n_top * (sizeof(IX) + sizeof(real)) + 2 * sizeof(long long) + 2 * sizeof(int);
+    const size_t per_long = 2 * entry;                      // double-buffered (id, key) of the segmented sort
+    struct Chunk { size_t u0, u1, n_long, long_total; };
+    std::vector<Chunk> chunks;
+    size_t max_m = 0, max_list = 0, max_long = 0, max_long_total = 0;
+    for (size_t u0 = 0; u0 < n_users;) {
+        Chunk c = {u0, u0, 0, 0};
+        size_t bytes = 0;
+        while (c.u1 < n_users && c.u1 - u0 < 32768) {
+            const size_t len = len_of(c.u1), lng = len > (size_t)cap ? len : 0;
+            const size_t add = per_user + len * sizeof(IX) + lng * per_long;
+            if (c.u1 > u0 && (bytes + add > budget || c.long_total + lng > (size_t)INT32_MAX)) break;
+            bytes += add; c.long_total += lng; c.n_long += lng ? 1 : 0; c.u1++;
+        }
+        max_m = std::max(max_m, c.u1 - u0);
+        max_list = std::max(max_list, (size_t)(incl_ptr[c.u1] - incl_ptr[u0]));
+        max_long = std::max(max_long, c.n_long);
+        max_long_total = std::max(max_long_total, c.long_total);
+        chunks.push_back(c);
+        u0 = c.u1;
+    }
+
+    real *dB = nullptr, *dA = nullptr, *dAsel = nullptr, *d_sc = nullptr;
+    IX *d_ix = nullptr, *d_out = nullptr;
+    long long *dusers = nullptr, *dptr = nullptr;
+    int *d_su = nullptr, *d_lu = nullptr, *d_seg = nullptr, *d_bad = nullptr;
+    uint32_t *id0 = nullptr, *id1 = nullptr;
+    K *key0 = nullptr, *key1 = nullptr;
+    void* tmp = nullptr;
+    bool B_resident = false, A_resident = false;
+    auto body = [&]() -> int {
+        if (rf) {
+            if (rf->ldf != ldf) return fail("topN_include: resident factors have another row pitch");
+            dB = (real*)rf->B; dA = (real*)rf->A;
+            B_resident = A_resident = true;
+        } else {
+            bool dummy = false;
+            if (upload_rows<real>(&dB, B, n, k, ldf, &B_resident, true)) return 1;
+            if (upload_rows<real>(&dA, A, dimA, k, ldf, &dummy, false)) return 1;
+        }
+        CK(dmalloc(&dAsel, max_m * pitch));
+        CK(dmalloc(&dusers, max_m * sizeof(long long)));
+        CK(dmalloc(&dptr, (max_m + 1) * sizeof(long long)));
+        CK(dmalloc(&d_su, max_m * sizeof(int)));
+        CK(dmalloc(&d_ix, std::max<size_t>(max_list, 1) * sizeof(IX)));
+        CK(dmalloc(&d_out, max_m * n_top * sizeof(IX)));
+        if (outp_score) CK(dmalloc(&d_sc, max_m * n_top * sizeof(real)));
+        CK(dmalloc(&d_bad, sizeof(int)));
+        int end_bit = 1;                                    // bits of the largest item id
+        while (end_bit < 32 && ((n - 1) >> end_bit)) end_bit++;
+        size_t tmp_bytes = 0;
+        if (max_long) {
+            CK(dmalloc(&d_lu, max_long * sizeof(int)));
+            CK(dmalloc(&d_seg, (max_long + 1) * sizeof(int)));
+            CK(dmalloc(&id0, max_long_total * sizeof(uint32_t))); CK(dmalloc(&id1, max_long_total * sizeof(uint32_t)));
+            CK(dmalloc(&key0, max_long_total * sizeof(K))); CK(dmalloc(&key1, max_long_total * sizeof(K)));
+            size_t t1 = 0, t2 = 0;
+            CK(cub::DeviceSegmentedRadixSort::SortPairs(nullptr, t1, id0, id1, key0, key1, (int)max_long_total,
+                                                        (int)max_long, d_seg, d_seg + 1, 0, end_bit));
+            CK(cub::DeviceSegmentedRadixSort::SortPairsDescending(nullptr, t2, key1, key0, id1, id0,
+                                                                  (int)max_long_total, (int)max_long, d_seg, d_seg + 1));
+            tmp_bytes = std::max(t1, t2);
+            CK(dmalloc(&tmp, std::max<size_t>(tmp_bytes, 1)));
+        }
+        // -> 0 ok, 2 a listed id outside [0, n), 1 CUDA error
+        auto upload_lists = [&](const Chunk& c, bool check) -> int {
+            const size_t off = (size_t)incl_ptr[c.u0], cnt = (size_t)incl_ptr[c.u1] - off;
+            CK(Stager::get().h2d(d_ix, incl_ix + off, cnt * sizeof(IX), 0));
+            if (!check) return 0;
+            int bad = 0;
+            CK(cudaMemsetAsync(d_bad, 0, sizeof(int)));
+            tc::any_id_out_of_range_kernel<IX><<<592, 256>>>(d_ix, cnt, n, d_bad);
+            LAUNCHED();
+            CK(cudaMemcpy(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost));
+            return bad ? 2 : 0;
+        };
+        // with several chunks every list is checked before the first result is written, and uploaded again
+        if (chunks.size() > 1)
+            for (const Chunk& c : chunks)
+                if (const int bad = upload_lists(c, true)) return bad;
+        std::vector<long long> hu, hp;
+        std::vector<int> hsu, hlu, hseg;
+        std::vector<std::pair<int, int>> classes;           // (capacity, users) of the path (a) launches
+        for (const Chunk& c : chunks) {
+            const size_t m = c.u1 - c.u0, off = (size_t)incl_ptr[c.u0];
+            if (const int bad = upload_lists(c, chunks.size() == 1)) return bad;
+            hu.resize(m); hp.resize(m + 1); hsu.clear(); classes.clear(); hlu.clear(); hseg.assign(1, 0);
+            for (size_t i = 0; i < m; i++) {
+                const size_t u = c.u0 + i, len = len_of(u);
+                hu[i] = user_ix ? (long long)user_ix[u] : (long long)u;
+                hp[i] = (long long)((size_t)incl_ptr[u] - off);
+                if (len > (size_t)cap) { hlu.push_back((int)i); hseg.push_back(hseg.back() + (int)len); }
+            }
+            // path (a) by length class, so that one long list does not size every CTA's shared memory: lists up
+            // to 4 K items share one launch (its 4 CTAs per SM, the register bound, fit in shared memory), longer
+            // ones go by power of two up to `cap`
+            for (size_t lo = 0, P = (size_t)std::min(cap, 4096);; lo = P, P <<= 1) {
+                const size_t start = hsu.size();
+                for (size_t i = 0; i < m; i++) {
+                    const size_t len = len_of(c.u0 + i);
+                    if (len > lo && len <= P) hsu.push_back((int)i);
+                }
+                if (hsu.size() > start) classes.push_back({(int)P, (int)(hsu.size() - start)});
+                if (P >= (size_t)cap) break;
+            }
+            hp[m] = (long long)((size_t)incl_ptr[c.u1] - off);
+            CK(cudaMemcpy(dusers, hu.data(), m * sizeof(long long), cudaMemcpyHostToDevice));
+            CK(cudaMemcpy(dptr, hp.data(), (m + 1) * sizeof(long long), cudaMemcpyHostToDevice));
+            gather_rows_kernel<real><<<(int)std::min<size_t>((m * ldf + 255) / 256, 4096), 256>>>(dA, dusers, (int)m, ldf, dAsel);
+            LAUNCHED();
+            if (!hsu.empty()) CK(cudaMemcpy(d_su, hsu.data(), hsu.size() * sizeof(int), cudaMemcpyHostToDevice));
+            for (size_t q = 0, first = 0; q < classes.size(); first += classes[q].second, q++) {
+                const size_t smem = rowb + (size_t)classes[q].first * entry;
+                CK(cudaFuncSetAttribute(incl::include_select_smem_kernel<real, IX>,
+                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                incl::include_select_smem_kernel<real, IX><<<(unsigned)classes[q].second, incl::SMEM_THREADS, smem>>>(
+                    dAsel, dB, k, ldf, dptr, d_ix, d_su + first, classes[q].first, (int)n_top, d_out, d_sc);
+                LAUNCHED();
+            }
+            if (!hlu.empty()) {
+                const int nl = (int)hlu.size(), total = hseg.back();
+                CK(cudaMemcpy(d_lu, hlu.data(), nl * sizeof(int), cudaMemcpyHostToDevice));
+                CK(cudaMemcpy(d_seg, hseg.data(), (nl + 1) * sizeof(int), cudaMemcpyHostToDevice));
+                CK(cudaFuncSetAttribute(incl::include_score_long_kernel<real, IX>,
+                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rowb));
+                incl::include_score_long_kernel<real, IX><<<dim3(64, (unsigned)nl), 256, rowb>>>(
+                    dAsel, dB, k, ldf, dptr, d_ix, d_lu, d_seg, id0, key0);
+                LAUNCHED();
+                // by item id, then stably by score: ties come out by ascending id
+                CK(cub::DeviceSegmentedRadixSort::SortPairs(tmp, tmp_bytes, id0, id1, key0, key1, total, nl,
+                                                            d_seg, d_seg + 1, 0, end_bit));
+                CK(cub::DeviceSegmentedRadixSort::SortPairsDescending(tmp, tmp_bytes, key1, key0, id1, id0, total, nl,
+                                                                      d_seg, d_seg + 1));
+                LAUNCHED(); LAUNCHED();
+                incl::include_emit_long_kernel<real, IX><<<(unsigned)nl, 128>>>(d_lu, d_seg, id0, key0, (int)n_top,
+                                                                                 d_out, d_sc);
+                LAUNCHED();
+            }
+            CK(cudaGetLastError());
+            CK(Stager::get().d2h(outp_ix + c.u0 * n_top, d_out, m * n_top * sizeof(IX), 0));
+            if (outp_score) CK(Stager::get().d2h(outp_score + c.u0 * n_top, d_sc, m * n_top * sizeof(real), 0));
+            CK(cudaStreamSynchronize(0));
+        }
+        return 0;
+    };
+    int rc = body();
+    if (rc) cudaDeviceSynchronize();
+    if (!B_resident) dfree(dB);
+    if (!A_resident) dfree(dA);
+    dfree(dAsel); dfree(dusers); dfree(dptr); dfree(d_ix); dfree(d_out); dfree(d_sc); dfree(d_bad);
+    dfree(d_su); dfree(d_lu); dfree(d_seg); dfree(id0); dfree(id1); dfree(key0); dfree(key1); dfree(tmp);
+    return rc;
+}
+
 template <class real, class IX>
 static int topn_single_impl(const real* a_vec, const real* B, int k, const IX* include_ix, size_t n_include,
                             IX* exclude_ix, size_t n_exclude, IX* outp_ix, real* outp_score, size_t n_top, size_t n)
@@ -2302,4 +2496,34 @@ extern "C" int pmf_b200_topN_batch(int dtype, int index_bytes, const void* A, co
     if (dtype == PMF_F64 && index_bytes == 8) return topn_batch_impl((const double*)A, (const double*)B, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)excl_ptr, (const uint64_t*)excl_ix, (uint64_t*)outp_ix, (double*)outp_score, n_top, n, false);
     if (dtype == PMF_F64 && index_bytes == 4) return topn_batch_impl((const double*)A, (const double*)B, k, (const int*)user_ix, n_users, dimA, (const int*)excl_ptr, (const int*)excl_ix, (int*)outp_ix, (double*)outp_score, n_top, n, false);
     return fail("topN_batch: bad dtype/index width");
+}
+
+extern "C" int pmf_b200_topN_batch_include(int dtype, int index_bytes, const void* A, const void* B, int k,
+                                           const void* user_ix, size_t n_users, size_t dimA,
+                                           const void* incl_ptr, const void* incl_ix,
+                                           void* outp_ix, void* outp_score, size_t n_top, size_t n)
+{
+    if (pmf_b200_device_count() <= 0) return fail("no usable CUDA device: poismf_b200 has no CPU fallback");
+    if (dtype == PMF_F32 && index_bytes == 8) return topn_include_impl((const float*)A, (const float*)B, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)incl_ptr, (const uint64_t*)incl_ix, (uint64_t*)outp_ix, (float*)outp_score, n_top, n);
+    if (dtype == PMF_F32 && index_bytes == 4) return topn_include_impl((const float*)A, (const float*)B, k, (const int*)user_ix, n_users, dimA, (const int*)incl_ptr, (const int*)incl_ix, (int*)outp_ix, (float*)outp_score, n_top, n);
+    if (dtype == PMF_F64 && index_bytes == 8) return topn_include_impl((const double*)A, (const double*)B, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)incl_ptr, (const uint64_t*)incl_ix, (uint64_t*)outp_ix, (double*)outp_score, n_top, n);
+    if (dtype == PMF_F64 && index_bytes == 4) return topn_include_impl((const double*)A, (const double*)B, k, (const int*)user_ix, n_users, dimA, (const int*)incl_ptr, (const int*)incl_ix, (int*)outp_ix, (double*)outp_score, n_top, n);
+    return fail("topN_batch_include: bad dtype/index width");
+}
+
+extern "C" int pmf_b200_topN_fitted_include(pmf_b200_handle* h, int index_bytes, const void* user_ix, size_t n_users,
+                                            const void* incl_ptr, const void* incl_ix, void* outp_ix, void* outp_score,
+                                            size_t n_top)
+{
+    if (!h) return fail("topN_fitted_include: null handle");
+    if (pmf_b200_sync(h)) return 1;
+    ResidentFactors rf = {h->factor_ptr(0), h->factor_ptr(1), h->device, h->ldf};
+    if (!rf.A || !rf.B) return fail("topN_fitted_include: the handle holds no factors");
+    const size_t dimA = h->dimA, n = h->dimB;
+    const int k = h->k;
+    if (h->dtype == PMF_F32 && index_bytes == 8) return topn_include_impl<float, uint64_t>(nullptr, nullptr, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)incl_ptr, (const uint64_t*)incl_ix, (uint64_t*)outp_ix, (float*)outp_score, n_top, n, &rf);
+    if (h->dtype == PMF_F32 && index_bytes == 4) return topn_include_impl<float, int>(nullptr, nullptr, k, (const int*)user_ix, n_users, dimA, (const int*)incl_ptr, (const int*)incl_ix, (int*)outp_ix, (float*)outp_score, n_top, n, &rf);
+    if (h->dtype == PMF_F64 && index_bytes == 8) return topn_include_impl<double, uint64_t>(nullptr, nullptr, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)incl_ptr, (const uint64_t*)incl_ix, (uint64_t*)outp_ix, (double*)outp_score, n_top, n, &rf);
+    if (h->dtype == PMF_F64 && index_bytes == 4) return topn_include_impl<double, int>(nullptr, nullptr, k, (const int*)user_ix, n_users, dimA, (const int*)incl_ptr, (const int*)incl_ix, (int*)outp_ix, (double*)outp_score, n_top, n, &rf);
+    return fail("topN_fitted_include: bad dtype/index width");
 }

@@ -65,18 +65,27 @@ class DeviceFit:
         assert rows.dtype == self.dtype and rows.flags.c_contiguous
         self._ck(self.L.pmf_b200_set_factor_rows(self.h, which, _lib.ptr(rows), row_begin, rows.shape[0]))
 
-    def topN(self, users=None, excl_ptr=None, excl_ix=None, top_n=10, output_score=False):
+    def topN(self, users=None, excl_ptr=None, excl_ix=None, top_n=10, output_score=False, incl_ptr=None,
+             incl_ix=None):
         """Batched top-N of `users` (default: every user) against the factors resident in this handle — after a
-        fit nothing but the ids travels (include/poismf_b200.h: pmf_b200_topN_fitted)."""
+        fit nothing but the ids travels (include/poismf_b200.h: pmf_b200_topN_fitted).  With `incl_ptr` /
+        `incl_ix` user u ranks only the items incl_ix[incl_ptr[u]:incl_ptr[u+1]] (pmf_b200_topN_fitted_include)."""
+        from .c_funs import _include_lists
         ixdt = np.uint64
         u = None if users is None else np.ascontiguousarray(users, dtype=ixdt)
         n_users = self.dimA if u is None else u.shape[0]
-        ep = None if excl_ptr is None else np.ascontiguousarray(excl_ptr, dtype=ixdt)
-        ei = None if excl_ix is None else np.ascontiguousarray(excl_ix, dtype=ixdt)
+        include = _include_lists(incl_ptr, incl_ix, excl_ptr, excl_ix, n_users)
         ids = np.empty((n_users, top_n), dtype=ixdt)
         sc = np.empty((n_users, top_n) if output_score else (0, 0), dtype=self.dtype)
-        rc = self.L.pmf_b200_topN_fitted(self.h, 8, _lib.ptr(u), n_users, _lib.ptr(ep), _lib.ptr(ei), _lib.ptr(ids),
-                                         _lib.ptr(sc) if output_score else None, top_n)
+        if include is not None:
+            rc = self.L.pmf_b200_topN_fitted_include(self.h, 8, _lib.ptr(u), n_users, _lib.ptr(include[0]),
+                                                     _lib.ptr(include[1]), _lib.ptr(ids),
+                                                     _lib.ptr(sc) if output_score else None, top_n)
+        else:
+            ep = None if excl_ptr is None else np.ascontiguousarray(excl_ptr, dtype=ixdt)
+            ei = None if excl_ix is None else np.ascontiguousarray(excl_ix, dtype=ixdt)
+            rc = self.L.pmf_b200_topN_fitted(self.h, 8, _lib.ptr(u), n_users, _lib.ptr(ep), _lib.ptr(ei),
+                                             _lib.ptr(ids), _lib.ptr(sc) if output_score else None, top_n)
         if rc == 2:
             raise ValueError("topN: invalid arguments")
         self._ck(rc)

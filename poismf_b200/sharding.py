@@ -264,17 +264,22 @@ class GpuBackend:
         return self.fit.get_factors(*(out or (None, None)))
 
 
-    def topN(self, top_n, users=None, excl_ptr=None, excl_ix=None, output_score=False, gather=True):
+    def topN(self, top_n, users=None, excl_ptr=None, excl_ix=None, output_score=False, gather=True, incl_ptr=None,
+             incl_ix=None):
         """Batched top-N after the fit, users split across the ranks: every rank ranks its share against ITS
         replicas of A and B (resident: pmf_b200_topN_fitted, no factor leaves or enters a GPU) and the per-user
         lists are all-gathered: every rank returns the full (n_users x top_n) result.  With gather=False a
-        rank returns the lists of its own share only (user_ranges(n_users, world)[rank])."""
+        rank returns the lists of its own share only (user_ranges(n_users, world)[rank]).  With `incl_ptr` /
+        `incl_ix` user u ranks only its listed items (pmf_b200_topN_fitted_include)."""
         dimA, dimB, dt = self.fit.dimA, self.fit.dimB, self.fit.dtype
-        scorer = lambda A_, B_, u_, p_, i_, n_, s_: self.fit.topN(users=u_, excl_ptr=p_, excl_ix=i_, top_n=n_,
-                                                                  output_score=s_)
+
+        def scorer(A_, B_, u_, p_, i_, n_, s_, include=False):
+            if include:
+                return self.fit.topN(users=u_, incl_ptr=p_, incl_ix=i_, top_n=n_, output_score=s_)
+            return self.fit.topN(users=u_, excl_ptr=p_, excl_ix=i_, top_n=n_, output_score=s_)
         return topn_sharded(np.empty((dimA, 0), dt), np.empty((dimB, 0), dt), top_n, users=users, excl_ptr=excl_ptr,
                             excl_ix=excl_ix, output_score=output_score, rank=self.rank, world=self.world,
-                            group=self.group, scorer=scorer, gather=gather)
+                            group=self.group, scorer=scorer, gather=gather, incl_ptr=incl_ptr, incl_ix=incl_ix)
 
 
 def user_ranges(n_users, nparts):
@@ -284,27 +289,40 @@ def user_ranges(n_users, nparts):
 
 
 def topn_sharded(A, B, top_n, users=None, excl_ptr=None, excl_ix=None, output_score=False, rank=0, world=1,
-                 group=None, scorer=None, gather=True):
+                 group=None, scorer=None, gather=True, incl_ptr=None, incl_ix=None):
     """Batched topN with the USERS split across ranks (SURVEY.md 8e): B is replicated, every rank ranks
     its own contiguous range of users on its GPU, and the per-user lists are all-gathered — no exchange
-    inside the scoring.  Every rank returns the full (n_users x top_n) result.
+    inside the scoring.  Every rank returns the full (n_users x top_n) result.  With `incl_ptr` / `incl_ix`
+    user u ranks only the items incl_ix[incl_ptr[u]:incl_ptr[u+1]]; they are sliced by user range like the
+    exclusion lists.
 
     `scorer(A, B, users, excl_ptr, excl_ix, top_n, output_score) -> (ids, scores)` defaults to the
-    device path (c_funs._topN_batch); the CPU tests inject a stand-in."""
+    device path (c_funs._topN_batch); the CPU tests inject a stand-in.  With include lists it is called as
+    `scorer(A, B, users, incl_ptr, incl_ix, top_n, output_score, include=True)`."""
+    include = incl_ptr is not None or incl_ix is not None
+    if include and (excl_ptr is not None or excl_ix is not None):
+        raise ValueError("topN: include and exclude lists cannot be combined")
     if scorer is None:
         from . import c_funs
-        scorer = lambda A_, B_, u_, p_, i_, n_, s_: c_funs._topN_batch(A_, B_, users=u_, excl_ptr=p_, excl_ix=i_,
-                                                                     top_n=n_, output_score=s_)
+
+        def scorer(A_, B_, u_, p_, i_, n_, s_, include=False):
+            if include:
+                return c_funs._topN_batch(A_, B_, users=u_, incl_ptr=p_, incl_ix=i_, top_n=n_, output_score=s_)
+            return c_funs._topN_batch(A_, B_, users=u_, excl_ptr=p_, excl_ix=i_, top_n=n_, output_score=s_)
     all_users = np.arange(A.shape[0], dtype=np.uint64) if users is None else np.ascontiguousarray(users, dtype=np.uint64)
     lo, hi = user_ranges(all_users.shape[0], world)[rank]
     mine = np.ascontiguousarray(all_users[lo:hi])
     p_loc = i_loc = None
-    if excl_ptr is not None and excl_ix is not None:
-        ep = np.asarray(excl_ptr).astype(np.int64)
+    lists = (incl_ptr, incl_ix) if include else (excl_ptr, excl_ix)
+    if lists[0] is not None and lists[1] is not None:
+        ep = np.asarray(lists[0]).astype(np.int64)
         p_loc = np.ascontiguousarray(ep[lo:hi + 1] - ep[lo]).astype(np.uint64)
-        i_loc = np.ascontiguousarray(np.asarray(excl_ix)[ep[lo]:ep[hi]]).astype(np.uint64)
+        i_loc = np.ascontiguousarray(np.asarray(lists[1])[ep[lo]:ep[hi]]).astype(np.uint64)
     if hi > lo:
-        ids, sc = scorer(A, B, mine, p_loc, i_loc, top_n, output_score)
+        if include:
+            ids, sc = scorer(A, B, mine, p_loc, i_loc, top_n, output_score, include=True)
+        else:
+            ids, sc = scorer(A, B, mine, p_loc, i_loc, top_n, output_score)
     else:
         ids = np.empty((0, top_n), np.uint64)
         sc = np.empty((0, top_n) if output_score else (0, 0), B.dtype)
