@@ -148,13 +148,16 @@ PMF_DEVINL void dots_fast(const RowView<real>& rv, const real* a, real* out, int
 }
 
 // Fast-mode dot products for a tile that is NOT staged (rows streamed from global memory / L2):
-// a group of G lanes reads one factor row with coalesced 16-byte loads (lane c takes chunk c),
-// keeps its chunk(s) of `a` in registers, and the G partial sums are folded with shuffles.
+// a group of G lanes reads one factor row with coalesced 16-byte loads (lane c takes chunks c, c+32, ...),
+// keeps its chunks of `a` in registers, and the G partial sums are folded with shuffles.
 template <class real, class Team>
 PMF_DEVINL void dots_stream(const Team& tm, const RowView<real>& rv, const real* a, real* out)
 {
     using VT = typename Vec16<real>::type;
     constexpr int V = RealTraits<real>::V;
+    // chunks per lane: enough for ldf = 256 (the largest k a handle takes), i.e. 64 chunks of 16 bytes in
+    // float and 128 in double
+    constexpr int NCH = (256 / V + 31) / 32;
     const int n = rv.n, L = rv.ldf / V;
     int G = 1;
     while (G < L && G < 32) G <<= 1;
@@ -164,8 +167,9 @@ PMF_DEVINL void dots_stream(const Team& tm, const RowView<real>& rv, const real*
     const VT* Fv = reinterpret_cast<const VT*>(rv.F);
     const size_t ldv = (size_t)rv.ldf / V;
     VT zero; vzero(zero);
-    const bool has0 = c < L, has1 = c + 32 < L;         // second chunk only when L > 32 (G == 32)
-    const VT a0 = has0 ? av[c] : zero, a1 = has1 ? av[c + 32] : zero;
+    bool has[NCH]; VT ac[NCH];                                  // chunk c + 32 j only when L > 32 j (G == 32)
+#pragma unroll
+    for (int j = 0; j < NCH; j++) { has[j] = c + 32 * j < L; ac[j] = has[j] ? av[c + 32 * j] : zero; }
     // warp-uniform trip count (the shuffles below need every lane of the warp): iterate on the
     // warp's first group and predicate the memory accesses
     const int gpw = 32 / G;                                     // groups per warp
@@ -180,14 +184,17 @@ PMF_DEVINL void dots_stream(const Team& tm, const RowView<real>& rv, const real*
         for (int u = 0; u < U; u++) id[u] = rv.ind[ok[u] ? tt[u] : 0];          // all index loads first
 #pragma unroll
         for (int u = 0; u < U; u++) r[u] = Fv + (size_t)id[u] * ldv;
-        VT b0[U], b1[U];
+        VT b[U][NCH];
 #pragma unroll
-        for (int u = 0; u < U; u++) {                                           // then all row loads
-            b0[u] = has0 ? __ldg(r[u] + c) : zero;
-            b1[u] = has1 ? __ldg(r[u] + c + 32) : zero;
+        for (int u = 0; u < U; u++)                                             // then all row loads
+#pragma unroll
+            for (int j = 0; j < NCH; j++) b[u][j] = has[j] ? __ldg(r[u] + c + 32 * j) : zero;
+#pragma unroll
+        for (int u = 0; u < U; u++) {
+            sacc[u] = vdot4(ac[0], b[u][0], (real)0);
+#pragma unroll
+            for (int j = 1; j < NCH; j++) if (has[j]) sacc[u] = vdot4(ac[j], b[u][j], sacc[u]);
         }
-#pragma unroll
-        for (int u = 0; u < U; u++) { sacc[u] = vdot4(a0, b0[u], (real)0); if (has1) sacc[u] = vdot4(a1, b1[u], sacc[u]); }
         for (int o = G >> 1; o > 0; o >>= 1) {
 #pragma unroll
             for (int u = 0; u < U; u++) sacc[u] += __shfl_xor_sync(0xffffffffu, sacc[u], o);
