@@ -74,6 +74,38 @@ extern "C" int pmf_b200_device_count(void)
     return n;
 }
 
+// fn(real(), IX()) for the value type (PMF_F32: float, PMF_F64: double) and index width (8: uint64_t, 4: int)
+// of a C call; `bad` is the error of any other pair
+template <class F>
+static int with_types(int dtype, int index_bytes, const char* bad, F&& fn)
+{
+    if (dtype == PMF_F32 && index_bytes == 8) return fn(float(), uint64_t());
+    if (dtype == PMF_F32 && index_bytes == 4) return fn(float(), int());
+    if (dtype == PMF_F64 && index_bytes == 8) return fn(double(), uint64_t());
+    if (dtype == PMF_F64 && index_bytes == 4) return fn(double(), int());
+    return fail("%s", bad);
+}
+
+// The device blocks of one call, released to the pool when it returns.  A call marks them settled once its
+// last result is back on the host; one that returns before (an error, a failed check) may leave kernels
+// using them, so the device is synchronised before they can go to another allocation.
+struct DeviceBlocks {
+    std::vector<void*> held;
+    bool settled = false;
+    template <class T> cudaError_t alloc(T** p, size_t bytes)
+    {
+        const cudaError_t e = dmalloc(p, bytes);
+        if (e == cudaSuccess) held.push_back(*p);
+        return e;
+    }
+    void adopt(void* p) { held.push_back(p); }
+    ~DeviceBlocks()
+    {
+        if (!settled) cudaDeviceSynchronize();
+        for (void* p : held) dfree(p);
+    }
+};
+
 static inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
 static inline size_t round_up_sz(size_t v, size_t m) { return (v + m - 1) / m * m; }
 
@@ -1708,14 +1740,12 @@ extern "C" int pmf_b200_factors_single(int dtype, int index_bytes, void* out, si
                                        double w_mult, int flags)
 {
     if (index_bytes != 4 && index_bytes != 8) return fail("factors_single: index_bytes must be 4 or 8");
-#define PMF_FS(real, IX)                                                                                            \
-    return factors_single_impl<real, IX>(dtype, (real*)out, k, (const real*)Amean, reuse_mean, (const real*)X,       \
-                                         (const IX*)X_ind, nnz, (const real*)B, (const real*)Bsum, maxupd, l2_reg,  \
-                                         l1_new, l1_old, w_mult, flags)
-    if (dtype == PMF_F32) { if (index_bytes == 8) PMF_FS(float, uint64_t); else PMF_FS(float, int); }
-    if (dtype == PMF_F64) { if (index_bytes == 8) PMF_FS(double, uint64_t); else PMF_FS(double, int); }
-#undef PMF_FS
-    return fail("bad dtype");
+    return with_types(dtype, index_bytes, "bad dtype", [&](auto r, auto i) {
+        using real = decltype(r); using IX = decltype(i);
+        return factors_single_impl<real, IX>(dtype, (real*)out, k, (const real*)Amean, reuse_mean, (const real*)X,
+                                             (const IX*)X_ind, nnz, (const real*)B, (const real*)Bsum, maxupd, l2_reg,
+                                             l1_new, l1_old, w_mult, flags);
+    });
 }
 
 // ---- dense host rows -> padded device rows, for the stateless inference entry points -----------------
@@ -1786,65 +1816,112 @@ static int predict_impl(real* out, const real* A, const real* B, const IX* ixA, 
                         size_t dimA, size_t dimB)
 {
     CK(cudaSetDevice(env_device()));
-    real *dA = nullptr, *dB = nullptr, *dout = nullptr;
-    IX *da = nullptr, *db = nullptr;
     if (n == 0) return 0;
     // Few pairs (the reference's per-user call pattern, poismf/__init__.py:726-835): only the rows the pairs
     // name travel — gathered on the host into two n x k blocks, 2 n k reals instead of both whole matrices.
     // (crossover measured on B200: the host gather costs ~0.3 us per pair, the two whole uploads ~10 ms at config #2's shape)
     const bool gathered = 32 * n < dimA + dimB;
     const size_t rowsA = gathered ? n : dimA, rowsB = gathered ? n : dimB;
-    auto body = [&]() -> int {
-        CK(dmalloc(&dA, rowsA * (size_t)k * sizeof(real))); CK(dmalloc(&dB, rowsB * (size_t)k * sizeof(real)));
-        CK(dmalloc(&dout, n * sizeof(real)));
-        if (gathered) {
-            std::vector<real> ga(n * (size_t)k), gb(n * (size_t)k);
-            for (size_t i = 0; i < n; i++) {
-                memcpy(&ga[i * k], A + (size_t)ixA[i] * k, (size_t)k * sizeof(real));
-                memcpy(&gb[i * k], B + (size_t)ixB[i] * k, (size_t)k * sizeof(real));
-            }
-            CK(cudaMemcpy(dA, ga.data(), n * (size_t)k * sizeof(real), cudaMemcpyHostToDevice));
-            CK(cudaMemcpy(dB, gb.data(), n * (size_t)k * sizeof(real), cudaMemcpyHostToDevice));
-        } else {
-            CK(dmalloc(&da, n * sizeof(IX))); CK(dmalloc(&db, n * sizeof(IX)));
-            CK(cudaMemcpy(dA, A, dimA * (size_t)k * sizeof(real), cudaMemcpyHostToDevice));      // rows stay k wide: the
-            CK(cudaMemcpy(dB, B, dimB * (size_t)k * sizeof(real), cudaMemcpyHostToDevice));      // kernel reads scalars
-            CK(cudaMemcpy(da, ixA, n * sizeof(IX), cudaMemcpyHostToDevice));
-            CK(cudaMemcpy(db, ixB, n * sizeof(IX), cudaMemcpyHostToDevice));
+    DeviceBlocks mem;
+    real *dA = nullptr, *dB = nullptr, *dout = nullptr;
+    IX *da = nullptr, *db = nullptr;
+    CK(mem.alloc(&dA, rowsA * (size_t)k * sizeof(real))); CK(mem.alloc(&dB, rowsB * (size_t)k * sizeof(real)));
+    CK(mem.alloc(&dout, n * sizeof(real)));
+    if (gathered) {
+        std::vector<real> ga(n * (size_t)k), gb(n * (size_t)k);
+        for (size_t i = 0; i < n; i++) {
+            memcpy(&ga[i * k], A + (size_t)ixA[i] * k, (size_t)k * sizeof(real));
+            memcpy(&gb[i * k], B + (size_t)ixB[i] * k, (size_t)k * sizeof(real));
         }
-        const int grid = (int)std::min<size_t>((n + 255) / 256, 148 * 16);
-        predict_pairs_kernel<real, IX><<<grid, 256>>>(dA, dB, da, db, n, k, k, dout);
-        LAUNCHED();
-        CK(cudaGetLastError());
-        CK(cudaMemcpy(out, dout, n * sizeof(real), cudaMemcpyDeviceToHost));
-        return 0;
-    };
-    int rc = body();
-    if (rc) cudaDeviceSynchronize();     // blocks go back to the cache: nothing may still be using them
-    dfree(dA); dfree(dB); dfree(dout); dfree(da); dfree(db);
-    return rc;
+        CK(cudaMemcpy(dA, ga.data(), n * (size_t)k * sizeof(real), cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(dB, gb.data(), n * (size_t)k * sizeof(real), cudaMemcpyHostToDevice));
+    } else {
+        CK(mem.alloc(&da, n * sizeof(IX))); CK(mem.alloc(&db, n * sizeof(IX)));
+        CK(cudaMemcpy(dA, A, dimA * (size_t)k * sizeof(real), cudaMemcpyHostToDevice));      // rows stay k wide: the
+        CK(cudaMemcpy(dB, B, dimB * (size_t)k * sizeof(real), cudaMemcpyHostToDevice));      // kernel reads scalars
+        CK(cudaMemcpy(da, ixA, n * sizeof(IX), cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(db, ixB, n * sizeof(IX), cudaMemcpyHostToDevice));
+    }
+    const int grid = (int)std::min<size_t>((n + 255) / 256, 148 * 16);
+    predict_pairs_kernel<real, IX><<<grid, 256>>>(dA, dB, da, db, n, k, k, dout);
+    LAUNCHED();
+    CK(cudaGetLastError());
+    CK(cudaMemcpy(out, dout, n * sizeof(real), cudaMemcpyDeviceToHost));
+    mem.settled = true;
+    return 0;
 }
 extern "C" int pmf_b200_predict_multiple(int dtype, int index_bytes, void* out, const void* A, const void* B,
                                          const void* ixA, const void* ixB, size_t n, int k, size_t dimA, size_t dimB)
 {
     if (pmf_b200_device_count() <= 0) return fail("no usable CUDA device: poismf_b200 has no CPU fallback");
-    if (dtype == PMF_F32 && index_bytes == 8) return predict_impl((float*)out, (const float*)A, (const float*)B, (const uint64_t*)ixA, (const uint64_t*)ixB, n, k, dimA, dimB);
-    if (dtype == PMF_F32 && index_bytes == 4) return predict_impl((float*)out, (const float*)A, (const float*)B, (const int*)ixA, (const int*)ixB, n, k, dimA, dimB);
-    if (dtype == PMF_F64 && index_bytes == 8) return predict_impl((double*)out, (const double*)A, (const double*)B, (const uint64_t*)ixA, (const uint64_t*)ixB, n, k, dimA, dimB);
-    if (dtype == PMF_F64 && index_bytes == 4) return predict_impl((double*)out, (const double*)A, (const double*)B, (const int*)ixA, (const int*)ixB, n, k, dimA, dimB);
-    return fail("predict_multiple: bad dtype/index width");
+    return with_types(dtype, index_bytes, "predict_multiple: bad dtype/index width", [&](auto r, auto i) {
+        using real = decltype(r); using IX = decltype(i);
+        return predict_impl((real*)out, (const real*)A, (const real*)B, (const IX*)ixA, (const IX*)ixB, n, k, dimA, dimB);
+    });
 }
 
 // ---- topN ----------------------------------------------------------------------
 struct ResidentFactors { const void* A; const void* B; int device; int ldf; };
 
-// v1: exact scores (same sums as the reference) + CUB segmented radix sort.
-// Ranking = descending score; ties by ascending item id (the reference's tie order
-// is qsort's, i.e. unspecified).
+// A (rowsA rows) and B (n rows) on the device, rows padded to ldf: a fit handle's replicas when rf is given
+// (nothing is uploaded), else uploaded, B through the resident-matrix cache.  Uploaded blocks that the cache
+// does not keep are released with `mem`.
+template <class real>
+static int factors_on_device(const ResidentFactors* rf, const real* A, size_t rowsA, const real* B, size_t n, int k,
+                             int ldf, DeviceBlocks& mem, real** dA, real** dB, const char* what)
+{
+    if (rf) {
+        if (rf->ldf != ldf) return fail("%s: resident factors have another row pitch", what);
+        *dA = (real*)rf->A; *dB = (real*)rf->B;
+        return 0;
+    }
+    bool resident = false;
+    if (upload_rows<real>(dB, B, n, k, ldf, &resident, true)) return 1;
+    if (!resident) mem.adopt(*dB);
+    if (upload_rows<real>(dA, A, rowsA, k, ldf, &resident, false)) return 1;
+    if (!resident) mem.adopt(*dA);
+    return 0;
+}
+
+// rows user_ix[u0 .. u0 + m) of dA (rows u0 .. u0 + m without a list) -> dAsel, through the device list dusers
+template <class real, class IX>
+static int gather_users(const real* dA, int ldf, const IX* user_ix, size_t u0, size_t m, long long* dusers, real* dAsel)
+{
+    std::vector<long long> hu(m);
+    for (size_t u = 0; u < m; u++) hu[u] = user_ix ? (long long)user_ix[u0 + u] : (long long)(u0 + u);
+    CK(cudaMemcpy(dusers, hu.data(), m * sizeof(long long), cudaMemcpyHostToDevice));
+    gather_rows_kernel<real><<<(int)std::min<size_t>((m * ldf + 255) / 256, 4096), 256>>>(dA, dusers, (int)m, ldf, dAsel);
+    LAUNCHED();
+    return 0;
+}
+
+// -> 0 when every one of the `count` ids on the device lies in [0, n), 2 when one does not (a negative id of a
+// signed type is a huge size_t), 1 on a CUDA error.  Callers run it before any result is written.
+template <class IX>
+static int ids_in_range(const IX* dev_ids, size_t count, size_t n)
+{
+    if (!count) return 0;
+    DeviceBlocks mem;
+    int* d_bad = nullptr;
+    int bad = 0;
+    CK(mem.alloc(&d_bad, sizeof(int)));
+    CK(cudaMemsetAsync(d_bad, 0, sizeof(int)));
+    tc::any_id_out_of_range_kernel<IX><<<592, 256>>>(dev_ids, count, n, d_bad);
+    LAUNCHED();
+    CK(cudaMemcpy(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost));
+    mem.settled = true;
+    return bad ? 2 : 0;
+}
+
+// Batched topN over every item but the user's exclusions.  Three routes give the same ids and scores: the fused
+// tensor-core select (topn_tc.cuh), the TF32 score matrix + CUB's segmented radix sort + exact re-score when the
+// items are too few for the fused select, else exact scores (the reference's sums) and the segmented sort.
+// Ranking = descending score; ties by ascending item id (the reference's tie order is
+// qsort's, i.e. unspecified).  A single vector is the matrix A of one row: dimA = 1, n_users = 1, no user list.
 template <class real, class IX>
 static int topn_batch_impl(const real* A, const real* B, int k, const IX* user_ix, size_t n_users, size_t dimA,
                            const IX* excl_ptr, const IX* excl_ix, IX* outp_ix, real* outp_score, size_t n_top, size_t n,
-                           bool A_is_single_vector, bool allow_tc = true, const ResidentFactors* rf = nullptr)
+                           bool allow_tc = true, const ResidentFactors* rf = nullptr)
 {
     // rf: the factors already sit on a device, padded to ldf (a fit handle's replicas): nothing is uploaded
     CK(cudaSetDevice(rf ? rf->device : env_device()));
@@ -1860,91 +1937,67 @@ static int topn_batch_impl(const real* A, const real* B, int k, const IX* user_i
         t_last = now;
     };
     // argument checks in the spirit of src/topN.c:121-128, per user: ids inside the matrices, offsets monotone,
-    // enough items left after the exclusions
-    if (user_ix && !A_is_single_vector)
+    // enough items left after the exclusions (the excluded ids are range-checked on the device once uploaded)
+    if (user_ix)
         for (size_t u = 0; u < n_users; u++)
             if ((size_t)user_ix[u] >= dimA) return 2;
-    if (excl_ptr && excl_ix) {
+    const bool have_excl = excl_ptr && excl_ix;
+    if (have_excl)
         for (size_t u = 0; u < n_users; u++) {
             if (excl_ptr[u + 1] < excl_ptr[u]) return 2;
             if ((size_t)(excl_ptr[u + 1] - excl_ptr[u]) > n - n_top) return 2;
         }
-        // (the ids themselves are range-checked on the device once uploaded: `excl_ids_ok` below)
-    }
-    // -> 0 ok, 2 an excluded id outside [0, n), 1 CUDA error.  Runs before any result is written.
-    auto excl_ids_ok = [&](const IX* dev_ids, size_t count) -> int {
-        if (!count) return 0;
-        int* d_bad = nullptr;
-        int bad = 0;
-        CK(dmalloc(&d_bad, sizeof(int)));
-        cudaError_t e = cudaMemsetAsync(d_bad, 0, sizeof(int));
-        if (e == cudaSuccess) {
-            tc::any_id_out_of_range_kernel<IX><<<592, 256>>>(dev_ids, count, n, d_bad);
-            LAUNCHED();
-            e = cudaMemcpy(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost);
-        }
-        dfree(d_bad);
-        if (e != cudaSuccess) return fail("topN: id check failed: %s", cudaGetErrorString(e));
-        return bad ? 2 : 0;
-    };
     const int V = RealTraits<real>::V, ldf = round_up(k, V);
-    const size_t w = (size_t)k * sizeof(real), pitch = (size_t)ldf * sizeof(real);
-    // users per chunk: bound the score matrix to ~1 GiB
-    size_t chunk = std::max<size_t>(1, std::min<size_t>(n_users, ((size_t)1 << 28) / std::max<size_t>(n, 1)));
-    chunk = std::min<size_t>(chunk, 65535);
-    real *dB = nullptr, *dA = nullptr, *dAsel = nullptr, *sc_in = nullptr, *sc_out = nullptr;
-    int *id_in = nullptr, *id_out = nullptr, *seg = nullptr;
-    long long* dusers = nullptr;
-    IX *dexp = nullptr, *dexi = nullptr;
-    void* tmp = nullptr;
-    std::vector<int> h_ids(chunk * n_top);
-    std::vector<real> h_sc(chunk * n_top);
-    // tensor-core candidate scorer (topn_tc.cuh): float, k <= 128, n_top <= 128, non-negative factors
-    bool use_tc = allow_tc && std::is_same<real, float>::value && k <= 128 && n_top <= 128 && n >= 256 &&
-                  !getenv("POISMF_B200_TOPN_EXACT");
+    const size_t pitch = (size_t)ldf * sizeof(real);
     const int kpad = round_up(k, 8);
     const int M_cand = (int)std::min<size_t>(n, std::min<size_t>(256, std::max<size_t>(2 * n_top, n_top + 32)));
-    long long* d_out_ids = nullptr; float* d_out_sc = nullptr; int* d_flag = nullptr; int* d_neg = nullptr;
-    bool B_resident = false;           // dB belongs to the resident-matrix cache: not released here
-    bool A_resident = false;           // (both belong to a fit handle)
+    const size_t ntiles = (n + tc::TN - 1) / tc::TN, ngroups = (n + tc::GROUP - 1) / tc::GROUP;
+    // TF32 candidates: float factors, k <= 128, n_top <= 128 and (checked on the device below) non-negative
+    // factors, which the TF32 error bound assumes.  The fused select needs the items to hold 2 M_cand groups.
+    // With fewer, the TF32 scores are sorted and the best M_cand re-scored exactly when there are >= 256 users
+    // and n k >= 2 M_cand (k + 32): the exact re-score costs about M_cand (k + 32) per user against n k for exact
+    // scores.  Wherever the exact route measured faster than this one, the rule picks it; it never picks it where
+    // this one measured faster (32 768 users down to 1, 256..6 384 items, k 16/64/128, top-10/100:
+    // profiles/r4_topn_sort_vs_exact.json)
+    const bool fits_fused = ngroups >= (size_t)2 * M_cand;
+    const bool sort_tf32 = n_users >= 256 && n * (size_t)k >= (size_t)2 * M_cand * (size_t)(k + 32);
+    bool use_tc = allow_tc && std::is_same<real, float>::value && k <= 128 && n_top <= 128 && n >= 256 &&
+                  (fits_fused || sort_tf32) && !getenv("POISMF_B200_TOPN_EXACT");
+    bool fused = false;
     std::vector<size_t> redo;          // users whose TF32 proof failed: redone exactly afterwards
-    auto body = [&]() -> int {
-        const size_t rowsA = A_is_single_vector ? 1 : dimA;
-        bool dummy = false;
+    {
+        DeviceBlocks mem;
+        real *dA = nullptr, *dB = nullptr;
         mark("argument checks");
-        if (rf) {
-            if (rf->ldf != ldf) return fail("topN: resident factors have another row pitch");
-            dB = (real*)rf->B; dA = (real*)rf->A;
-            B_resident = A_resident = true;
-        } else {
-            if (upload_rows<real>(&dB, B, n, k, ldf, &B_resident, true)) return 1;
-            mark("upload B");
-            if (upload_rows<real>(&dA, A, rowsA, k, ldf, &dummy, false)) return 1;
-            mark("upload A");
+        if (factors_on_device(rf, A, dimA, B, n, k, ldf, mem, &dA, &dB, "topN")) return 1;
+        mark("factors on device");
+        IX *dexp = nullptr, *dexi = nullptr;
+        if (have_excl) {
+            const size_t n_excl_total = (size_t)excl_ptr[n_users];
+            CK(mem.alloc(&dexp, (n_users + 1) * sizeof(IX)));
+            CK(mem.alloc(&dexi, std::max<size_t>(n_excl_total, 1) * sizeof(IX)));
+            CK(cudaMemcpy(dexp, excl_ptr, (n_users + 1) * sizeof(IX), cudaMemcpyHostToDevice));
+            CK(Stager::get().h2d(dexi, excl_ix, n_excl_total * sizeof(IX), 0));
+            if (const int bad = ids_in_range(dexi + (size_t)excl_ptr[0], n_excl_total - (size_t)excl_ptr[0], n)) return bad;
         }
+        CUtensorMap mapB;                  // B for the TMA unit, the same for every chunk of users
         if (use_tc) {
-            CK(dmalloc(&d_neg, sizeof(int)));
+            int* d_neg = nullptr;
+            CK(mem.alloc(&d_neg, sizeof(int)));
             CK(cudaMemset(d_neg, 0, sizeof(int)));
             tc::any_negative_kernel<<<256, 256>>>((const float*)dB, n * (size_t)ldf, d_neg);
-            tc::any_negative_kernel<<<256, 256>>>((const float*)dA, rowsA * (size_t)ldf, d_neg);
+            tc::any_negative_kernel<<<256, 256>>>((const float*)dA, dimA * (size_t)ldf, d_neg);
             LAUNCHED(); LAUNCHED();
             int neg = 0;
             CK(cudaMemcpy(&neg, d_neg, sizeof(int), cudaMemcpyDeviceToHost));
-            if (neg) use_tc = false;      // the TF32 error bound below assumes non-negative factors
+            use_tc = !neg && tc::make_operand_map(&mapB, (const float*)dB, n, ldf) == 0;
+            fused = use_tc && fits_fused;
         }
-        const size_t ntiles = (n + tc::TN - 1) / tc::TN, ngroups = (n + tc::GROUP - 1) / tc::GROUP;
-        int num_sms = 148;
-        {
-            int dev = 0;
-            CK(cudaGetDevice(&dev));
-            CK(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
-        }
-        if (use_tc && ngroups >= (size_t)2 * M_cand && !getenv("POISMF_B200_TOPN_SORT")) {
+        if (fused) {
             // ---- fused select (topn_tc.cuh): no score matrix; two passes over the tensor-core tiles ----
             const size_t words = ntiles * 4;     // exclusion bitmap: 128 bits per tile and user
-            const bool have_excl = excl_ptr && excl_ix;
-            // group maxima per user: whole tiles (the pipelined scorer numbers 8 groups per visited tile, the last
-            // tile's groups beyond n included)
+            // group maxima per user: whole tiles (the scorer numbers 8 groups per visited tile, the last tile's
+            // groups beyond n included)
             const size_t ngroups_alloc = ntiles * (tc::TN / tc::GROUP);
             const size_t per_user = ngroups_alloc * 4 + (have_excl ? words * 4 : 0) + (size_t)tc::CAND_SLACK * tc::CAND_CAP * 8 +
                                     (size_t)tc::CAND_TOP * 8 + pitch + n_top * 12 + 64;
@@ -1954,270 +2007,226 @@ static int topn_batch_impl(const real* A, const real* B, int k, const IX* user_i
             const size_t budget = std::max<size_t>((size_t)1 << 30, std::min<size_t>(mem_free / 4, (size_t)32 << 30));
             size_t fchunk = std::max<size_t>(1, std::min<size_t>(n_users, budget / per_user));
             fchunk = std::min<size_t>(fchunk, 32768);
-            float *gmax = nullptr, *tau = nullptr, *cand_sc = nullptr, *top_sc = nullptr;
-            int *cand_id = nullptr, *cand_cnt = nullptr, *top_id = nullptr, *d_ovf = nullptr;
+            real* dAsel = nullptr;
+            long long *dusers = nullptr, *d_out_ids = nullptr;
+            float *gmax = nullptr, *tau = nullptr, *cand_sc = nullptr, *top_sc = nullptr, *d_out_sc = nullptr;
+            int *cand_id = nullptr, *cand_cnt = nullptr, *top_id = nullptr, *d_ovf = nullptr, *d_flag = nullptr;
             uint32_t* bits = nullptr;
-            std::vector<void*> mine;
-            auto take = [&](void* q) { mine.push_back(q); };
-            auto fused = [&]() -> int {
-                CK(dmalloc(&dAsel, fchunk * pitch));
-                CK(dmalloc(&dusers, fchunk * sizeof(long long)));
-                CK(dmalloc(&gmax, fchunk * ngroups_alloc * sizeof(float))); take(gmax);
-                CK(dmalloc(&tau, fchunk * sizeof(float))); take(tau);
-                CK(dmalloc(&cand_sc, fchunk * tc::CAND_SLACK * tc::CAND_CAP * sizeof(float))); take(cand_sc);
-                CK(dmalloc(&cand_id, fchunk * tc::CAND_SLACK * tc::CAND_CAP * sizeof(int))); take(cand_id);
-                CK(dmalloc(&cand_cnt, fchunk * 64 * sizeof(int))); take(cand_cnt);      // [user][region], regions <= 64
-                CK(dmalloc(&top_sc, fchunk * tc::CAND_TOP * sizeof(float))); take(top_sc);
-                CK(dmalloc(&top_id, fchunk * tc::CAND_TOP * sizeof(int))); take(top_id);
-                CK(dmalloc(&d_ovf, fchunk * sizeof(int))); take(d_ovf);
-                CK(dmalloc(&d_out_ids, fchunk * n_top * sizeof(long long)));
-                CK(dmalloc(&d_out_sc, fchunk * n_top * sizeof(float)));
-                CK(dmalloc(&d_flag, fchunk * sizeof(int)));
-                if (have_excl) {
-                    const size_t n_excl_total = (size_t)excl_ptr[n_users];
-                    CK(dmalloc(&bits, fchunk * words * sizeof(uint32_t))); take(bits);
-                    CK(dmalloc(&dexp, (n_users + 1) * sizeof(IX)));
-                    CK(dmalloc(&dexi, std::max<size_t>(n_excl_total, 1) * sizeof(IX)));
-                    CK(cudaMemcpy(dexp, excl_ptr, (n_users + 1) * sizeof(IX), cudaMemcpyHostToDevice));
-                    CK(Stager::get().h2d(dexi, excl_ix, n_excl_total * sizeof(IX), 0));
-                    if (const int bad = excl_ids_ok(dexi + (size_t)excl_ptr[0], n_excl_total - (size_t)excl_ptr[0])) return bad;
-                }
-                mark("work arrays + exclusions up");
-                CK(cudaFuncSetAttribute(tc::score_tiles_tf32_kernel<tc::MODE_GROUPMAX>,
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, kpad * 1024));
-                CK(cudaFuncSetAttribute(tc::score_tiles_tf32_kernel<tc::MODE_EMIT>,
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, kpad * 1024));
-                std::vector<long long> hu, hid;
-                std::vector<float> hsc;
-                std::vector<int> hfl, hov;
-                for (size_t u0 = 0; u0 < n_users; u0 += fchunk) {
-                    const size_t m = std::min(fchunk, n_users - u0);
-                    hu.resize(m);
-                    for (size_t u = 0; u < m; u++)
-                        hu[u] = A_is_single_vector ? 0 : (user_ix ? (long long)user_ix[u0 + u] : (long long)(u0 + u));
-                    CK(cudaMemcpy(dusers, hu.data(), m * sizeof(long long), cudaMemcpyHostToDevice));
-                    gather_rows_kernel<real><<<(int)std::min<size_t>((m * ldf + 255) / 256, 4096), 256>>>(dA, dusers, (int)m, ldf, dAsel);
-                    LAUNCHED();
-                    tc::TileOut o = {};
-                    if (have_excl) {
-                        CK(cudaMemsetAsync(bits, 0, m * words * sizeof(uint32_t)));
-                        tc::exclusion_bitmap_kernel<IX><<<dim3(4, (unsigned)m), 128>>>(bits, words, dexp, dexi, u0, n);
-                        LAUNCHED();
-                        o.excl_bits = bits; o.excl_words = words;
-                    }
-                    o.gmax = gmax; o.ngroups = ngroups; o.tau = tau;
-                    o.cand_sc = cand_sc; o.cand_id = cand_id; o.cand_cnt = cand_cnt;
-                    o.cand_regions = 1; o.cand_cap = tc::CAND_CAP;
-                    const dim3 tgrid((unsigned)ntiles, (unsigned)((m + tc::TM - 1) / tc::TM));
-                    // pipelined scorer (persistent CTAs, TMA operands, two TMEM accumulators) unless disabled
-                    CUtensorMap mapA, mapB;
-                    const bool piped = !getenv("POISMF_B200_TOPN_NOPIPE") &&
-                                       tc::make_operand_map(&mapA, (const float*)dAsel, m, ldf) == 0 &&
-                                       tc::make_operand_map(&mapB, (const float*)dB, n, ldf) == 0;
-                    const unsigned ut = (unsigned)((m + tc::PIPE_UT * tc::TM - 1) / (tc::PIPE_UT * tc::TM));   // CTAs along the users
-                    // one CTA per SM (shared memory), every CTA the same run of item tiles: the split of the items
-                    // that fills whole waves best (fewest chunks among the best: the A tiles load once per CTA)
-                    unsigned chunks = 1;
-                    {
-                        double best = 0;
-                        const unsigned cmax = (unsigned)std::max<size_t>(1, std::min<size_t>(ntiles / 32, 64));
-                        for (unsigned c = 1; c <= cmax; c++) {
-                            const size_t ctas = (size_t)c * ut, waves = (ctas + num_sms - 1) / num_sms;
-                            const double eff = (double)ctas / (double)(waves * num_sms);
-                            if (eff > best + 0.02) { best = eff; chunks = c; }
-                        }
-                    }
-                    // The threshold pass visits every S-th item tile only: the M-th largest group maximum of a SAMPLE
-                    // of the items is a lower bound of the one over all items, so every wanted item still passes
-                    // tau; about S M items do (instead of M), which the candidate slots must hold (S M <= 1/4 of them)
-                    int S = 1;
-                    if (piped) {
-                        for (int c : {4, 2})
-                            if (ntiles >= (size_t)c * M_cand && (size_t)c * M_cand <= (size_t)tc::CAND_CAP / 4) { S = c; break; }
-                        if (const char* e = getenv("POISMF_B200_TOPN_SAMPLE")) S = std::max(1, std::min(atoi(e), 8));
-                        o.cand_regions = (int)chunks;
-                        // (4x the even share: a user's candidates may cluster in a few tiles)
-                        o.cand_cap = std::min(tc::CAND_CAP, tc::CAND_SLACK * tc::CAND_CAP / (int)chunks);
-                        o.ngroups = ((ntiles + S - 1) / S) * (tc::TN / tc::GROUP);
-                    }
-                    const size_t pipe_smem = tc::pipe_smem_bytes(kpad);
-                    const int pipe_stages = tc::pipe_stages(kpad);
-                    if (piped) {
-                        CK(cudaFuncSetAttribute(tc::score_pipe_tf32_kernel<tc::MODE_GROUPMAX>,
-                                                cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pipe_smem));
-                        CK(cudaFuncSetAttribute(tc::score_pipe_tf32_kernel<tc::MODE_EMIT>,
-                                                cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pipe_smem));
-                        tc::score_pipe_tf32_kernel<tc::MODE_GROUPMAX><<<dim3(chunks, ut), tc::PIPE_THREADS, pipe_smem>>>(
-                            mapA, mapB, (int)m, n, kpad, S, pipe_stages, o);
-                    } else
-                        tc::score_tiles_tf32_kernel<tc::MODE_GROUPMAX><<<tgrid, 128, (size_t)kpad * 1024>>>(
-                            (const float*)dAsel, (int)m, (const float*)dB, n, ldf, kpad, o);
-                    LAUNCHED();
-                    tc::select_threshold_kernel<<<(unsigned)m, 256>>>(gmax, o.ngroups, M_cand, tau);
-                    LAUNCHED();
-                    CK(cudaMemsetAsync(cand_cnt, 0, m * o.cand_regions * sizeof(int)));
-                    if (piped)
-                        tc::score_pipe_tf32_kernel<tc::MODE_EMIT><<<dim3(chunks, ut), tc::PIPE_THREADS, pipe_smem>>>(
-                            mapA, mapB, (int)m, n, kpad, 1, pipe_stages, o);
-                    else
-                        tc::score_tiles_tf32_kernel<tc::MODE_EMIT><<<tgrid, 128, (size_t)kpad * 1024>>>(
-                            (const float*)dAsel, (int)m, (const float*)dB, n, ldf, kpad, o);
-                    LAUNCHED();
-                    tc::sort_candidates_kernel<<<(unsigned)m, 512>>>(cand_sc, cand_id, cand_cnt, o.cand_regions, o.cand_cap,
-                                                                     top_sc, top_id, d_ovf);
-                    LAUNCHED();
-                    tc::rescore_select_kernel<<<(unsigned)m, 128>>>((const float*)dAsel, (const float*)dB, k, ldf, top_id,
-                                                                    top_sc, (size_t)tc::CAND_TOP, M_cand, 0, (int)n_top,
-                                                                    4e-3f, d_out_ids, d_out_sc, d_flag);
-                    LAUNCHED();
-                    CK(cudaGetLastError());
-                    mark("batch kernels");
-                    // results straight into the caller's arrays when the element types agree (they do for the
-                    // reference's size_t / float build); staged through page-locked blocks when those are pageable
-                    hfl.resize(m); hov.resize(m);
-                    if (sizeof(IX) == sizeof(long long)) {
-                        CK(Stager::get().d2h((void*)(outp_ix + u0 * n_top), d_out_ids, m * n_top * sizeof(long long), 0));
-                    } else {
-                        hid.resize(m * n_top);
-                        CK(cudaMemcpy(hid.data(), d_out_ids, m * n_top * sizeof(long long), cudaMemcpyDeviceToHost));
-                        for (size_t i = 0; i < m * n_top; i++) outp_ix[u0 * n_top + i] = (IX)hid[i];
-                    }
-                    if (outp_score) {
-                        if (std::is_same<real, float>::value) {
-                            CK(Stager::get().d2h((void*)(outp_score + u0 * n_top), d_out_sc, m * n_top * sizeof(float), 0));
-                        } else {
-                            hsc.resize(m * n_top);
-                            CK(cudaMemcpy(hsc.data(), d_out_sc, m * n_top * sizeof(float), cudaMemcpyDeviceToHost));
-                            for (size_t i = 0; i < m * n_top; i++) outp_score[u0 * n_top + i] = (real)hsc[i];
-                        }
-                    }
-                    CK(cudaMemcpy(hfl.data(), d_flag, m * sizeof(int), cudaMemcpyDeviceToHost));
-                    CK(cudaMemcpy(hov.data(), d_ovf, m * sizeof(int), cudaMemcpyDeviceToHost));
-                    for (size_t u = 0; u < m; u++) if (hfl[u] || hov[u]) redo.push_back(u0 + u);
-                    g_topn_stats[0] += m;
-                    mark("batch results down");
-                }
-                return 0;
-            };
-            const int frc = fused();
-            if (frc) cudaDeviceSynchronize();
-            for (void* q : mine) dfree(q);
-            mark("release");
-            return frc;
-        }
-        if (use_tc) {
-            CK(dmalloc(&d_out_ids, chunk * n_top * sizeof(long long)));
-            CK(dmalloc(&d_out_sc, chunk * n_top * sizeof(float)));
-            CK(dmalloc(&d_flag, chunk * sizeof(int)));
-            CK(cudaFuncSetAttribute(tc::score_tiles_tf32_kernel<tc::MODE_SCORES>,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, kpad * 1024));
-        }
-        CK(dmalloc(&dAsel, chunk * pitch));
-        CK(dmalloc(&sc_in, chunk * n * sizeof(real))); CK(dmalloc(&sc_out, chunk * n * sizeof(real)));
-        CK(dmalloc(&id_in, chunk * n * sizeof(int))); CK(dmalloc(&id_out, chunk * n * sizeof(int)));
-        CK(dmalloc(&seg, (chunk + 1) * sizeof(int)));
-        CK(dmalloc(&dusers, chunk * sizeof(long long)));
-        std::vector<int> h_seg(chunk + 1);
-        for (size_t u = 0; u <= chunk; u++) h_seg[u] = (int)(u * n);
-        if (chunk * n > (size_t)INT32_MAX) return fail("topN: chunk too large");
-        CK(cudaMemcpy(seg, h_seg.data(), (chunk + 1) * sizeof(int), cudaMemcpyHostToDevice));
-        size_t n_excl_total = 0;
-        if (excl_ptr && excl_ix) {
-            n_excl_total = (size_t)excl_ptr[n_users];
-            CK(dmalloc(&dexp, (n_users + 1) * sizeof(IX)));
-            CK(dmalloc(&dexi, std::max<size_t>(n_excl_total, 1) * sizeof(IX)));
-            CK(cudaMemcpy(dexp, excl_ptr, (n_users + 1) * sizeof(IX), cudaMemcpyHostToDevice));
-            CK(Stager::get().h2d(dexi, excl_ix, n_excl_total * sizeof(IX), 0));
-            if (const int bad = excl_ids_ok(dexi + (size_t)excl_ptr[0], n_excl_total - (size_t)excl_ptr[0])) return bad;
-        }
-        size_t tmp_bytes = 0;
-        CK(cub::DeviceSegmentedRadixSort::SortPairsDescending(nullptr, tmp_bytes, sc_in, sc_out, id_in, id_out,
-                                                              (int)(chunk * n), (int)chunk, seg, seg + 1));
-        CK(dmalloc(&tmp, std::max<size_t>(tmp_bytes, 1)));
-        for (size_t u0 = 0; u0 < n_users; u0 += chunk) {
-            const size_t m = std::min(chunk, n_users - u0);
-            std::vector<long long> hu(m);
-            for (size_t u = 0; u < m; u++) hu[u] = A_is_single_vector ? 0 : (user_ix ? (long long)user_ix[u0 + u] : (long long)(u0 + u));
-            CK(cudaMemcpy(dusers, hu.data(), m * sizeof(long long), cudaMemcpyHostToDevice));
-            gather_rows_kernel<real><<<(int)std::min<size_t>((m * ldf + 255) / 256, 4096), 256>>>(dA, dusers, (int)m, ldf, dAsel);
-            LAUNCHED();
-            if (use_tc) {
-                dim3 tgrid((unsigned)((n + tc::TN - 1) / tc::TN), (unsigned)((m + tc::TM - 1) / tc::TM));
+            CK(mem.alloc(&dAsel, fchunk * pitch));
+            CK(mem.alloc(&dusers, fchunk * sizeof(long long)));
+            CK(mem.alloc(&gmax, fchunk * ngroups_alloc * sizeof(float)));
+            CK(mem.alloc(&tau, fchunk * sizeof(float)));
+            CK(mem.alloc(&cand_sc, fchunk * tc::CAND_SLACK * tc::CAND_CAP * sizeof(float)));
+            CK(mem.alloc(&cand_id, fchunk * tc::CAND_SLACK * tc::CAND_CAP * sizeof(int)));
+            CK(mem.alloc(&cand_cnt, fchunk * 64 * sizeof(int)));      // [user][region], regions <= 64
+            CK(mem.alloc(&top_sc, fchunk * tc::CAND_TOP * sizeof(float)));
+            CK(mem.alloc(&top_id, fchunk * tc::CAND_TOP * sizeof(int)));
+            CK(mem.alloc(&d_ovf, fchunk * sizeof(int)));
+            CK(mem.alloc(&d_out_ids, fchunk * n_top * sizeof(long long)));
+            CK(mem.alloc(&d_out_sc, fchunk * n_top * sizeof(float)));
+            CK(mem.alloc(&d_flag, fchunk * sizeof(int)));
+            if (have_excl) CK(mem.alloc(&bits, fchunk * words * sizeof(uint32_t)));
+            mark("work arrays");
+            // The threshold pass visits every S-th item tile only: the M-th largest group maximum of a SAMPLE of
+            // the items is a lower bound of the one over all items, so every wanted item still passes tau; about
+            // S M items do (instead of M), which the candidate slots must hold (S M <= 1/4 of them)
+            int S = 1;
+            for (int c : {4, 2})
+                if (ntiles >= (size_t)c * M_cand && (size_t)c * M_cand <= (size_t)tc::CAND_CAP / 4) { S = c; break; }
+            const size_t pipe_smem = tc::pipe_smem_bytes(kpad);
+            const int pipe_stages = tc::pipe_stages(kpad);
+            CK(cudaFuncSetAttribute(tc::score_pipe_tf32_kernel<tc::MODE_GROUPMAX>,
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pipe_smem));
+            CK(cudaFuncSetAttribute(tc::score_pipe_tf32_kernel<tc::MODE_EMIT>,
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pipe_smem));
+            int num_sms = 148, dev = 0;
+            CK(cudaGetDevice(&dev));
+            CK(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
+            std::vector<long long> hid;
+            std::vector<float> hsc;
+            std::vector<int> hfl, hov;
+            for (size_t u0 = 0; u0 < n_users; u0 += fchunk) {
+                const size_t m = std::min(fchunk, n_users - u0);
+                if (gather_users(dA, ldf, user_ix, u0, m, dusers, dAsel)) return 1;
+                CUtensorMap mapA;          // the chunk's rows: those beyond m read as zeros
+                if (tc::make_operand_map(&mapA, (const float*)dAsel, m, ldf))
+                    return fail("topN: cannot encode the tensor map of %zu user rows", m);
                 tc::TileOut o = {};
-                o.scores = (float*)sc_in; o.ids = id_in;
-                tc::score_tiles_tf32_kernel<tc::MODE_SCORES><<<tgrid, 128, (size_t)kpad * 1024>>>(
-                    (const float*)dAsel, (int)m, (const float*)dB, n, ldf, kpad, o);
-            } else {
-                dim3 grid((unsigned)std::min<size_t>((n + 255) / 256, 1024), (unsigned)m);
-                score_items_kernel<real><<<grid, 256, (size_t)ldf * sizeof(real)>>>(dAsel, dB, n, k, ldf, sc_in, id_in);
-            }
-            LAUNCHED();
-            if (dexp) {
-                dim3 g2(8, (unsigned)m);
-                mask_excluded_kernel<real, IX><<<g2, 256>>>(sc_in, n, dexp, dexi, u0);
+                if (have_excl) {
+                    CK(cudaMemsetAsync(bits, 0, m * words * sizeof(uint32_t)));
+                    tc::exclusion_bitmap_kernel<IX><<<dim3(4, (unsigned)m), 128>>>(bits, words, dexp, dexi, u0, n);
+                    LAUNCHED();
+                    o.excl_bits = bits; o.excl_words = words;
+                }
+                o.gmax = gmax; o.tau = tau;
+                o.cand_sc = cand_sc; o.cand_id = cand_id; o.cand_cnt = cand_cnt;
+                o.ngroups = ((ntiles + S - 1) / S) * (tc::TN / tc::GROUP);
+                const unsigned ut = (unsigned)((m + tc::PIPE_UT * tc::TM - 1) / (tc::PIPE_UT * tc::TM));   // CTAs along the users
+                // one CTA per SM (shared memory), every CTA the same run of item tiles: the split of the items
+                // that fills whole waves best (fewest chunks among the best: the A tiles load once per CTA)
+                unsigned chunks = 1;
+                {
+                    double best = 0;
+                    const unsigned cmax = (unsigned)std::max<size_t>(1, std::min<size_t>(ntiles / 32, 64));
+                    for (unsigned c = 1; c <= cmax; c++) {
+                        const size_t ctas = (size_t)c * ut, waves = (ctas + num_sms - 1) / num_sms;
+                        const double eff = (double)ctas / (double)(waves * num_sms);
+                        if (eff > best + 0.02) { best = eff; chunks = c; }
+                    }
+                }
+                o.cand_regions = (int)chunks;
+                // (4x the even share: a user's candidates may cluster in a few tiles)
+                o.cand_cap = std::min(tc::CAND_CAP, tc::CAND_SLACK * tc::CAND_CAP / (int)chunks);
+                tc::score_pipe_tf32_kernel<tc::MODE_GROUPMAX><<<dim3(chunks, ut), tc::PIPE_THREADS, pipe_smem>>>(
+                    mapA, mapB, (int)m, n, kpad, S, pipe_stages, o);
                 LAUNCHED();
-            }
-            CK(cudaGetLastError());
-            CK(cub::DeviceSegmentedRadixSort::SortPairsDescending(tmp, tmp_bytes, sc_in, sc_out, id_in, id_out,
-                                                                  (int)(m * n), (int)m, seg, seg + 1));
-            LAUNCHED();
-            if (use_tc) {
-                // exact FP32 re-score of the best M TF32 candidates, final order, and the proof that
-                // nothing outside the candidates can reach the top n_top
-                tc::rescore_select_kernel<<<(unsigned)m, 128>>>((const float*)dAsel, (const float*)dB, k, ldf, id_out,
-                                                                (const float*)sc_out, n, M_cand, M_cand >= (int)n ? 1 : 0,
-                                                                (int)n_top, 4e-3f, d_out_ids, d_out_sc, d_flag);
+                tc::select_threshold_kernel<<<(unsigned)m, 256>>>(gmax, o.ngroups, M_cand, tau);
+                LAUNCHED();
+                CK(cudaMemsetAsync(cand_cnt, 0, m * o.cand_regions * sizeof(int)));
+                tc::score_pipe_tf32_kernel<tc::MODE_EMIT><<<dim3(chunks, ut), tc::PIPE_THREADS, pipe_smem>>>(
+                    mapA, mapB, (int)m, n, kpad, 1, pipe_stages, o);
+                LAUNCHED();
+                tc::sort_candidates_kernel<<<(unsigned)m, 512>>>(cand_sc, cand_id, cand_cnt, o.cand_regions, o.cand_cap,
+                                                                 top_sc, top_id, d_ovf);
+                LAUNCHED();
+                tc::rescore_select_kernel<<<(unsigned)m, 128>>>((const float*)dAsel, (const float*)dB, k, ldf, top_id,
+                                                                top_sc, (size_t)tc::CAND_TOP, M_cand, 0, (int)n_top,
+                                                                4e-3f, d_out_ids, d_out_sc, d_flag);
                 LAUNCHED();
                 CK(cudaGetLastError());
-                std::vector<long long> hid(m * n_top); std::vector<float> hsc(m * n_top); std::vector<int> hfl(m);
-                CK(cudaMemcpy(hid.data(), d_out_ids, m * n_top * sizeof(long long), cudaMemcpyDeviceToHost));
-                CK(cudaMemcpy(hsc.data(), d_out_sc, m * n_top * sizeof(float), cudaMemcpyDeviceToHost));
+                mark("batch kernels");
+                // results straight into the caller's arrays when the element types agree (they do for the
+                // reference's size_t / float build); staged through page-locked blocks when those are pageable
+                hfl.resize(m); hov.resize(m);
+                if (sizeof(IX) == sizeof(long long)) {
+                    CK(Stager::get().d2h((void*)(outp_ix + u0 * n_top), d_out_ids, m * n_top * sizeof(long long), 0));
+                } else {
+                    hid.resize(m * n_top);
+                    CK(cudaMemcpy(hid.data(), d_out_ids, m * n_top * sizeof(long long), cudaMemcpyDeviceToHost));
+                    for (size_t i = 0; i < m * n_top; i++) outp_ix[u0 * n_top + i] = (IX)hid[i];
+                }
+                if (outp_score) {
+                    if (std::is_same<real, float>::value) {
+                        CK(Stager::get().d2h((void*)(outp_score + u0 * n_top), d_out_sc, m * n_top * sizeof(float), 0));
+                    } else {
+                        hsc.resize(m * n_top);
+                        CK(cudaMemcpy(hsc.data(), d_out_sc, m * n_top * sizeof(float), cudaMemcpyDeviceToHost));
+                        for (size_t i = 0; i < m * n_top; i++) outp_score[u0 * n_top + i] = (real)hsc[i];
+                    }
+                }
                 CK(cudaMemcpy(hfl.data(), d_flag, m * sizeof(int), cudaMemcpyDeviceToHost));
-                for (size_t i = 0; i < m * n_top; i++) outp_ix[u0 * n_top + i] = (IX)hid[i];
-                if (outp_score) for (size_t i = 0; i < m * n_top; i++) outp_score[u0 * n_top + i] = (real)hsc[i];
-                for (size_t u = 0; u < m; u++) if (hfl[u]) redo.push_back(u0 + u);
+                CK(cudaMemcpy(hov.data(), d_ovf, m * sizeof(int), cudaMemcpyDeviceToHost));
+                for (size_t u = 0; u < m; u++) if (hfl[u] || hov[u]) redo.push_back(u0 + u);
                 g_topn_stats[0] += m;
-                continue;
+                mark("batch results down");
             }
-            CK(cudaMemcpy2D(h_ids.data(), n_top * sizeof(int), id_out, n * sizeof(int), n_top * sizeof(int), m, cudaMemcpyDeviceToHost));
-            CK(cudaMemcpy2D(h_sc.data(), n_top * sizeof(real), sc_out, n * sizeof(real), n_top * sizeof(real), m, cudaMemcpyDeviceToHost));
-            for (size_t i = 0; i < m * n_top; i++) outp_ix[u0 * n_top + i] = (IX)h_ids[i];
-            if (outp_score) memcpy(outp_score + u0 * n_top, h_sc.data(), m * n_top * sizeof(real));
-        }
-        return 0;
-    };
-    int rc = body();
-    if (rc) cudaDeviceSynchronize();
-    if (!B_resident) dfree(dB);
-    if (!A_resident) dfree(dA);
-    dfree(dAsel); dfree(sc_in); dfree(sc_out); dfree(id_in);
-    dfree(id_out); dfree(seg); dfree(dusers); dfree(dexp); dfree(dexi); dfree(tmp);
-    dfree(d_out_ids); dfree(d_out_sc); dfree(d_flag); dfree(d_neg);
-    // users whose candidate set could not be proven complete: exact scorer, one call for all of them
-    if (!rc && !redo.empty()) {
-        const size_t R = redo.size();
-        g_topn_stats[1] += R;
-        std::vector<IX> ru(R), rptr(R + 1, 0), rix;
-        for (size_t i = 0; i < R; i++) {
-            const size_t u = redo[i];
-            ru[i] = A_is_single_vector ? (IX)0 : (user_ix ? user_ix[u] : (IX)u);
-            if (excl_ptr && excl_ix) {
-                for (size_t t = (size_t)excl_ptr[u]; t < (size_t)excl_ptr[u + 1]; t++) rix.push_back(excl_ix[t]);
+        } else {
+            // ---- TF32 or exact scores of every item, then a segmented sort of each user's n scores ----
+            // users per chunk: bound the score matrix to ~1 GiB
+            size_t chunk = std::max<size_t>(1, std::min<size_t>(n_users, ((size_t)1 << 28) / std::max<size_t>(n, 1)));
+            chunk = std::min<size_t>(chunk, 65535);
+            if (chunk * n > (size_t)INT32_MAX) return fail("topN: chunk too large");
+            real *dAsel = nullptr, *sc_in = nullptr, *sc_out = nullptr;
+            int *id_in = nullptr, *id_out = nullptr, *seg = nullptr;
+            long long* dusers = nullptr;
+            void* tmp = nullptr;
+            CK(mem.alloc(&dAsel, chunk * pitch));
+            CK(mem.alloc(&sc_in, chunk * n * sizeof(real))); CK(mem.alloc(&sc_out, chunk * n * sizeof(real)));
+            CK(mem.alloc(&id_in, chunk * n * sizeof(int))); CK(mem.alloc(&id_out, chunk * n * sizeof(int)));
+            CK(mem.alloc(&seg, (chunk + 1) * sizeof(int)));
+            CK(mem.alloc(&dusers, chunk * sizeof(long long)));
+            std::vector<int> h_seg(chunk + 1);
+            for (size_t u = 0; u <= chunk; u++) h_seg[u] = (int)(u * n);
+            CK(cudaMemcpy(seg, h_seg.data(), (chunk + 1) * sizeof(int), cudaMemcpyHostToDevice));
+            size_t tmp_bytes = 0;
+            CK(cub::DeviceSegmentedRadixSort::SortPairsDescending(nullptr, tmp_bytes, sc_in, sc_out, id_in, id_out,
+                                                                  (int)(chunk * n), (int)chunk, seg, seg + 1));
+            CK(mem.alloc(&tmp, std::max<size_t>(tmp_bytes, 1)));
+            long long* d_out_ids = nullptr;
+            float* d_out_sc = nullptr;
+            int* d_flag = nullptr;
+            if (use_tc) {
+                CK(mem.alloc(&d_out_ids, chunk * n_top * sizeof(long long)));
+                CK(mem.alloc(&d_out_sc, chunk * n_top * sizeof(float)));
+                CK(mem.alloc(&d_flag, chunk * sizeof(int)));
+                CK(cudaFuncSetAttribute(tc::score_tiles_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kpad * 1024));
             }
-            rptr[i + 1] = (IX)rix.size();
+            std::vector<long long> hid;
+            std::vector<int> h_ids, hfl;
+            std::vector<real> h_sc;
+            std::vector<float> hsc;
+            for (size_t u0 = 0; u0 < n_users; u0 += chunk) {
+                const size_t m = std::min(chunk, n_users - u0);
+                if (gather_users(dA, ldf, user_ix, u0, m, dusers, dAsel)) return 1;
+                if (use_tc) {
+                    const dim3 tgrid((unsigned)ntiles, (unsigned)((m + tc::TM - 1) / tc::TM));
+                    tc::score_tiles_tf32_kernel<<<tgrid, 128, (size_t)kpad * 1024>>>((const float*)dAsel, (int)m,
+                                                                                   (const float*)dB, n, ldf, kpad,
+                                                                                   (float*)sc_in, id_in);
+                } else {
+                    dim3 grid((unsigned)std::min<size_t>((n + 255) / 256, 1024), (unsigned)m);
+                    score_items_kernel<real><<<grid, 256, (size_t)ldf * sizeof(real)>>>(dAsel, dB, n, k, ldf, sc_in, id_in);
+                }
+                LAUNCHED();
+                if (have_excl) {
+                    mask_excluded_kernel<real, IX><<<dim3(8, (unsigned)m), 256>>>(sc_in, n, dexp, dexi, u0);
+                    LAUNCHED();
+                }
+                CK(cudaGetLastError());
+                CK(cub::DeviceSegmentedRadixSort::SortPairsDescending(tmp, tmp_bytes, sc_in, sc_out, id_in, id_out,
+                                                                      (int)(m * n), (int)m, seg, seg + 1));
+                LAUNCHED();
+                if (use_tc) {
+                    // exact FP32 re-score of the best M TF32 candidates, final order, and the proof that nothing
+                    // outside the candidates can reach the top n_top
+                    tc::rescore_select_kernel<<<(unsigned)m, 128>>>((const float*)dAsel, (const float*)dB, k, ldf, id_out,
+                                                                    (const float*)sc_out, n, M_cand, M_cand >= (int)n ? 1 : 0,
+                                                                    (int)n_top, 4e-3f, d_out_ids, d_out_sc, d_flag);
+                    LAUNCHED();
+                    CK(cudaGetLastError());
+                    hid.resize(m * n_top); hsc.resize(m * n_top); hfl.resize(m);
+                    CK(cudaMemcpy(hid.data(), d_out_ids, m * n_top * sizeof(long long), cudaMemcpyDeviceToHost));
+                    CK(cudaMemcpy(hsc.data(), d_out_sc, m * n_top * sizeof(float), cudaMemcpyDeviceToHost));
+                    CK(cudaMemcpy(hfl.data(), d_flag, m * sizeof(int), cudaMemcpyDeviceToHost));
+                    for (size_t i = 0; i < m * n_top; i++) outp_ix[u0 * n_top + i] = (IX)hid[i];
+                    if (outp_score) for (size_t i = 0; i < m * n_top; i++) outp_score[u0 * n_top + i] = (real)hsc[i];
+                    for (size_t u = 0; u < m; u++) if (hfl[u]) redo.push_back(u0 + u);
+                    g_topn_stats[0] += m;
+                    continue;
+                }
+                h_ids.resize(m * n_top); h_sc.resize(m * n_top);
+                CK(cudaMemcpy2D(h_ids.data(), n_top * sizeof(int), id_out, n * sizeof(int), n_top * sizeof(int), m, cudaMemcpyDeviceToHost));
+                CK(cudaMemcpy2D(h_sc.data(), n_top * sizeof(real), sc_out, n * sizeof(real), n_top * sizeof(real), m, cudaMemcpyDeviceToHost));
+                for (size_t i = 0; i < m * n_top; i++) outp_ix[u0 * n_top + i] = (IX)h_ids[i];
+                if (outp_score) memcpy(outp_score + u0 * n_top, h_sc.data(), m * n_top * sizeof(real));
+            }
         }
-        std::vector<IX> rout(R * n_top);
-        std::vector<real> rsc(outp_score ? R * n_top : 0);
-        rc = topn_batch_impl<real, IX>(A, B, k, A_is_single_vector ? nullptr : ru.data(), R, dimA,
-                                       (excl_ptr && excl_ix) ? rptr.data() : nullptr,
-                                       (excl_ptr && excl_ix) ? (rix.empty() ? rptr.data() : rix.data()) : nullptr,
-                                       rout.data(), outp_score ? rsc.data() : nullptr, n_top, n, A_is_single_vector, false, rf);
-        for (size_t i = 0; i < R && !rc; i++) {
-            memcpy(outp_ix + redo[i] * n_top, &rout[i * n_top], n_top * sizeof(IX));
-            if (outp_score) memcpy(outp_score + redo[i] * n_top, &rsc[i * n_top], n_top * sizeof(real));
-        }
+        mem.settled = true;
     }
-    return rc;
+    mark("release");
+    // users whose candidate set could not be proven complete: exact scorer, one call for all of them
+    if (redo.empty()) return 0;
+    const size_t R = redo.size();
+    g_topn_stats[1] += R;
+    std::vector<IX> ru(R), rptr(R + 1, 0), rix;
+    for (size_t i = 0; i < R; i++) {
+        const size_t u = redo[i];
+        ru[i] = user_ix ? user_ix[u] : (IX)u;
+        if (have_excl)
+            for (size_t t = (size_t)excl_ptr[u]; t < (size_t)excl_ptr[u + 1]; t++) rix.push_back(excl_ix[t]);
+        rptr[i + 1] = (IX)rix.size();
+    }
+    std::vector<IX> rout(R * n_top);
+    std::vector<real> rsc(outp_score ? R * n_top : 0);
+    const int rc = topn_batch_impl<real, IX>(A, B, k, ru.data(), R, dimA, have_excl ? rptr.data() : nullptr,
+                                             have_excl ? (rix.empty() ? rptr.data() : rix.data()) : nullptr,
+                                             rout.data(), outp_score ? rsc.data() : nullptr, n_top, n, false, rf);
+    if (rc) return rc;
+    for (size_t i = 0; i < R; i++) {
+        memcpy(outp_ix + redo[i] * n_top, &rout[i * n_top], n_top * sizeof(IX));
+        if (outp_score) memcpy(outp_score + redo[i] * n_top, &rsc[i * n_top], n_top * sizeof(real));
+    }
+    return 0;
 }
 
 // Batched top-N over per-user candidate lists (topn_include.cuh).  Lists up to `cap` items are ranked in
@@ -2281,136 +2290,110 @@ static int topn_include_impl(const real* A, const real* B, int k, const IX* user
         u0 = c.u1;
     }
 
+    DeviceBlocks mem;
     real *dB = nullptr, *dA = nullptr, *dAsel = nullptr, *d_sc = nullptr;
     IX *d_ix = nullptr, *d_out = nullptr;
     long long *dusers = nullptr, *dptr = nullptr;
-    int *d_su = nullptr, *d_lu = nullptr, *d_seg = nullptr, *d_bad = nullptr;
+    int *d_su = nullptr, *d_lu = nullptr, *d_seg = nullptr;
     uint32_t *id0 = nullptr, *id1 = nullptr;
     K *key0 = nullptr, *key1 = nullptr;
     void* tmp = nullptr;
-    bool B_resident = false, A_resident = false;
-    auto body = [&]() -> int {
-        if (rf) {
-            if (rf->ldf != ldf) return fail("topN_include: resident factors have another row pitch");
-            dB = (real*)rf->B; dA = (real*)rf->A;
-            B_resident = A_resident = true;
-        } else {
-            bool dummy = false;
-            if (upload_rows<real>(&dB, B, n, k, ldf, &B_resident, true)) return 1;
-            if (upload_rows<real>(&dA, A, dimA, k, ldf, &dummy, false)) return 1;
-        }
-        CK(dmalloc(&dAsel, max_m * pitch));
-        CK(dmalloc(&dusers, max_m * sizeof(long long)));
-        CK(dmalloc(&dptr, (max_m + 1) * sizeof(long long)));
-        CK(dmalloc(&d_su, max_m * sizeof(int)));
-        CK(dmalloc(&d_ix, std::max<size_t>(max_list, 1) * sizeof(IX)));
-        CK(dmalloc(&d_out, max_m * n_top * sizeof(IX)));
-        if (outp_score) CK(dmalloc(&d_sc, max_m * n_top * sizeof(real)));
-        CK(dmalloc(&d_bad, sizeof(int)));
-        int end_bit = 1;                                    // bits of the largest item id
-        while (end_bit < 32 && ((n - 1) >> end_bit)) end_bit++;
-        size_t tmp_bytes = 0;
-        if (max_long) {
-            CK(dmalloc(&d_lu, max_long * sizeof(int)));
-            CK(dmalloc(&d_seg, (max_long + 1) * sizeof(int)));
-            CK(dmalloc(&id0, max_long_total * sizeof(uint32_t))); CK(dmalloc(&id1, max_long_total * sizeof(uint32_t)));
-            CK(dmalloc(&key0, max_long_total * sizeof(K))); CK(dmalloc(&key1, max_long_total * sizeof(K)));
-            size_t t1 = 0, t2 = 0;
-            CK(cub::DeviceSegmentedRadixSort::SortPairs(nullptr, t1, id0, id1, key0, key1, (int)max_long_total,
-                                                        (int)max_long, d_seg, d_seg + 1, 0, end_bit));
-            CK(cub::DeviceSegmentedRadixSort::SortPairsDescending(nullptr, t2, key1, key0, id1, id0,
-                                                                  (int)max_long_total, (int)max_long, d_seg, d_seg + 1));
-            tmp_bytes = std::max(t1, t2);
-            CK(dmalloc(&tmp, std::max<size_t>(tmp_bytes, 1)));
-        }
-        // -> 0 ok, 2 a listed id outside [0, n), 1 CUDA error
-        auto upload_lists = [&](const Chunk& c, bool check) -> int {
-            const size_t off = (size_t)incl_ptr[c.u0], cnt = (size_t)incl_ptr[c.u1] - off;
-            CK(Stager::get().h2d(d_ix, incl_ix + off, cnt * sizeof(IX), 0));
-            if (!check) return 0;
-            int bad = 0;
-            CK(cudaMemsetAsync(d_bad, 0, sizeof(int)));
-            tc::any_id_out_of_range_kernel<IX><<<592, 256>>>(d_ix, cnt, n, d_bad);
-            LAUNCHED();
-            CK(cudaMemcpy(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost));
-            return bad ? 2 : 0;
-        };
-        // with several chunks every list is checked before the first result is written, and uploaded again
-        if (chunks.size() > 1)
-            for (const Chunk& c : chunks)
-                if (const int bad = upload_lists(c, true)) return bad;
-        std::vector<long long> hu, hp;
-        std::vector<int> hsu, hlu, hseg;
-        std::vector<std::pair<int, int>> classes;           // (capacity, users) of the path (a) launches
-        for (const Chunk& c : chunks) {
-            const size_t m = c.u1 - c.u0, off = (size_t)incl_ptr[c.u0];
-            if (const int bad = upload_lists(c, chunks.size() == 1)) return bad;
-            hu.resize(m); hp.resize(m + 1); hsu.clear(); classes.clear(); hlu.clear(); hseg.assign(1, 0);
-            for (size_t i = 0; i < m; i++) {
-                const size_t u = c.u0 + i, len = len_of(u);
-                hu[i] = user_ix ? (long long)user_ix[u] : (long long)u;
-                hp[i] = (long long)((size_t)incl_ptr[u] - off);
-                if (len > (size_t)cap) { hlu.push_back((int)i); hseg.push_back(hseg.back() + (int)len); }
-            }
-            // path (a) by length class, so that one long list does not size every CTA's shared memory: lists up
-            // to 4 K items share one launch (its 4 CTAs per SM, the register bound, fit in shared memory), longer
-            // ones go by power of two up to `cap`
-            for (size_t lo = 0, P = (size_t)std::min(cap, 4096);; lo = P, P <<= 1) {
-                const size_t start = hsu.size();
-                for (size_t i = 0; i < m; i++) {
-                    const size_t len = len_of(c.u0 + i);
-                    if (len > lo && len <= P) hsu.push_back((int)i);
-                }
-                if (hsu.size() > start) classes.push_back({(int)P, (int)(hsu.size() - start)});
-                if (P >= (size_t)cap) break;
-            }
-            hp[m] = (long long)((size_t)incl_ptr[c.u1] - off);
-            CK(cudaMemcpy(dusers, hu.data(), m * sizeof(long long), cudaMemcpyHostToDevice));
-            CK(cudaMemcpy(dptr, hp.data(), (m + 1) * sizeof(long long), cudaMemcpyHostToDevice));
-            gather_rows_kernel<real><<<(int)std::min<size_t>((m * ldf + 255) / 256, 4096), 256>>>(dA, dusers, (int)m, ldf, dAsel);
-            LAUNCHED();
-            if (!hsu.empty()) CK(cudaMemcpy(d_su, hsu.data(), hsu.size() * sizeof(int), cudaMemcpyHostToDevice));
-            for (size_t q = 0, first = 0; q < classes.size(); first += classes[q].second, q++) {
-                const size_t smem = rowb + (size_t)classes[q].first * entry;
-                CK(cudaFuncSetAttribute(incl::include_select_smem_kernel<real, IX>,
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                incl::include_select_smem_kernel<real, IX><<<(unsigned)classes[q].second, incl::SMEM_THREADS, smem>>>(
-                    dAsel, dB, k, ldf, dptr, d_ix, d_su + first, classes[q].first, (int)n_top, d_out, d_sc);
-                LAUNCHED();
-            }
-            if (!hlu.empty()) {
-                const int nl = (int)hlu.size(), total = hseg.back();
-                CK(cudaMemcpy(d_lu, hlu.data(), nl * sizeof(int), cudaMemcpyHostToDevice));
-                CK(cudaMemcpy(d_seg, hseg.data(), (nl + 1) * sizeof(int), cudaMemcpyHostToDevice));
-                CK(cudaFuncSetAttribute(incl::include_score_long_kernel<real, IX>,
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rowb));
-                incl::include_score_long_kernel<real, IX><<<dim3(64, (unsigned)nl), 256, rowb>>>(
-                    dAsel, dB, k, ldf, dptr, d_ix, d_lu, d_seg, id0, key0);
-                LAUNCHED();
-                // by item id, then stably by score: ties come out by ascending id
-                CK(cub::DeviceSegmentedRadixSort::SortPairs(tmp, tmp_bytes, id0, id1, key0, key1, total, nl,
-                                                            d_seg, d_seg + 1, 0, end_bit));
-                CK(cub::DeviceSegmentedRadixSort::SortPairsDescending(tmp, tmp_bytes, key1, key0, id1, id0, total, nl,
-                                                                      d_seg, d_seg + 1));
-                LAUNCHED(); LAUNCHED();
-                incl::include_emit_long_kernel<real, IX><<<(unsigned)nl, 128>>>(d_lu, d_seg, id0, key0, (int)n_top,
-                                                                                 d_out, d_sc);
-                LAUNCHED();
-            }
-            CK(cudaGetLastError());
-            CK(Stager::get().d2h(outp_ix + c.u0 * n_top, d_out, m * n_top * sizeof(IX), 0));
-            if (outp_score) CK(Stager::get().d2h(outp_score + c.u0 * n_top, d_sc, m * n_top * sizeof(real), 0));
-            CK(cudaStreamSynchronize(0));
-        }
-        return 0;
+    if (factors_on_device(rf, A, dimA, B, n, k, ldf, mem, &dA, &dB, "topN_include")) return 1;
+    CK(mem.alloc(&dAsel, max_m * pitch));
+    CK(mem.alloc(&dusers, max_m * sizeof(long long)));
+    CK(mem.alloc(&dptr, (max_m + 1) * sizeof(long long)));
+    CK(mem.alloc(&d_su, max_m * sizeof(int)));
+    CK(mem.alloc(&d_ix, std::max<size_t>(max_list, 1) * sizeof(IX)));
+    CK(mem.alloc(&d_out, max_m * n_top * sizeof(IX)));
+    if (outp_score) CK(mem.alloc(&d_sc, max_m * n_top * sizeof(real)));
+    int end_bit = 1;                                        // bits of the largest item id
+    while (end_bit < 32 && ((n - 1) >> end_bit)) end_bit++;
+    size_t tmp_bytes = 0;
+    if (max_long) {
+        CK(mem.alloc(&d_lu, max_long * sizeof(int)));
+        CK(mem.alloc(&d_seg, (max_long + 1) * sizeof(int)));
+        CK(mem.alloc(&id0, max_long_total * sizeof(uint32_t))); CK(mem.alloc(&id1, max_long_total * sizeof(uint32_t)));
+        CK(mem.alloc(&key0, max_long_total * sizeof(K))); CK(mem.alloc(&key1, max_long_total * sizeof(K)));
+        size_t t1 = 0, t2 = 0;
+        CK(cub::DeviceSegmentedRadixSort::SortPairs(nullptr, t1, id0, id1, key0, key1, (int)max_long_total,
+                                                    (int)max_long, d_seg, d_seg + 1, 0, end_bit));
+        CK(cub::DeviceSegmentedRadixSort::SortPairsDescending(nullptr, t2, key1, key0, id1, id0,
+                                                              (int)max_long_total, (int)max_long, d_seg, d_seg + 1));
+        tmp_bytes = std::max(t1, t2);
+        CK(mem.alloc(&tmp, std::max<size_t>(tmp_bytes, 1)));
+    }
+    // -> 0 ok, 2 a listed id outside [0, n), 1 CUDA error
+    auto upload_lists = [&](const Chunk& c, bool check) -> int {
+        const size_t off = (size_t)incl_ptr[c.u0], cnt = (size_t)incl_ptr[c.u1] - off;
+        CK(Stager::get().h2d(d_ix, incl_ix + off, cnt * sizeof(IX), 0));
+        return check ? ids_in_range(d_ix, cnt, n) : 0;
     };
-    int rc = body();
-    if (rc) cudaDeviceSynchronize();
-    if (!B_resident) dfree(dB);
-    if (!A_resident) dfree(dA);
-    dfree(dAsel); dfree(dusers); dfree(dptr); dfree(d_ix); dfree(d_out); dfree(d_sc); dfree(d_bad);
-    dfree(d_su); dfree(d_lu); dfree(d_seg); dfree(id0); dfree(id1); dfree(key0); dfree(key1); dfree(tmp);
-    return rc;
+    // with several chunks every list is checked before the first result is written, and uploaded again
+    if (chunks.size() > 1)
+        for (const Chunk& c : chunks)
+            if (const int bad = upload_lists(c, true)) return bad;
+    std::vector<long long> hp;
+    std::vector<int> hsu, hlu, hseg;
+    std::vector<std::pair<int, int>> classes;           // (capacity, users) of the path (a) launches
+    for (const Chunk& c : chunks) {
+        const size_t m = c.u1 - c.u0, off = (size_t)incl_ptr[c.u0];
+        if (const int bad = upload_lists(c, chunks.size() == 1)) return bad;
+        hp.resize(m + 1); hsu.clear(); classes.clear(); hlu.clear(); hseg.assign(1, 0);
+        for (size_t i = 0; i < m; i++) {
+            const size_t u = c.u0 + i, len = len_of(u);
+            hp[i] = (long long)((size_t)incl_ptr[u] - off);
+            if (len > (size_t)cap) { hlu.push_back((int)i); hseg.push_back(hseg.back() + (int)len); }
+        }
+        // path (a) by length class, so that one long list does not size every CTA's shared memory: lists up
+        // to 4 K items share one launch (its 4 CTAs per SM, the register bound, fit in shared memory), longer
+        // ones go by power of two up to `cap`
+        for (size_t lo = 0, P = (size_t)std::min(cap, 4096);; lo = P, P <<= 1) {
+            const size_t start = hsu.size();
+            for (size_t i = 0; i < m; i++) {
+                const size_t len = len_of(c.u0 + i);
+                if (len > lo && len <= P) hsu.push_back((int)i);
+            }
+            if (hsu.size() > start) classes.push_back({(int)P, (int)(hsu.size() - start)});
+            if (P >= (size_t)cap) break;
+        }
+        hp[m] = (long long)((size_t)incl_ptr[c.u1] - off);
+        CK(cudaMemcpy(dptr, hp.data(), (m + 1) * sizeof(long long), cudaMemcpyHostToDevice));
+        if (gather_users(dA, ldf, user_ix, c.u0, m, dusers, dAsel)) return 1;
+        if (!hsu.empty()) CK(cudaMemcpy(d_su, hsu.data(), hsu.size() * sizeof(int), cudaMemcpyHostToDevice));
+        for (size_t q = 0, first = 0; q < classes.size(); first += classes[q].second, q++) {
+            const size_t smem = rowb + (size_t)classes[q].first * entry;
+            CK(cudaFuncSetAttribute(incl::include_select_smem_kernel<real, IX>,
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            incl::include_select_smem_kernel<real, IX><<<(unsigned)classes[q].second, incl::SMEM_THREADS, smem>>>(
+                dAsel, dB, k, ldf, dptr, d_ix, d_su + first, classes[q].first, (int)n_top, d_out, d_sc);
+            LAUNCHED();
+        }
+        if (!hlu.empty()) {
+            const int nl = (int)hlu.size(), total = hseg.back();
+            CK(cudaMemcpy(d_lu, hlu.data(), nl * sizeof(int), cudaMemcpyHostToDevice));
+            CK(cudaMemcpy(d_seg, hseg.data(), (nl + 1) * sizeof(int), cudaMemcpyHostToDevice));
+            CK(cudaFuncSetAttribute(incl::include_score_long_kernel<real, IX>,
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rowb));
+            incl::include_score_long_kernel<real, IX><<<dim3(64, (unsigned)nl), 256, rowb>>>(
+                dAsel, dB, k, ldf, dptr, d_ix, d_lu, d_seg, id0, key0);
+            LAUNCHED();
+            // by item id, then stably by score: ties come out by ascending id
+            CK(cub::DeviceSegmentedRadixSort::SortPairs(tmp, tmp_bytes, id0, id1, key0, key1, total, nl,
+                                                        d_seg, d_seg + 1, 0, end_bit));
+            CK(cub::DeviceSegmentedRadixSort::SortPairsDescending(tmp, tmp_bytes, key1, key0, id1, id0, total, nl,
+                                                                  d_seg, d_seg + 1));
+            LAUNCHED(); LAUNCHED();
+            incl::include_emit_long_kernel<real, IX><<<(unsigned)nl, 128>>>(d_lu, d_seg, id0, key0, (int)n_top,
+                                                                             d_out, d_sc);
+            LAUNCHED();
+        }
+        CK(cudaGetLastError());
+        CK(Stager::get().d2h(outp_ix + c.u0 * n_top, d_out, m * n_top * sizeof(IX), 0));
+        if (outp_score) CK(Stager::get().d2h(outp_score + c.u0 * n_top, d_sc, m * n_top * sizeof(real), 0));
+        CK(cudaStreamSynchronize(0));
+    }
+    mem.settled = true;
+    return 0;
 }
 
 template <class real, class IX>
@@ -2432,7 +2415,7 @@ static int topn_single_impl(const real* a_vec, const real* B, int k, const IX* i
             memcpy(&cand[t * k], B + (size_t)include_ix[t] * k, (size_t)k * sizeof(real));
         std::vector<IX> pos(n_top);
         int rc = topn_batch_impl<real, IX>(a_vec, cand.data(), k, nullptr, 1, 1, nullptr, nullptr, pos.data(),
-                                           outp_score, n_top, n_include, true);
+                                           outp_score, n_top, n_include);
         if (rc) return rc;
         for (size_t t = 0; t < n_top; t++) outp_ix[t] = include_ix[(size_t)pos[t]];
         return 0;
@@ -2441,9 +2424,9 @@ static int topn_single_impl(const real* a_vec, const real* B, int k, const IX* i
         // the reference sorts the caller's exclusion list in place (src/topN.c:159-160)
         std::sort(exclude_ix, exclude_ix + n_exclude);
         IX ptr[2] = {0, (IX)n_exclude};
-        return topn_batch_impl<real, IX>(a_vec, B, k, nullptr, 1, 1, ptr, exclude_ix, outp_ix, outp_score, n_top, n, true);
+        return topn_batch_impl<real, IX>(a_vec, B, k, nullptr, 1, 1, ptr, exclude_ix, outp_ix, outp_score, n_top, n);
     }
-    return topn_batch_impl<real, IX>(a_vec, B, k, nullptr, 1, 1, nullptr, nullptr, outp_ix, outp_score, n_top, n, true);
+    return topn_batch_impl<real, IX>(a_vec, B, k, nullptr, 1, 1, nullptr, nullptr, outp_ix, outp_score, n_top, n);
 }
 
 extern "C" int pmf_b200_topN(int dtype, int index_bytes, const void* a_vec, const void* B, int k,
@@ -2451,11 +2434,11 @@ extern "C" int pmf_b200_topN(int dtype, int index_bytes, const void* a_vec, cons
                              void* outp_ix, void* outp_score, size_t n_top, size_t n)
 {
     if (pmf_b200_device_count() <= 0) return fail("no usable CUDA device: poismf_b200 has no CPU fallback");
-    if (dtype == PMF_F32 && index_bytes == 8) return topn_single_impl((const float*)a_vec, (const float*)B, k, (const uint64_t*)include_ix, n_include, (uint64_t*)exclude_ix, n_exclude, (uint64_t*)outp_ix, (float*)outp_score, n_top, n);
-    if (dtype == PMF_F32 && index_bytes == 4) return topn_single_impl((const float*)a_vec, (const float*)B, k, (const int*)include_ix, n_include, (int*)exclude_ix, n_exclude, (int*)outp_ix, (float*)outp_score, n_top, n);
-    if (dtype == PMF_F64 && index_bytes == 8) return topn_single_impl((const double*)a_vec, (const double*)B, k, (const uint64_t*)include_ix, n_include, (uint64_t*)exclude_ix, n_exclude, (uint64_t*)outp_ix, (double*)outp_score, n_top, n);
-    if (dtype == PMF_F64 && index_bytes == 4) return topn_single_impl((const double*)a_vec, (const double*)B, k, (const int*)include_ix, n_include, (int*)exclude_ix, n_exclude, (int*)outp_ix, (double*)outp_score, n_top, n);
-    return fail("topN: bad dtype/index width");
+    return with_types(dtype, index_bytes, "topN: bad dtype/index width", [&](auto r, auto i) {
+        using real = decltype(r); using IX = decltype(i);
+        return topn_single_impl((const real*)a_vec, (const real*)B, k, (const IX*)include_ix, n_include, (IX*)exclude_ix,
+                                n_exclude, (IX*)outp_ix, (real*)outp_score, n_top, n);
+    });
 }
 
 extern "C" void pmf_b200_topN_stats(unsigned long long* tensor_core_users, unsigned long long* redone_exact, int reset)
@@ -2478,11 +2461,11 @@ extern "C" int pmf_b200_topN_fitted(pmf_b200_handle* h, int index_bytes, const v
     if (!rf.A || !rf.B) return fail("topN_fitted: the handle holds no factors");
     const size_t dimA = h->dimA, n = h->dimB;
     const int k = h->k;
-    if (h->dtype == PMF_F32 && index_bytes == 8) return topn_batch_impl<float, uint64_t>(nullptr, nullptr, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)excl_ptr, (const uint64_t*)excl_ix, (uint64_t*)outp_ix, (float*)outp_score, n_top, n, false, true, &rf);
-    if (h->dtype == PMF_F32 && index_bytes == 4) return topn_batch_impl<float, int>(nullptr, nullptr, k, (const int*)user_ix, n_users, dimA, (const int*)excl_ptr, (const int*)excl_ix, (int*)outp_ix, (float*)outp_score, n_top, n, false, true, &rf);
-    if (h->dtype == PMF_F64 && index_bytes == 8) return topn_batch_impl<double, uint64_t>(nullptr, nullptr, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)excl_ptr, (const uint64_t*)excl_ix, (uint64_t*)outp_ix, (double*)outp_score, n_top, n, false, true, &rf);
-    if (h->dtype == PMF_F64 && index_bytes == 4) return topn_batch_impl<double, int>(nullptr, nullptr, k, (const int*)user_ix, n_users, dimA, (const int*)excl_ptr, (const int*)excl_ix, (int*)outp_ix, (double*)outp_score, n_top, n, false, true, &rf);
-    return fail("topN_fitted: bad dtype/index width");
+    return with_types(h->dtype, index_bytes, "topN_fitted: bad dtype/index width", [&](auto r, auto i) {
+        using real = decltype(r); using IX = decltype(i);
+        return topn_batch_impl<real, IX>(nullptr, nullptr, k, (const IX*)user_ix, n_users, dimA, (const IX*)excl_ptr,
+                                         (const IX*)excl_ix, (IX*)outp_ix, (real*)outp_score, n_top, n, true, &rf);
+    });
 }
 
 extern "C" int pmf_b200_topN_batch(int dtype, int index_bytes, const void* A, const void* B, int k,
@@ -2491,11 +2474,11 @@ extern "C" int pmf_b200_topN_batch(int dtype, int index_bytes, const void* A, co
                                    void* outp_ix, void* outp_score, size_t n_top, size_t n)
 {
     if (pmf_b200_device_count() <= 0) return fail("no usable CUDA device: poismf_b200 has no CPU fallback");
-    if (dtype == PMF_F32 && index_bytes == 8) return topn_batch_impl((const float*)A, (const float*)B, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)excl_ptr, (const uint64_t*)excl_ix, (uint64_t*)outp_ix, (float*)outp_score, n_top, n, false);
-    if (dtype == PMF_F32 && index_bytes == 4) return topn_batch_impl((const float*)A, (const float*)B, k, (const int*)user_ix, n_users, dimA, (const int*)excl_ptr, (const int*)excl_ix, (int*)outp_ix, (float*)outp_score, n_top, n, false);
-    if (dtype == PMF_F64 && index_bytes == 8) return topn_batch_impl((const double*)A, (const double*)B, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)excl_ptr, (const uint64_t*)excl_ix, (uint64_t*)outp_ix, (double*)outp_score, n_top, n, false);
-    if (dtype == PMF_F64 && index_bytes == 4) return topn_batch_impl((const double*)A, (const double*)B, k, (const int*)user_ix, n_users, dimA, (const int*)excl_ptr, (const int*)excl_ix, (int*)outp_ix, (double*)outp_score, n_top, n, false);
-    return fail("topN_batch: bad dtype/index width");
+    return with_types(dtype, index_bytes, "topN_batch: bad dtype/index width", [&](auto r, auto i) {
+        using real = decltype(r); using IX = decltype(i);
+        return topn_batch_impl((const real*)A, (const real*)B, k, (const IX*)user_ix, n_users, dimA, (const IX*)excl_ptr,
+                               (const IX*)excl_ix, (IX*)outp_ix, (real*)outp_score, n_top, n);
+    });
 }
 
 extern "C" int pmf_b200_topN_batch_include(int dtype, int index_bytes, const void* A, const void* B, int k,
@@ -2504,11 +2487,11 @@ extern "C" int pmf_b200_topN_batch_include(int dtype, int index_bytes, const voi
                                            void* outp_ix, void* outp_score, size_t n_top, size_t n)
 {
     if (pmf_b200_device_count() <= 0) return fail("no usable CUDA device: poismf_b200 has no CPU fallback");
-    if (dtype == PMF_F32 && index_bytes == 8) return topn_include_impl((const float*)A, (const float*)B, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)incl_ptr, (const uint64_t*)incl_ix, (uint64_t*)outp_ix, (float*)outp_score, n_top, n);
-    if (dtype == PMF_F32 && index_bytes == 4) return topn_include_impl((const float*)A, (const float*)B, k, (const int*)user_ix, n_users, dimA, (const int*)incl_ptr, (const int*)incl_ix, (int*)outp_ix, (float*)outp_score, n_top, n);
-    if (dtype == PMF_F64 && index_bytes == 8) return topn_include_impl((const double*)A, (const double*)B, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)incl_ptr, (const uint64_t*)incl_ix, (uint64_t*)outp_ix, (double*)outp_score, n_top, n);
-    if (dtype == PMF_F64 && index_bytes == 4) return topn_include_impl((const double*)A, (const double*)B, k, (const int*)user_ix, n_users, dimA, (const int*)incl_ptr, (const int*)incl_ix, (int*)outp_ix, (double*)outp_score, n_top, n);
-    return fail("topN_batch_include: bad dtype/index width");
+    return with_types(dtype, index_bytes, "topN_batch_include: bad dtype/index width", [&](auto r, auto i) {
+        using real = decltype(r); using IX = decltype(i);
+        return topn_include_impl((const real*)A, (const real*)B, k, (const IX*)user_ix, n_users, dimA, (const IX*)incl_ptr,
+                                 (const IX*)incl_ix, (IX*)outp_ix, (real*)outp_score, n_top, n);
+    });
 }
 
 extern "C" int pmf_b200_topN_fitted_include(pmf_b200_handle* h, int index_bytes, const void* user_ix, size_t n_users,
@@ -2521,9 +2504,9 @@ extern "C" int pmf_b200_topN_fitted_include(pmf_b200_handle* h, int index_bytes,
     if (!rf.A || !rf.B) return fail("topN_fitted_include: the handle holds no factors");
     const size_t dimA = h->dimA, n = h->dimB;
     const int k = h->k;
-    if (h->dtype == PMF_F32 && index_bytes == 8) return topn_include_impl<float, uint64_t>(nullptr, nullptr, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)incl_ptr, (const uint64_t*)incl_ix, (uint64_t*)outp_ix, (float*)outp_score, n_top, n, &rf);
-    if (h->dtype == PMF_F32 && index_bytes == 4) return topn_include_impl<float, int>(nullptr, nullptr, k, (const int*)user_ix, n_users, dimA, (const int*)incl_ptr, (const int*)incl_ix, (int*)outp_ix, (float*)outp_score, n_top, n, &rf);
-    if (h->dtype == PMF_F64 && index_bytes == 8) return topn_include_impl<double, uint64_t>(nullptr, nullptr, k, (const uint64_t*)user_ix, n_users, dimA, (const uint64_t*)incl_ptr, (const uint64_t*)incl_ix, (uint64_t*)outp_ix, (double*)outp_score, n_top, n, &rf);
-    if (h->dtype == PMF_F64 && index_bytes == 4) return topn_include_impl<double, int>(nullptr, nullptr, k, (const int*)user_ix, n_users, dimA, (const int*)incl_ptr, (const int*)incl_ix, (int*)outp_ix, (double*)outp_score, n_top, n, &rf);
-    return fail("topN_fitted_include: bad dtype/index width");
+    return with_types(h->dtype, index_bytes, "topN_fitted_include: bad dtype/index width", [&](auto r, auto i) {
+        using real = decltype(r); using IX = decltype(i);
+        return topn_include_impl<real, IX>(nullptr, nullptr, k, (const IX*)user_ix, n_users, dimA, (const IX*)incl_ptr,
+                                           (const IX*)incl_ix, (IX*)outp_ix, (real*)outp_score, n_top, n, &rf);
+    });
 }

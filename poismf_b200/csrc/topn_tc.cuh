@@ -2,20 +2,10 @@
 //
 // topN's scoring step, scores[u, j] = <A[u], B[j]>, is the one dense contraction of the path
 // (/root/reference/src/topN.c:215-224 does it as one GEMV per user).  Batched over users it is a
-// GEMM; here it runs on the 5th-generation tensor cores in TF32:
-//
-// Two scorers share the epilogue logic:
-//   * `score_pipe_tf32_kernel` (the product path): warp-specialised persistent CTAs, operands by TMA
-//     (128-byte-swizzled 2-D boxes), a ring of shared-memory stages, accumulators double-buffered in TMEM,
-//     eight epilogue warps — described in front of the kernel;
-//   * `score_tiles_tf32_kernel` (r1; MODE_SCORES for the full-sort path and POISMF_B200_TOPN_NOPIPE): one CTA per
-//     128 users x 128 items tile; both operand tiles staged K-major in shared memory with generic loads in the
-//     canonical no-swizzle UMMA layout (8-row x 16-byte core matrices; for tile row r and 16-byte K-chunk c
-//     the chunk sits at (c * 128 + r) * 16 bytes, i.e. stride-byte-offset 128 B between 8-row groups,
-//     leading-byte-offset 2048 B between K-chunks); one elected thread issues k/8
-//     `tcgen05.mma.cta_group::1.kind::tf32` instructions (M = 128, N = 128, K = 8 each) accumulating into 128
-//     TMEM columns, then `tcgen05.commit` onto an mbarrier; the four warps read their 32 TMEM lanes back with
-//     `tcgen05.ld.32x32b.x32`.
+// GEMM; `score_pipe_tf32_kernel` runs it on the 5th-generation tensor cores in TF32: warp-specialised
+// persistent CTAs, operands by TMA (128-byte-swizzled 2-D boxes), a ring of shared-memory stages, accumulators
+// double-buffered in TMEM, eight epilogue warps — described in front of the kernel.  With too few items for
+// the fused select below, `score_tiles_tf32_kernel` writes the TF32 score matrix for a segmented sort instead.
 //
 // TF32 scores are only used to pick CANDIDATES: the caller keeps the best 2N+ per user, re-scores
 // them exactly in FP32 (same left-to-right sums as the reference) and proves from the TF32 error
@@ -25,12 +15,12 @@
 // The select is fused into the scorer's epilogue so that the U x n score matrix never exists
 // (SURVEY.md 8d).  Two passes over the tiles, the GEMM being far cheaper than any sort of n scores:
 //   pass 1 (MODE_GROUPMAX)  per user, the maximum of every group of 16 consecutive items — of every S-th item
-//           tile only (pipelined scorer; S = 4, 2 or 1)
+//           tile only (S = 4, 2 or 1)
 //           -> tau[u] = the M-th largest of these group maxima: a lower bound of the M-th largest over all
 //              items, so at least M items score >= tau[u], and about S M of them do;
 //   pass 2 (MODE_EMIT)      all tiles; items with score >= tau[u] are appended to the user's candidate list,
 // then the (<= 4096) candidates are ordered by (score desc, id asc) and the best M go to the exact
-// re-scoring as before.  Excluded items are masked in the epilogue from a per-user bitmap.
+// re-scoring.  Excluded items are masked in the epilogue from a per-user bitmap.
 #pragma once
 #include <cuda.h>
 #include "common.cuh"
@@ -44,7 +34,7 @@ constexpr int GROUP = 16;        // items per group maximum
 constexpr int CAND_CAP = 4096;   // candidates per user that are ordered (>= GROUP * 256)
 constexpr int CAND_SLACK = 4;    // the per-CTA regions of a user hold CAND_SLACK x CAND_CAP slots together
 constexpr int CAND_TOP = 256;    // candidates handed to the exact re-scoring (>= M)
-enum { MODE_SCORES = 0, MODE_GROUPMAX = 1, MODE_EMIT = 2 };
+enum { MODE_GROUPMAX = 1, MODE_EMIT = 2 };
 
 // order-preserving key of a non-negative score; masked entries (negative) sort below everything
 PMF_DEVINL uint32_t score_key(float s) { return s < 0.f ? 0u : __float_as_uint(s) + 1u; }
@@ -63,6 +53,7 @@ PMF_DEVINL uint64_t make_smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t 
     d |= (uint64_t)1 << 46;
     return d;
 }
+
 // Instruction descriptor for kind::tf32: D = F32 (bits [4,6) = 1), A = B = TF32 (bits [7,10), [10,13) = 2),
 // both K-major (bits 15, 16 = 0), N >> 3 in [17,23), M >> 4 in [24,29).
 constexpr uint32_t make_idesc_tf32(int M, int N)
@@ -136,21 +127,27 @@ PMF_DEVINL void stage_operand(float4* s, const float* __restrict__ G, size_t row
 
 // What the epilogue of a tile does with its scores
 struct TileOut {
-    float* scores; int* ids;                 // MODE_SCORES: scores[u, j] (TF32), ids[u, j] = j
     const uint32_t* excl_bits; size_t excl_words;   // bitmap of excluded items, excl_words 32-bit words per user (or null)
     float* gmax; size_t ngroups;             // MODE_GROUPMAX: gmax[u, j / GROUP]
     const float* tau;                        // MODE_EMIT: per-user threshold ...
     float* cand_sc; int* cand_id; int* cand_cnt;   // ... and candidate lists (CAND_CAP slots per user)
-    // the pipelined scorer splits a user's slots into `cand_regions` regions of `cand_cap` slots, one per CTA
+    // the scorer splits a user's slots into `cand_regions` regions of `cand_cap` slots, one per CTA
     // along the items (each written by exactly one thread: no atomics); cand_cnt is [user][region]
     int cand_regions, cand_cap;
 };
 
-// grid = (ceil(n/TN), ceil(U/TM)), 128 threads.
-template <int MODE>
+// The TF32 score matrix of a chunk of users, for the segmented-sort select (items too few for the fused one):
+// scores[u, j] and ids[u, j] = j, row stride n.  One CTA per 128 users x 128 items tile, both operand tiles
+// staged K-major in shared memory by generic loads in the canonical no-swizzle UMMA layout (8-row x 16-byte
+// core matrices; for tile row r and 16-byte K-chunk c the chunk sits at (c * 128 + r) * 16 bytes, i.e.
+// stride-byte-offset 128 B between 8-row groups, leading-byte-offset 2048 B between K-chunks); one thread
+// issues k/8 `tcgen05.mma.cta_group::1.kind::tf32` (M = N = 128, K = 8) into 128 TMEM columns and commits onto
+// an mbarrier; the four warps read their 32 TMEM lanes back with `tcgen05.ld.32x32b.x32`.
+// grid = (ceil(n/TN), ceil(U/TM)), 128 threads, kpad * 1024 bytes of dynamic shared memory.
 __global__ void __launch_bounds__(128) score_tiles_tf32_kernel(const float* __restrict__ Asel, int U,
                                                                const float* __restrict__ B, size_t n, int ldf,
-                                                               int kpad, TileOut out)
+                                                               int kpad, float* __restrict__ scores,
+                                                               int* __restrict__ ids)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     float4* sA = reinterpret_cast<float4*>(smem_raw);
@@ -190,55 +187,17 @@ __global__ void __launch_bounds__(128) score_tiles_tf32_kernel(const float* __re
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 
     // epilogue: warp w owns TMEM lanes 32w .. 32w+31 (= tile rows), 32 columns at a time
-    const int row = warp * 32 + lane;
-    const int u = u0 + row;
-    const float NEG = -RealTraits<float>::huge();
-    uint4 ex = make_uint4(0u, 0u, 0u, 0u);       // this user's exclusion bits of the tile's 128 items
-    if (MODE != MODE_SCORES && out.excl_bits && u < U)
-        ex = __ldg(reinterpret_cast<const uint4*>(out.excl_bits + (size_t)u * out.excl_words + (j0 >> 5)));
-    const float tau = (MODE == MODE_EMIT && u < U) ? out.tau[u] : 0.f;
+    const int u = u0 + warp * 32 + lane;
     for (int c = 0; c < TN / 32; c++) {
         uint32_t r[32];
         tmem_ld32(tmem + ((uint32_t)(warp * 32) << 16) + (uint32_t)(c * 32), r);
         if (u >= U) continue;
         const size_t jc = j0 + c * 32;
-        if (MODE == MODE_SCORES) {
-            float* srow = out.scores + (size_t)u * n + jc;
-            int* irow = out.ids + (size_t)u * n + jc;
+        float* srow = scores + (size_t)u * n + jc;
+        int* irow = ids + (size_t)u * n + jc;
 #pragma unroll
-            for (int i = 0; i < 32; i++)
-                if (jc + i < n) { srow[i] = __uint_as_float(r[i]); irow[i] = (int)(jc + i); }
-        } else {
-            const uint32_t exw = c == 0 ? ex.x : (c == 1 ? ex.y : (c == 2 ? ex.z : ex.w));
-            // valid = inside [0, n) and not excluded
-            uint32_t valid = ~exw;
-            if (jc + 32 > n) valid &= (jc >= n) ? 0u : ((1u << (unsigned)(n - jc)) - 1u);
-            if (MODE == MODE_GROUPMAX) {
-#pragma unroll
-                for (int g = 0; g < 32 / GROUP; g++) {
-                    float m = NEG;
-#pragma unroll
-                    for (int i = 0; i < GROUP; i++) {
-                        const float v = __uint_as_float(r[g * GROUP + i]);
-                        if ((valid >> (g * GROUP + i)) & 1u) m = fmaxf(m, v);
-                    }
-                    const size_t gi = jc / GROUP + g;
-                    if (gi < out.ngroups) out.gmax[(size_t)u * out.ngroups + gi] = m;
-                }
-            } else {
-#pragma unroll
-                for (int i = 0; i < 32; i++) {
-                    const float v = __uint_as_float(r[i]);
-                    if (((valid >> i) & 1u) && v >= tau) {
-                        const int pos = atomicAdd(out.cand_cnt + u, 1);
-                        if (pos < CAND_CAP) {
-                            out.cand_sc[(size_t)u * CAND_CAP + pos] = v;
-                            out.cand_id[(size_t)u * CAND_CAP + pos] = (int)(jc + i);
-                        }
-                    }
-                }
-            }
-        }
+        for (int i = 0; i < 32; i++)
+            if (jc + i < n) { srow[i] = __uint_as_float(r[i]); irow[i] = (int)(jc + i); }
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
@@ -246,7 +205,7 @@ __global__ void __launch_bounds__(128) score_tiles_tf32_kernel(const float* __re
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"((uint32_t)TN) : "memory");
 }
 
-// ---- the pipelined scorer (r2): persistent CTAs, operands by TMA, accumulators double-buffered in TMEM ------
+// ---- the scorer: persistent CTAs, operands by TMA, accumulators double-buffered in TMEM ------
 // One CTA keeps TWO user tiles (256 users: the A operands, loaded once) and walks a contiguous range of item
 // tiles; every item tile brought on chip is used by both (half the L2 -> SM traffic of one tile per CTA).
 // Operands arrive by TMA (`cp.async.bulk.tensor.2d`, SASS UTMALDG): the factor matrices are described to the

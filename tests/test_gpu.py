@@ -651,7 +651,7 @@ def test_topn_batch_tensor_core_path_is_exact(k, n_top):
 
 
 def test_topn_fused_select_edge_cases(monkeypatch):
-    """The fused select (group maxima -> threshold -> candidates) against the full-sort path and the
+    """The fused select (group maxima -> threshold -> candidates) against the exact route and the
     oracle: items sorted by popularity (the worst case for group maxima), an item count that is not a
     multiple of the tile, unsorted exclusion lists, and massive score ties (candidate overflow ->
     exact fallback)."""
@@ -668,9 +668,9 @@ def test_topn_fused_select_edge_cases(monkeypatch):
     ix, sc = c_funs._topN_batch(A, B, excl_ptr=ptr, excl_ix=eix, top_n=n_top, output_score=True)
     n_tc, n_redo = _lib.topn_stats(reset=True)
     assert n_tc == n_users and n_redo <= 0.1 * n_users
-    monkeypatch.setenv("POISMF_B200_TOPN_SORT", "1")                           # full-sort path
+    monkeypatch.setenv("POISMF_B200_TOPN_EXACT", "1")                          # exact route
     ix2, sc2 = c_funs._topN_batch(A, B, excl_ptr=ptr, excl_ix=eix, top_n=n_top, output_score=True)
-    monkeypatch.delenv("POISMF_B200_TOPN_SORT")
+    monkeypatch.delenv("POISMF_B200_TOPN_EXACT")
     assert np.array_equal(sc, sc2)
     assert all((sc[u] == sc[u][t]).sum() > 1 for u, t in zip(*np.nonzero(ix != ix2)))
     orc = Restatement(np.float32)
@@ -684,6 +684,50 @@ def test_topn_fused_select_edge_cases(monkeypatch):
     ix3, sc3 = c_funs._topN_batch(A[:8], Bt, top_n=n_top, output_score=True)
     assert _lib.topn_stats(reset=True)[1] == 8
     assert all(len(set(r.tolist())) == n_top for r in ix3) and (sc3 == sc3[:, :1]).all()
+
+
+@pytest.mark.parametrize("n_items,n_top,n_users", [(300, 10, 48), (300, 100, 48), (1000, 10, 48), (1000, 100, 48),
+                                                   (5000, 10, 48), (5000, 100, 48), (5000, 100, 256), (1328, 10, 48),
+                                                   (1329, 10, 48), (6384, 100, 48), (6385, 100, 48)])
+def test_topn_routes_around_fused_threshold(n_items, n_top, n_users, monkeypatch, capfd):
+    """Item counts around the fused select's threshold (the items must hold 2 M candidate groups of 16, M =
+    max(2 N, N + 32)).  At and above it every user goes through the fused select; below it the TF32 scores are
+    sorted when there are >= 256 users and n k >= 2 M (k + 32), else the call is exact (no user on the tensor
+    cores).  Host arrays and a fit handle's resident factors, with and without exclusion lists: scores are the
+    oracle's bits, ids equal outside score ties, no excluded id."""
+    from poismf_b200 import _lib, c_funs
+    from poismf_b200.device import DeviceFit
+    rng = np.random.default_rng(n_items + n_top + n_users)
+    k = 24
+    A = np.ascontiguousarray(rng.gamma(0.5, 0.5, size=(n_users, k)).astype(np.float32))
+    B = np.ascontiguousarray(rng.gamma(0.5, 0.5, size=(n_items, k)).astype(np.float32))
+    lens = rng.integers(0, min(60, n_items - n_top), n_users)
+    ptr = np.concatenate([[0], np.cumsum(lens)]).astype(np.uint64)
+    eix = np.concatenate([rng.choice(n_items, int(m), replace=False) for m in lens]).astype(np.uint64)
+    fused = -(-n_items // 16) >= 2 * max(2 * n_top, n_top + 32)
+    on_tc = fused or (n_users >= 256 and n_items * k >= 2 * min(n_items, max(2 * n_top, n_top + 32)) * (k + 32))
+    monkeypatch.setenv("POISMF_B200_TOPN_TRACE", "1")          # the fused route's phases include "work arrays"
+    orc = Restatement(np.float32)
+    fit = DeviceFit(n_users, n_items, k, np.float32)
+    try:
+        fit.set_factors(A, B)
+        for excl in (dict(), dict(excl_ptr=ptr, excl_ix=eix)):
+            for rank in (lambda: c_funs._topN_batch(A, B, top_n=n_top, output_score=True, **excl),
+                         lambda: fit.topN(top_n=n_top, output_score=True, **excl)):
+                capfd.readouterr()
+                _lib.topn_stats(reset=True)
+                ix, sc = rank()
+                n_tc, _ = _lib.topn_stats(reset=True)
+                assert n_tc == (n_users if on_tc else 0)
+                assert ("[topN] work arrays" in capfd.readouterr().err) == fused
+                for u in range(0, n_users, 1 if n_users <= 48 else 5):
+                    ex = eix[int(ptr[u]):int(ptr[u + 1])] if excl else np.empty(0, np.uint64)
+                    rc, ix_r, sc_r = orc.topN(np.ascontiguousarray(A[u]), B, n_top, exclude=ex if ex.size else None)
+                    assert rc == 0 and np.array_equal(sc[u], sc_r)
+                    assert all((sc_r == sc_r[t]).sum() > 1 for t in np.nonzero(ix[u] != ix_r)[0])
+                    assert not np.isin(ix[u], ex).any()
+    finally:
+        fit.close()
 
 
 @pytest.mark.parametrize("dtype", DTYPES)
