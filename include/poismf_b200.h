@@ -222,6 +222,42 @@ int pmf_b200_topN_fitted_include(pmf_b200_handle* h, int index_bytes, const void
                                  const void* incl_ptr, const void* incl_ix,
                                  void* outp_ix, void* outp_score, size_t n_top);
 
+/* Batched top-N for NEW users (PoisMF.topN_new / predict_factors for many users at once, poismf/__init__.py:502-576,
+ * :977-1075): the n_new users given as CSR rows (values real_t[nnz], indptr sparse_ix[n_new+1], indices
+ * sparse_ix[nnz]) are folded in against the fixed item factors B [n x k], then ranked against B.
+ * Fold-in = factors_multiple (src/pred.c:66-199) with the parameters of *p: method, numiter (niter), maxupd,
+ * step_size, limit_step, l2_reg, w_mult, flags as there; reuse_prev = reuse_mean; early_stop must be 0; the column
+ * sums used are Bsum + l1_reg (in real_t, added when l1_reg > 0).  A caller holding the model's Bsum (old l1 already
+ * in it) passes the positive part of l1_new - l1_old as l1_reg.  PoisMF.topN_new is method PMF_TNCG, numiter 1,
+ * step_size 0, limit_step 0.  Rows without non-zeros get zero factors.  The new users' factors stay on the device.
+ * Ranking = pmf_b200_topN_batch of those rows (same routes, ids and scores), or with include lists
+ * pmf_b200_topN_batch_include.  Exclusion lists (excl_ptr/excl_ix) or include lists (incl_ptr/incl_ix) per new user
+ * are optional, not both; nothing is excluded implicitly (pass the fold-in CSR's indptr/indices as the exclusion lists
+ * to leave out the users' own items).  Bsum, Amean: k reals each, required.  outp_ix [n_new x n_top] required,
+ * outp_score optional, A_out [n_new x k] optional.  B goes through the POISMF_B200_CACHE_FACTORS cache.
+ * Returns 2, before any output is written, when Xr_indptr is not monotone, a fold-in item id is >= n, early_stop is
+ * set or the method is unknown, both kinds of lists are given, n_top is 0 or > n, a list fails the checks of the
+ * two ranking entries, Bsum or Amean is NULL, or no output is requested; 1 on a CUDA failure. */
+int pmf_b200_topN_new_batch(int dtype, int index_bytes, const void* B, const void* Bsum, const void* Amean,
+                            int k, size_t n, const void* Xr, const void* Xr_indptr, const void* Xr_indices,
+                            size_t n_new, const pmf_b200_params* p,
+                            const void* excl_ptr, const void* excl_ix, const void* incl_ptr, const void* incl_ix,
+                            void* outp_ix, void* outp_score, size_t n_top, void* A_out);
+/* The same against the factors resident in a fit handle: B = the handle's item factors, read in place (nothing but
+ * the new users' rows, k reals of statistics and the lists travels to the device).  Bsum / Amean may be NULL: they
+ * are then computed on the device from the handle's B and A as pmf_b200_fit_stats(h, 0, ...) does.  outp_ix may be
+ * NULL: fold-in only (PoisMF.transform against a resident fit) into A_out; at least one of outp_ix / A_out.  Waits
+ * like pmf_b200_topN_fitted first; the handle's factors, matrices and plans are left untouched. */
+int pmf_b200_topN_new_fitted(pmf_b200_handle* h, int index_bytes, const void* Bsum, const void* Amean,
+                             const void* Xr, const void* Xr_indptr, const void* Xr_indices, size_t n_new,
+                             const pmf_b200_params* p,
+                             const void* excl_ptr, const void* excl_ix, const void* incl_ptr, const void* incl_ix,
+                             void* outp_ix, void* outp_score, size_t n_top, void* A_out);
+/* Column sums of the handle's B plus l1_reg (when > 0) into Bsum_out, column means of its A into Amean_out (k reals
+ * each, either may be NULL): the Bsum / Amean attributes PoisMF keeps after a fit (poismf/__init__.py:438-439).
+ * Summed in a fixed order on the device, so every call and every replica of a sharded fit gives the same bits. */
+int pmf_b200_fit_stats(pmf_b200_handle* h, double l1_reg, void* Bsum_out, void* Amean_out);
+
 /* Counters of the calling thread's topN calls: users scored by the tensor-core candidate scorer,
  * and how many of those had to be redone by the exact scorer because the TF32 error bound could
  * not prove their candidate set complete. */

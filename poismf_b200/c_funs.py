@@ -169,6 +169,68 @@ def _topN_batch(A, B, users=None, excl_ptr=None, excl_ix=None, top_n=10, output_
     return outp_ix, outp_score
 
 
+def _new_users(call, Xr_indptr, Xr_indices, Xr, k, dtype, params, top_n=10, output_score=False, excl_ptr=None,
+               excl_ix=None, incl_ptr=None, incl_ix=None, rank=True, return_factors=False):
+    """Argument marshalling of pmf_b200_topN_new_batch / _fitted: `call(index_bytes, Xr, indptr, indices, n_new, params,
+    excl_ptr, excl_ix, incl_ptr, incl_ix, outp_ix, outp_score, n_top, A_out)` -> return code.  Index arrays go at the
+    width of Xr_indptr (8 bytes: uint64, 4: int32).  Returns (ids, scores), (ids, scores, A) or, with rank=False, A."""
+    _lib.require_gpu()
+    if Xr.dtype != dtype:
+        raise TypeError("Xr and the item factors must share one dtype")
+    ib = _lib.index_bytes(Xr_indptr)
+    ixdt = np.uint64 if ib == 8 else np.int32
+    n_new = Xr_indptr.shape[0] - 1
+    ptr = np.ascontiguousarray(Xr_indptr).view(ixdt) if ib == 8 else np.ascontiguousarray(Xr_indptr)
+    ind = np.ascontiguousarray(Xr_indices, dtype=ixdt)
+    xv = np.ascontiguousarray(Xr)
+    include = _include_lists(incl_ptr, incl_ix, excl_ptr, excl_ix, n_new)
+    lists = [None] * 4
+    if include is not None:
+        lists[2:] = [np.ascontiguousarray(a, dtype=ixdt) for a in include]
+    elif excl_ptr is not None and excl_ix is not None:
+        lists[:2] = [np.ascontiguousarray(a, dtype=ixdt) for a in (excl_ptr, excl_ix)]
+    ids = np.empty((n_new, top_n) if rank else (0, 0), dtype=ixdt)
+    sc = np.empty((n_new, top_n) if rank and output_score else (0, 0), dtype=dtype)
+    A = np.empty((n_new, k), dtype=dtype) if return_factors or not rank else None
+    rc = call(ib, _lib.ptr(xv), _lib.ptr(ptr), _lib.ptr(ind), n_new, ctypes.byref(params), *map(_lib.ptr, lists),
+              _lib.ptr(ids) if rank else None, _lib.ptr(sc) if rank and output_score else None,
+              top_n if rank else 0, _lib.ptr(A))
+    if rc == 1:
+        raise MemoryError(_lib.last_error())
+    if rc == 2:
+        raise ValueError("topN_new: invalid arguments")
+    if not rank:
+        return A
+    return (ids, sc, A) if return_factors else (ids, sc)
+
+
+def _positive_l1(dtype, l1_new, l1_old):
+    """l1_new - l1_old in the model's real type when positive, else 0 (pmf_b200_factors_single's rule)."""
+    real = np.dtype(dtype).type
+    d = real(l1_new) - real(l1_old)
+    return float(d) if d > 0 else 0.0
+
+
+def _topN_new_batch(Xr_indptr, Xr_indices, Xr, B, Bsum, Amean, top_n=10, output_score=False, excl_ptr=None,
+                    excl_ix=None, incl_ptr=None, incl_ix=None, reuse_mean=True, maxupd=20, l2_reg=1e5, l1_new=0.0,
+                    l1_old=0.0, w_mult=1.0, return_factors=False, flags=0):
+    """Batched PoisMF.topN_new (no reference equivalent; include/poismf_b200.h: pmf_b200_topN_new_batch): the new users'
+    CSR rows are folded in against B as `_predict_factors` folds in one row (same keywords), then ranked as
+    `_topN_batch` ranks them, with optional per-user exclusion or include lists.  Nothing is excluded implicitly:
+    pass excl_ptr=Xr_indptr, excl_ix=Xr_indices to leave out the users' own items.  Returns (ids, scores), or
+    (ids, scores, A) with `return_factors`."""
+    k = B.shape[1]
+    params = _lib.make_params("tncg", l2_reg, l1_reg=_positive_l1(B.dtype, l1_new, l1_old), w_mult=w_mult,
+                              step_size=0.0, numiter=1, maxupd=maxupd, reuse_prev=reuse_mean, flags=flags)
+    Bc, Bs, Am = (np.ascontiguousarray(a, dtype=B.dtype) for a in (B, Bsum, Amean))
+
+    def call(ib, *args):
+        return _lib.lib().pmf_b200_topN_new_batch(_lib.dtype_code(B.dtype), ib, _lib.ptr(Bc), _lib.ptr(Bs),
+                                                  _lib.ptr(Am), k, Bc.shape[0], *args)
+    return _new_users(call, Xr_indptr, Xr_indices, Xr, k, B.dtype, params, top_n, output_score, excl_ptr, excl_ix,
+                      incl_ptr, incl_ix, return_factors=return_factors)
+
+
 def _fit_coo(rows, cols, counts, A, B, method="tncg", limit_step=False, l2_reg=1e9, l1_reg=0.0, w_mult=1.0,
              step_size=1e-7, niter=10, maxupd=1, early_stop=True, reuse_prev=True, flags=0):
     """PoisMF._process_data + _fit (poismf/__init__.py:376-440) in one call: the COO triplets are turned

@@ -118,6 +118,32 @@ static int tile_stride(int k, int V)
     return units * V;
 }
 
+// column sums of M [nrow x ldf] -> out [k], finished by `fin`, on `st`.  Both orders are fixed, so the sums are the
+// same run to run and on every replica: strict = the reference's sequential order; else per-CTA partials over
+// n_partial (at least) CTAs' strided rows, folded in CTA order.  `partial` holds n_partial x ldf reals.
+template <class real>
+static int launch_column_sums(const real* M, size_t nrow, int k, int ldf, const ColsumFinal<real>& fin, bool strict,
+                              real* partial, int n_partial, real* out, cudaStream_t st)
+{
+    if (strict) {
+        colsum_seq_kernel<real><<<(k + 63) / 64, 64, 0, st>>>(M, nrow, k, ldf, fin, out);
+        LAUNCHED();
+    } else {
+        const int threads = 256;
+        if (ldf > threads) return fail("k too large for the column-sum kernel");
+        const int rpb = threads / ldf;
+        int grid = (int)std::min<size_t>((size_t)n_partial, (nrow + rpb - 1) / rpb);
+        grid = std::max(grid, 1);
+        colsum_partial_kernel<real><<<grid, threads, threads * sizeof(real), st>>>(M, nrow, ldf, partial);
+        LAUNCHED();
+        colsum_fold_kernel<real><<<(k + 63) / 64, 64, 0, st>>>(partial, grid, k, ldf, fin, out);
+        LAUNCHED();
+    }
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail("column sums: %s", cudaGetErrorString(e));
+    return 0;
+}
+
 // ---------------------------------------------------------------------------
 // one orientation (CSR or CSC) of the count matrix on the device + its row plan
 // ---------------------------------------------------------------------------
@@ -306,7 +332,8 @@ template <class real> struct HandleT : pmf_b200_handle {
         return 0;
     }
 
-    int init()
+    // B_dev: bind this device matrix [dimB x ldf] as B instead of allocating one (a fold-in against resident factors)
+    int init(real* B_dev = nullptr)
     {
         CK(cudaSetDevice(device));
         CK(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, device));
@@ -316,10 +343,14 @@ template <class real> struct HandleT : pmf_b200_handle {
         own_stream = true; have_stream = true;
         CK(dmalloc(&A, dimA * (size_t)ldf * sizeof(real)));
         ownA = true;
-        CK(dmalloc(&B, dimB * (size_t)ldf * sizeof(real)));
-        ownB = true;
         CK(cudaMemsetAsync(A, 0, dimA * (size_t)ldf * sizeof(real), stream));
-        CK(cudaMemsetAsync(B, 0, dimB * (size_t)ldf * sizeof(real), stream));
+        if (B_dev) {
+            B = B_dev;
+        } else {
+            CK(dmalloc(&B, dimB * (size_t)ldf * sizeof(real)));
+            ownB = true;
+            CK(cudaMemsetAsync(B, 0, dimB * (size_t)ldf * sizeof(real), stream));
+        }
         CK(dmalloc(&csum, (size_t)kp * sizeof(real)));
         n_partial = num_sms * 4;
         CK(dmalloc(&partial, (size_t)n_partial * ldf * sizeof(real)));
@@ -861,22 +892,7 @@ template <class real> struct HandleT : pmf_b200_handle {
     // ---- column sums of the fixed factor matrix -------------------------------
     int column_sums(const real* F, size_t nrow, const ColsumFinal<real>& fin, bool strict)
     {
-        if (strict) {
-            colsum_seq_kernel<real><<<(k + 63) / 64, 64, 0, stream>>>(F, nrow, k, ldf, fin, csum);
-            LAUNCHED();
-        } else {
-            const int threads = 256;
-            if (ldf > threads) return fail("k too large for the column-sum kernel");
-            const int rpb = threads / ldf;
-            int grid = (int)std::min<size_t>((size_t)n_partial, (nrow + rpb - 1) / rpb);
-            grid = std::max(grid, 1);
-            colsum_partial_kernel<real><<<grid, threads, threads * sizeof(real), stream>>>(F, nrow, ldf, partial);
-            LAUNCHED();
-            colsum_fold_kernel<real><<<(k + 63) / 64, 64, 0, stream>>>(partial, grid, k, ldf, fin, csum);
-            LAUNCHED();
-        }
-        CK(cudaGetLastError());
-        return 0;
+        return launch_column_sums(F, nrow, k, ldf, fin, strict, partial, n_partial, csum, stream);
     }
 
     static cudaError_t launch_regtile(const LaunchCfg& cfg, const SideParams<float>& P)
@@ -1280,7 +1296,8 @@ template <class real> struct HandleT : pmf_b200_handle {
     }
 
     // ---- factors_multiple (src/pred.c:66-199): rows of A for new data, B and Bsum fixed ---------
-    // The handle holds the new rows' CSR on the CSR side and B; A (dimA rows) is produced here.
+    // The handle holds the new rows' CSR on the CSR side and B; A (dimA rows) is produced here.  Bsum and Amean
+    // are k host reals.  A_out == NULL leaves the rows on the device only (A of this handle).
     int factors_multiple(void* A_out, const void* Bsum_v, const void* Amean_v, const pmf_b200_params& p,
                          int reuse_mean) override
     {
@@ -1291,10 +1308,17 @@ template <class real> struct HandleT : pmf_b200_handle {
         real step = (real)p.step_size;
         {   // initialise every row to the mean of the old A (:144-147); tncg without reuse_mean starts
             // from 1e-3 inside the solver, rows are zero-filled here only to be deterministic
-            std::vector<real> init(dimA * (size_t)k, (real)0);
-            if (reuse_mean || p.method != PMF_TNCG)
-                for (size_t r = 0; r < dimA; r++) memcpy(&init[r * k], Amean, (size_t)k * sizeof(real));
-            if (copy_in(A, init.data(), dimA, stream)) return 1;
+            const bool mean = reuse_mean || p.method != PMF_TNCG;
+            real* d_mean = nullptr;
+            if (mean) {
+                CK(dmalloc(&d_mean, (size_t)k * sizeof(real)));
+                deferred.push_back(d_mean);
+                CK(cudaMemcpyAsync(d_mean, Amean, (size_t)k * sizeof(real), cudaMemcpyHostToDevice, stream));
+            }
+            const int grid = (int)std::min<size_t>((dimA * (size_t)ldf + 255) / 256, (size_t)num_sms * 8);
+            fill_rows_kernel<real><<<std::max(grid, 1), 256, 0, stream>>>(A, dimA, k, ldf, d_mean);
+            LAUNCHED();
+            CK(cudaGetLastError());
             if (sync_all()) return 1;
         }
         pmf_b200_params q = p;
@@ -2508,5 +2532,169 @@ extern "C" int pmf_b200_topN_fitted_include(pmf_b200_handle* h, int index_bytes,
         using real = decltype(r); using IX = decltype(i);
         return topn_include_impl<real, IX>(nullptr, nullptr, k, (const IX*)user_ix, n_users, dimA, (const IX*)incl_ptr,
                                            (const IX*)incl_ix, (IX*)outp_ix, (real*)outp_score, n_top, n, &rf);
+    });
+}
+
+// ---- batched top-N for new users: fold them in against fixed item factors, then rank them ------------------------
+// = PoisMF.topN_new / predict_factors (poismf/__init__.py:502-576, :977-1075) for many users in one call: the rows
+// are solved by factors_multiple (src/pred.c:66-199) on a second handle that binds the item factors in place, and
+// ranked by topn_batch_impl / topn_include_impl straight from the device.
+
+// Bsum = column sums of B + l1 (when > 0), Amean = column means of A, k host reals each (the attributes PoisMF keeps
+// after a fit, poismf/__init__.py:438-439).  Fixed-order sums (launch_column_sums): the same bits on every call and on
+// every replica of a sharded fit.
+template <class real>
+static int fit_stats_impl(const real* dA, size_t dimA, const real* dB, size_t dimB, int k, int ldf, int device,
+                          double l1, real* Bsum, real* Amean)
+{
+    CK(cudaSetDevice(device));
+    int num_sms = 148;
+    CK(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, device));
+    const int n_partial = num_sms * 4;
+    DeviceBlocks mem;
+    real *partial = nullptr, *d_out = nullptr;
+    CK(mem.alloc(&partial, (size_t)n_partial * ldf * sizeof(real)));
+    CK(mem.alloc(&d_out, 2 * (size_t)k * sizeof(real)));
+    ColsumFinal<real> fin = {};
+    fin.l1 = (real)l1;
+    if (launch_column_sums(dB, dimB, k, ldf, fin, false, partial, n_partial, d_out, (cudaStream_t)0)) return 1;
+    fin.l1 = (real)0;
+    if (launch_column_sums(dA, dimA, k, ldf, fin, false, partial, n_partial, d_out + k, (cudaStream_t)0)) return 1;
+    std::vector<real> h(2 * (size_t)k);
+    CK(cudaMemcpy(h.data(), d_out, 2 * (size_t)k * sizeof(real), cudaMemcpyDeviceToHost));
+    mem.settled = true;
+    for (int c = 0; c < k; c++) {
+        if (Bsum) Bsum[c] = h[c];
+        if (Amean) Amean[c] = h[k + c] / (real)dimA;
+    }
+    return 0;
+}
+
+// -> 2 when the arguments of a new-user call are invalid (checked on the host before anything reaches the device),
+// else 0.  The fold-in ids are range-checked here: they are narrowed to int32 on upload and gather rows of B.
+template <class IX>
+static int check_new_users(const void* Xr, const IX* Xr_indptr, const IX* Xr_indices, size_t n_new, size_t n,
+                           const pmf_b200_params* p, const void* excl_ptr, const void* excl_ix, const void* incl_ptr,
+                           const void* incl_ix, const void* outp_ix, size_t n_top, const void* A_out)
+{
+    if (!p || p->early_stop) return 2;
+    if (p->method != PMF_PG && p->method != PMF_CG && p->method != PMF_TNCG) return 2;
+    if (!outp_ix && !A_out) return 2;
+    if ((excl_ptr || excl_ix) && (incl_ptr || incl_ix)) return 2;
+    if (outp_ix && (n_top == 0 || n_top > n)) return 2;
+    if (n_new > (size_t)INT32_MAX || n > (size_t)INT32_MAX) return 2;
+    if (n_new == 0) return 0;
+    if (!Xr_indptr) return 2;
+    if (std::is_signed<IX>::value && (long long)Xr_indptr[0] < 0) return 2;
+    for (size_t u = 0; u < n_new; u++)
+        if (Xr_indptr[u + 1] < Xr_indptr[u]) return 2;
+    const size_t nnz = (size_t)(Xr_indptr[n_new] - Xr_indptr[0]);
+    if (nnz && (!Xr || !Xr_indices)) return 2;
+    size_t top = 0;                       // a negative id of a signed type is a huge size_t
+    for (size_t t = 0; t < nnz; t++) top = std::max(top, (size_t)Xr_indices[t]);
+    if (nnz && top >= n) return 2;
+    return 0;
+}
+
+// The fold-in and the ranking, B = dB [n x ldf] on `device`.  Bsum_used = Bsum + l1 (in real, when l1 > 0).
+template <class real, class IX>
+static int topn_new_impl(real* dB, size_t n, int k, int device, const real* Bsum, const real* Amean, double l1,
+                         const real* Xr, const IX* Xr_indptr, const IX* Xr_indices, size_t n_new, const pmf_b200_params& p,
+                         const IX* excl_ptr, const IX* excl_ix, const IX* incl_ptr, const IX* incl_ix, IX* outp_ix,
+                         real* outp_score, size_t n_top, real* A_out)
+{
+    if (n_new == 0) return 0;
+    std::vector<real> bs(Bsum, Bsum + k);
+    const real l1r = (real)l1;
+    if (l1r > (real)0) for (int c = 0; c < k; c++) bs[c] += l1r;
+    HandleT<real> fold;                   // the new users' rows against the bound B: only A and the CSR are allocated
+    fold.dtype = std::is_same<real, float>::value ? PMF_F32 : PMF_F64;
+    fold.device = device; fold.dimA = n_new; fold.dimB = n; fold.k = k;
+    if (fold.init(dB)) return 1;
+    const size_t nnz = (size_t)(Xr_indptr[n_new] - Xr_indptr[0]);
+    if (fold.set_matrix(PMF_SIDE_CSR, Xr, Xr_indptr, Xr_indices, nnz, (int)sizeof(IX), 0, n_new)) return 1;
+    pmf_b200_params q = p;                // as pmf_b200_factors_multiple passes them; reuse_prev is reuse_mean
+    q.l1_reg = 0; q.early_stop = 0; q.reuse_prev = 0;
+    if (fold.factors_multiple(nullptr, bs.data(), Amean, q, p.reuse_prev)) return 1;
+    if (outp_ix) {
+        const ResidentFactors rf = {fold.A, dB, device, fold.ldf};
+        const int rc = (incl_ptr || incl_ix)
+            ? topn_include_impl<real, IX>(nullptr, nullptr, k, nullptr, n_new, n_new, incl_ptr, incl_ix, outp_ix,
+                                          outp_score, n_top, n, &rf)
+            : topn_batch_impl<real, IX>(nullptr, nullptr, k, nullptr, n_new, n_new, excl_ptr, excl_ix, outp_ix,
+                                        outp_score, n_top, n, true, &rf);
+        if (rc) return rc;
+    }
+    return A_out ? fold.get_factors(A_out, nullptr) : 0;
+}
+
+extern "C" int pmf_b200_topN_new_batch(int dtype, int index_bytes, const void* B, const void* Bsum, const void* Amean,
+                                       int k, size_t n, const void* Xr, const void* Xr_indptr, const void* Xr_indices,
+                                       size_t n_new, const pmf_b200_params* p,
+                                       const void* excl_ptr, const void* excl_ix, const void* incl_ptr,
+                                       const void* incl_ix, void* outp_ix, void* outp_score, size_t n_top, void* A_out)
+{
+    if (pmf_b200_device_count() <= 0) return fail("no usable CUDA device: poismf_b200 has no CPU fallback");
+    return with_types(dtype, index_bytes, "topN_new_batch: bad dtype/index width", [&](auto r, auto i) {
+        using real = decltype(r); using IX = decltype(i);
+        if (!B || !Bsum || !Amean || k < 1 || k > 256) return 2;
+        if (const int bad = check_new_users<IX>(Xr, (const IX*)Xr_indptr, (const IX*)Xr_indices, n_new, n, p, excl_ptr,
+                                                excl_ix, incl_ptr, incl_ix, outp_ix, n_top, A_out)) return bad;
+        if (n_new == 0) return 0;
+        const int device = env_device();
+        CK(cudaSetDevice(device));
+        DeviceBlocks mem;
+        real* dB = nullptr;
+        bool resident = false;
+        if (upload_rows<real>(&dB, (const real*)B, n, k, round_up(k, RealTraits<real>::V), &resident, true)) return 1;
+        if (!resident) mem.adopt(dB);
+        const int rc = topn_new_impl<real, IX>(dB, n, k, device, (const real*)Bsum, (const real*)Amean, p->l1_reg,
+                                               (const real*)Xr, (const IX*)Xr_indptr, (const IX*)Xr_indices, n_new, *p,
+                                               (const IX*)excl_ptr, (const IX*)excl_ix, (const IX*)incl_ptr,
+                                               (const IX*)incl_ix, (IX*)outp_ix, (real*)outp_score, n_top, (real*)A_out);
+        mem.settled = rc != 1;
+        return rc;
+    });
+}
+
+extern "C" int pmf_b200_topN_new_fitted(pmf_b200_handle* h, int index_bytes, const void* Bsum, const void* Amean,
+                                        const void* Xr, const void* Xr_indptr, const void* Xr_indices, size_t n_new,
+                                        const pmf_b200_params* p,
+                                        const void* excl_ptr, const void* excl_ix, const void* incl_ptr,
+                                        const void* incl_ix, void* outp_ix, void* outp_score, size_t n_top, void* A_out)
+{
+    if (!h) return fail("topN_new_fitted: null handle");
+    if (pmf_b200_sync(h)) return 1;             // every row of the last half-sweep (own and peers') has landed
+    return with_types(h->dtype, index_bytes, "topN_new_fitted: bad dtype/index width", [&](auto r, auto i) {
+        using real = decltype(r); using IX = decltype(i);
+        const size_t n = h->dimB;
+        const int k = h->k;
+        if (const int bad = check_new_users<IX>(Xr, (const IX*)Xr_indptr, (const IX*)Xr_indices, n_new, n, p, excl_ptr,
+                                                excl_ix, incl_ptr, incl_ix, outp_ix, n_top, A_out)) return bad;
+        real* dB = (real*)h->factor_ptr(1);
+        if (!dB) return fail("topN_new_fitted: the handle holds no factors");
+        std::vector<real> stats;
+        if (!Bsum || !Amean) {
+            stats.resize(2 * (size_t)k);
+            if (fit_stats_impl<real>((const real*)h->factor_ptr(0), h->dimA, dB, n, k, h->ldf, h->device, 0.0,
+                                     stats.data(), stats.data() + k)) return 1;
+        }
+        return topn_new_impl<real, IX>(dB, n, k, h->device, Bsum ? (const real*)Bsum : stats.data(),
+                                       Amean ? (const real*)Amean : stats.data() + k, p->l1_reg, (const real*)Xr,
+                                       (const IX*)Xr_indptr, (const IX*)Xr_indices, n_new, *p, (const IX*)excl_ptr,
+                                       (const IX*)excl_ix, (const IX*)incl_ptr, (const IX*)incl_ix, (IX*)outp_ix,
+                                       (real*)outp_score, n_top, (real*)A_out);
+    });
+}
+
+extern "C" int pmf_b200_fit_stats(pmf_b200_handle* h, double l1_reg, void* Bsum_out, void* Amean_out)
+{
+    if (!h) return fail("fit_stats: null handle");
+    if (!Bsum_out && !Amean_out) return 2;
+    if (pmf_b200_sync(h)) return 1;
+    return with_types(h->dtype, 8, "fit_stats: bad dtype", [&](auto r, auto) {
+        using real = decltype(r);
+        return fit_stats_impl<real>((const real*)h->factor_ptr(0), h->dimA, (const real*)h->factor_ptr(1), h->dimB,
+                                    h->k, h->ldf, h->device, l1_reg, (real*)Bsum_out, (real*)Amean_out);
     });
 }

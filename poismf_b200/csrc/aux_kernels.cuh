@@ -107,6 +107,18 @@ __global__ void colsum_fold_kernel(const real* __restrict__ partial, int nparts,
     out[c] = colsum_finish(acc, fin);
 }
 
+// every row of M [n x ldf] := mean [k] (pads zero), or zero without `mean`: the starting point of the rows
+// of factors_multiple (src/pred.c:144-147)
+template <class real>
+__global__ void fill_rows_kernel(real* __restrict__ M, size_t n, int k, int ldf, const real* __restrict__ mean)
+{
+    const size_t total = n * (size_t)ldf;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const int c = (int)(i % (size_t)ldf);
+        M[i] = (mean && c < k) ? mean[c] : (real)0;
+    }
+}
+
 template <class real>
 __global__ void zero_rows_kernel(real* __restrict__ M, const int* __restrict__ rows, int nrows, int ldf)
 {

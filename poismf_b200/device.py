@@ -91,6 +91,45 @@ class DeviceFit:
         self._ck(rc)
         return ids, sc
 
+    def fit_stats(self, l1_reg=0.0):
+        """(Bsum, Amean) of the resident factors: column sums of B plus l1_reg, column means of A — the attributes
+        PoisMF keeps after a fit (pmf_b200_fit_stats; fixed summation order, the same bits on every replica)."""
+        Bsum, Amean = np.empty(self.k, self.dtype), np.empty(self.k, self.dtype)
+        self._ck(self.L.pmf_b200_fit_stats(self.h, float(l1_reg), _lib.ptr(Bsum), _lib.ptr(Amean)))
+        return Bsum, Amean
+
+    def _new_users(self, Xr_indptr, Xr_indices, Xr, params, Bsum, Amean, **kw):
+        from .c_funs import _new_users
+        Bs = None if Bsum is None else np.ascontiguousarray(Bsum, dtype=self.dtype)
+        Am = None if Amean is None else np.ascontiguousarray(Amean, dtype=self.dtype)
+
+        def call(ib, *args):
+            return self.L.pmf_b200_topN_new_fitted(self.h, ib, _lib.ptr(Bs), _lib.ptr(Am), *args)
+        return _new_users(call, Xr_indptr, Xr_indices, Xr, self.k, self.dtype, params, **kw)
+
+    def topN_new(self, Xr_indptr, Xr_indices, Xr, top_n=10, output_score=False, excl_ptr=None, excl_ix=None,
+                 incl_ptr=None, incl_ix=None, reuse_mean=True, maxupd=20, l2_reg=1e5, l1_new=0.0, l1_old=0.0,
+                 w_mult=1.0, return_factors=False, flags=0, Bsum=None, Amean=None, l1_reg=0.0):
+        """c_funs._topN_new_batch against the item factors resident in this handle (pmf_b200_topN_new_fitted): the new
+        users' CSR rows are folded in and ranked without B leaving the device.  With Bsum=None the column sums come
+        from the resident B and the model's total `l1_reg` is added to them; with the model's Bsum given, the positive
+        part of l1_new - l1_old is (as in `_predict_factors`).  Amean=None: the column means of the resident A."""
+        from .c_funs import _positive_l1
+        l1 = float(self.dtype.type(l1_reg)) if Bsum is None else _positive_l1(self.dtype, l1_new, l1_old)
+        params = _lib.make_params("tncg", l2_reg, l1_reg=l1, w_mult=w_mult, step_size=0.0, numiter=1, maxupd=maxupd,
+                                  reuse_prev=reuse_mean, flags=flags)
+        return self._new_users(Xr_indptr, Xr_indices, Xr, params, Bsum, Amean, top_n=top_n, output_score=output_score,
+                               excl_ptr=excl_ptr, excl_ix=excl_ix, incl_ptr=incl_ptr, incl_ix=incl_ix,
+                               return_factors=return_factors)
+
+    def transform(self, Xr_indptr, Xr_indices, Xr, method="tncg", niter=10, maxupd=1, l2_reg=1e9, w_mult=1.0,
+                  step_size=1e-7, limit_step=False, reuse_mean=True, Bsum=None, Amean=None, flags=0):
+        """Factors of new users' CSR rows against the resident item factors (PoisMF.transform): the fold-in of
+        c_funs._predict_factors_multiple (same keywords) with B read in place.  Bsum / Amean default to fit_stats()."""
+        params = _lib.make_params(method, l2_reg, w_mult=w_mult, step_size=step_size, limit_step=limit_step,
+                                  numiter=niter, maxupd=maxupd, reuse_prev=reuse_mean, flags=flags)
+        return self._new_users(Xr_indptr, Xr_indices, Xr, params, Bsum, Amean, rank=False)
+
     def factor_ptr(self, which):
         return self.L.pmf_b200_factor_ptr(self.h, which)
 

@@ -281,11 +281,58 @@ class GpuBackend:
                             excl_ix=excl_ix, output_score=output_score, rank=self.rank, world=self.world,
                             group=self.group, scorer=scorer, gather=gather, incl_ptr=incl_ptr, incl_ix=incl_ix)
 
+    def topN_new(self, Xr_indptr, Xr_indices, Xr, top_n=10, excl_ptr=None, excl_ix=None, incl_ptr=None, incl_ix=None,
+                 gather=True, **kw):
+        """DeviceFit.topN_new with the new users split across the ranks (new_users_sharded): every rank folds in and
+        ranks its share against ITS replicas; returns (ids, scores) or, with return_factors=True, (ids, scores, A)."""
+
+        def fold(csr, p_, i_, include):
+            lists = dict(incl_ptr=p_, incl_ix=i_) if include else dict(excl_ptr=p_, excl_ix=i_)
+            return self.fit.topN_new(csr[1], csr[2], csr[0], top_n=top_n, **lists, **kw)
+        return new_users_sharded((Xr, Xr_indptr, Xr_indices), fold, self.rank, self.world, self.group, excl_ptr,
+                                 excl_ix, incl_ptr, incl_ix, gather)
+
+    def transform(self, Xr_indptr, Xr_indices, Xr, gather=True, **kw):
+        """DeviceFit.transform with the new users split across the ranks; returns their factors."""
+        return new_users_sharded((Xr, Xr_indptr, Xr_indices),
+                                 lambda csr, p_, i_, include: (self.fit.transform(csr[1], csr[2], csr[0], **kw),),
+                                 self.rank, self.world, self.group, gather=gather)[0]
+
 
 def user_ranges(n_users, nparts):
     """Contiguous, near-equal user ranges (topN work per user is the same: n items x k)."""
     cuts = [n_users * p // nparts for p in range(nparts + 1)]
     return [(cuts[i], cuts[i + 1]) for i in range(nparts)]
+
+
+def _slice_lists(ptr, ix, lo, hi):
+    """The per-user lists of users [lo, hi) as (offsets rebased to 0, ids), uint64; (None, None) without lists."""
+    if ptr is None or ix is None:
+        return None, None
+    ep = np.asarray(ptr).astype(np.int64)
+    return (np.ascontiguousarray(ep[lo:hi + 1] - ep[lo]).astype(np.uint64),
+            np.ascontiguousarray(np.asarray(ix)[ep[lo]:ep[hi]]).astype(np.uint64))
+
+
+def new_users_sharded(csr, fold, rank=0, world=1, group=None, excl_ptr=None, excl_ix=None, incl_ptr=None,
+                      incl_ix=None, gather=True):
+    """New users (CSR rows `csr` = (values, indptr, indices)) split across ranks: rank r folds in and ranks the
+    contiguous range user_ranges(n_new, world)[r] against its own replicas, and the per-user results are all-gathered
+    (with gather=False a rank returns its own range only).  Exclusion or include lists are sliced by the same range.
+    `fold(csr_slice, list_ptr, list_ix, include) -> tuple of arrays with one row per user of the slice` does the
+    work (GpuBackend.topN_new / transform pass the resident handle's; the CPU tests inject a stand-in)."""
+    include = incl_ptr is not None or incl_ix is not None
+    if include and (excl_ptr is not None or excl_ix is not None):
+        raise ValueError("topN: include and exclude lists cannot be combined")
+    lo, hi = user_ranges(csr[1].shape[0] - 1, world)[rank]
+    p_loc, i_loc = _slice_lists(*((incl_ptr, incl_ix) if include else (excl_ptr, excl_ix)), lo, hi)
+    out = tuple(fold(slice_compressed(csr, lo, hi), p_loc, i_loc, include))
+    if world == 1 or not gather:
+        return out
+    import torch.distributed as dist
+    parts = [None] * world
+    dist.all_gather_object(parts, out, group=group)
+    return tuple(np.concatenate([p[j] for p in parts], axis=0) for j in range(len(out)))
 
 
 def topn_sharded(A, B, top_n, users=None, excl_ptr=None, excl_ix=None, output_score=False, rank=0, world=1,
@@ -312,12 +359,7 @@ def topn_sharded(A, B, top_n, users=None, excl_ptr=None, excl_ix=None, output_sc
     all_users = np.arange(A.shape[0], dtype=np.uint64) if users is None else np.ascontiguousarray(users, dtype=np.uint64)
     lo, hi = user_ranges(all_users.shape[0], world)[rank]
     mine = np.ascontiguousarray(all_users[lo:hi])
-    p_loc = i_loc = None
-    lists = (incl_ptr, incl_ix) if include else (excl_ptr, excl_ix)
-    if lists[0] is not None and lists[1] is not None:
-        ep = np.asarray(lists[0]).astype(np.int64)
-        p_loc = np.ascontiguousarray(ep[lo:hi + 1] - ep[lo]).astype(np.uint64)
-        i_loc = np.ascontiguousarray(np.asarray(lists[1])[ep[lo]:ep[hi]]).astype(np.uint64)
+    p_loc, i_loc = _slice_lists(*((incl_ptr, incl_ix) if include else (excl_ptr, excl_ix)), lo, hi)
     if hi > lo:
         if include:
             ids, sc = scorer(A, B, mine, p_loc, i_loc, top_n, output_score, include=True)
