@@ -147,25 +147,14 @@ static int launch_column_sums(const real* M, size_t nrow, int k, int ldf, const 
 // ---------------------------------------------------------------------------
 // one orientation (CSR or CSC) of the count matrix on the device + its row plan
 // ---------------------------------------------------------------------------
-struct Bin {
-    bool block = false;     // CTA per row (else warp per row)
-    int cluster = 1;        // > 1: a thread-block cluster of this many CTAs per row
-    int width = 32;         // lanes per row for the warp-level bins
-    int cap = 0;            // staged tile capacity; 0 = tile stays in global memory
-    int acap = -1;          // capacity of the per-non-zero arrays kept in shared memory (-1: == cap)
-    int threads = 256;
-    int rt_nw = 0, rt_tpl = 0, rt_nc = 0;   // > 0: register-tile bin (regtile.cuh): warps per row, tile rows and chunks per lane
-    size_t slice = 0, smem = 0;
-    std::vector<int> rows;  // local row ids, longest first
-    int* d_rows = nullptr;
-    long long max_nnz = 0;
-    unsigned long long nnz = 0;
+struct Bin : PlannedBin {
+    int* d_rows = nullptr;         // device copy of `rows`
     std::vector<cudaEvent_t> ev;   // profiling: start/stop pairs of this bin's launches
 };
 
 // the heaviest rows of a side, solved in lock-step by the whole GPU (dense_rows.cuh)
 struct DensePlan {
-    int H = 0, T = 0, U = 256, nnzH = 0, nchunks = 0, G = 0;
+    int H = 0, T = 0, nnzH = 0, nchunks = 0, G = 0;
     unsigned long long nnz = 0;
     std::vector<int> rows;                 // local row ids, heaviest first
     void* blocks[20] = {};                 // every device allocation below, for release
@@ -198,7 +187,6 @@ template <class real> struct Side {
     int planned_method = -1;
     int* d_empty = nullptr;
     int n_empty = 0;
-    std::vector<int> h_empty;
     int* d_all_rows = nullptr;
     real* gscratch = nullptr;
     long long gs_stride = 0;
@@ -258,10 +246,6 @@ struct pmf_b200_handle {
     virtual void clear_profile() = 0;
     bool profiling = false;
 };
-
-static const size_t SMEM_PER_SM = 233472;     // 228 KB
-static const size_t SMEM_CTA_MAX = 232448;    // 227 KB opt-in maximum per CTA
-static const size_t SMEM_CTA_RESERVED = 1024; // per-CTA system reservation
 
 template <class real> struct HandleT : pmf_b200_handle {
     real *A = nullptr, *B = nullptr;
@@ -491,54 +475,40 @@ template <class real> struct HandleT : pmf_b200_handle {
     }
     void* factor_ptr(int which) override { return which == 0 ? (void*)A : (void*)B; }
 
-    // ---- planner: bin the local rows of one side by non-zero count -------------
-    // (sub-)warp teams need no reduction scratch: their 640 bytes go to the tile instead
-    size_t slice_bytes(int team_threads, int nvec, int cap) const
-    {
-        size_t b = (team_threads > 32 ? 640 : 0) + (size_t)team_threads * 16 + (size_t)nvec * kp * sizeof(real) +
-                   (size_t)4 * cap * sizeof(real) + (size_t)cap * kp * sizeof(real);
-        return round_up_sz(b, 16);
-    }
     // ---- lock-step path for the heaviest rows (dense_rows.cuh) ------------------------------------
-    // returns 0: built, 1: error, 2: not applicable (sizes out of range)
-    std::vector<long long> dn_hbeg;
-    std::vector<int> dn_i32;
     int build_dense(Side<real>& S, const std::vector<int>& hrows, size_t other, cudaStream_t st)
     {
         DensePlan& D = S.dense;
         D.release();
         const int H = (int)hrows.size();
-        int U = DN_TILE_ROWS;
-        if (const char* e = getenv("POISMF_B200_DENSE_TILE")) U = std::min(DN_TILE_ROWS, std::max(16, atoi(e)));   // tuning
+        const int U = DN_TILE_ROWS;
         const long long T = ((long long)other + U - 1) / U;
         long long nnzH = 0;
         for (int r : hrows) nnzH += S.h_ptr[r + 1] - S.h_ptr[r];
-        if (nnzH >= (1LL << 31) || T * H >= (1LL << 32) || S.nnz >= ((size_t)1 << 31)) return 2;
-        D.H = H; D.U = U; D.T = (int)T; D.nnzH = (int)nnzH; D.nnz = (unsigned long long)nnzH; D.rows = hrows;
+        D.H = H; D.T = (int)T; D.nnzH = (int)nnzH; D.nnz = (unsigned long long)nnzH; D.rows = hrows;
         D.G = (int)std::min<long long>(num_sms, T);         // persistent CTAs of the gaxpy pass
         // host tables: [hrow H][hcol0 H+1][chunk_ptr H+1][chunk_h nchunks]
-        dn_hbeg.resize(H);
+        std::vector<long long> hbeg(H);
         std::vector<int> hcol0(H + 1, 0), chunk_ptr(H + 1, 0);
         for (int h = 0; h < H; h++) {
             const long long n = S.h_ptr[hrows[h] + 1] - S.h_ptr[hrows[h]];
-            dn_hbeg[h] = S.h_ptr[hrows[h]];
+            hbeg[h] = S.h_ptr[hrows[h]];
             hcol0[h + 1] = hcol0[h] + (int)n;
             chunk_ptr[h + 1] = chunk_ptr[h] + (int)((n + DN_LS_CHUNK - 1) / DN_LS_CHUNK);
         }
         D.nchunks = chunk_ptr[H];
-        dn_i32.clear();
-        dn_i32.insert(dn_i32.end(), hrows.begin(), hrows.end());
-        dn_i32.insert(dn_i32.end(), hcol0.begin(), hcol0.end());
-        dn_i32.insert(dn_i32.end(), chunk_ptr.begin(), chunk_ptr.end());
+        std::vector<int> i32(hrows);
+        i32.insert(i32.end(), hcol0.begin(), hcol0.end());
+        i32.insert(i32.end(), chunk_ptr.begin(), chunk_ptr.end());
         for (int h = 0; h < H; h++)
-            for (int c = chunk_ptr[h]; c < chunk_ptr[h + 1]; c++) dn_i32.push_back(h);
+            for (int c = chunk_ptr[h]; c < chunk_ptr[h + 1]; c++) i32.push_back(h);
         auto grab = [&](auto** ptr, size_t bytes) -> int {
             CK(dmalloc(ptr, std::max<size_t>(bytes, 16)));
             D.blocks[D.nblocks++] = (void*)*ptr;
             return 0;
         };
         int* tables = nullptr;
-        if (grab(&tables, dn_i32.size() * sizeof(int))) return 1;
+        if (grab(&tables, i32.size() * sizeof(int))) return 1;
         D.hrow = tables; D.hcol0 = tables + H; D.chunk_ptr = D.hcol0 + H + 1; D.chunk_h = D.chunk_ptr + H + 1;
         if (grab(&D.hbeg, (size_t)H * sizeof(long long))) return 1;
         if (grab(&D.ent, (size_t)nnzH * sizeof(uint2))) return 1;
@@ -553,8 +523,8 @@ template <class real> struct HandleT : pmf_b200_handle {
         if (grab(&D.lsp, (size_t)D.nchunks * DN_TRIALS * sizeof(float))) return 1;
         if (grab(&D.sc, (size_t)H * sizeof(DenseScal))) return 1;
         if (grab(&D.tile_counters, 64 * sizeof(int))) return 1;
-        CK(cudaMemcpyAsync(tables, dn_i32.data(), dn_i32.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(D.hbeg, dn_hbeg.data(), (size_t)H * sizeof(long long), cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(tables, i32.data(), i32.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(D.hbeg, hbeg.data(), (size_t)H * sizeof(long long), cudaMemcpyHostToDevice, st));
         CK(cudaMemsetAsync(D.q, 0, (size_t)nnzH * sizeof(float), st));
         // sort the heavy rows' non-zeros by (tile of the fixed matrix, heavy row); stable: ascending position inside
         int *slot = nullptr, *pos = nullptr, *spos = nullptr;
@@ -588,300 +558,117 @@ template <class real> struct HandleT : pmf_b200_handle {
     // one half-sweep of the heavy rows: ~5 launches per cg iteration, all on `st`
     int run_dense(Side<real>& S, real* M, const real* F, const HalfSweepConsts<real>& hc, int which_factor, cudaStream_t st)
     {
-        return run_dense_impl(S, M, F, hc, which_factor, st);
-    }
-    int run_dense_impl(Side<float>& S, float* M, const float* F, const HalfSweepConsts<float>& hc, int which_factor,
-                       cudaStream_t st)
-    {
-        DensePlan& D = S.dense;
-        DenseParams P;
-        P.H = D.H; P.T = D.T; P.U = D.U; P.ldf = ldf; P.k = k; P.L = ldf / 4;
-        P.nnzH = D.nnzH; P.nchunks = D.nchunks; P.G = D.G;
-        P.R = (int)(which_factor == 0 ? dimB : dimA);
-        P.F = F; P.M = M + S.row_begin * (size_t)ldf; P.xv = S.xv; P.csum = csum;
-        P.hrow = D.hrow; P.hbeg = D.hbeg; P.hcol0 = D.hcol0; P.ent = D.ent; P.sx = D.sx;
-        P.seg_ptr = D.seg_ptr; P.chunk_h = D.chunk_h; P.chunk_ptr = D.chunk_ptr;
-        P.p = D.p; P.q = D.q; P.dvec = D.dvec; P.gprev = D.gprev; P.dprev = D.dprev; P.gpart = D.gpart; P.lsp = D.lsp;
-        P.sc = D.sc; P.hc = hc;
-        P.npeers = npeers[which_factor];
-        for (int q = 0; q < 7; q++)
-            P.peerM[q] = q < P.npeers ? peer[which_factor][q] + S.row_begin * (size_t)ldf : nullptr;
-        const size_t tile_bytes = (size_t)D.U * ldf * sizeof(float);
-        const size_t smem_dots = tile_bytes + (size_t)D.H * sizeof(int);
-        const size_t smem_g = 2 * tile_bytes + (size_t)(D.H + DN_GROUPS) * ldf * sizeof(float);
-        {
-            static std::mutex mu;
-            static std::map<int, std::pair<size_t, size_t>> done;      // per device: the attribute is a per-kernel maximum
-            std::lock_guard<std::mutex> lk(mu);
-            auto it = done.find(device);
-            if (it == done.end() || it->second.first < smem_dots || it->second.second < smem_g) {
-                CK(cudaFuncSetAttribute(dense_walk_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_dots));
-                CK(cudaFuncSetAttribute(dense_walk_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_dots));
-                CK(cudaFuncSetAttribute(dense_walk_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_g));
-                done[device] = std::make_pair(smem_dots, smem_g);
-            }
-        }
-        const int hg = (D.H + 3) / 4;
-        const int gd = (int)std::min<long long>(4 * num_sms, D.T);   // dots passes: four persistent CTAs per SM
-        CK(cudaMemsetAsync(D.tile_counters, 0, 64 * sizeof(int), st));
-        int n_dots = 0;
-        dense_reset_kernel<<<(D.H + 127) / 128, 128, 0, st>>>(P);
-        P.tile_counter = D.tile_counters + (n_dots++ & 63);
-        dense_walk_kernel<0><<<gd, DnWalk<0>::threads, smem_dots, st>>>(P);
-        dense_ls_kernel<<<D.nchunks, 256, 0, st>>>(P, 0);
-        dense_init_kernel<<<hg, 128, 0, st>>>(P);
-        g_launches.fetch_add(4, std::memory_order_relaxed);
-        const long long maxiter = hc.maxupd <= 0 ? (1LL << 40) : hc.maxupd;
-        for (long long it = 0; it < maxiter; it++) {
-            dense_walk_kernel<2><<<D.G, DnWalk<2>::threads, smem_g, st>>>(P);
-            dense_k_kernel<<<D.H, 256, 0, st>>>(P);
-            if ((n_dots & 63) == 0) CK(cudaMemsetAsync(D.tile_counters, 0, 64 * sizeof(int), st));   // all 64 used up
+        if constexpr (!std::is_same<real, float>::value) {
+            return fail("lock-step path is float32 only");
+        } else {
+            DensePlan& D = S.dense;
+            DenseParams P;
+            P.H = D.H; P.T = D.T; P.U = DN_TILE_ROWS; P.ldf = ldf; P.k = k; P.L = ldf / 4;
+            P.nnzH = D.nnzH; P.nchunks = D.nchunks; P.G = D.G;
+            P.R = (int)(which_factor == 0 ? dimB : dimA);
+            P.F = F; P.M = M + S.row_begin * (size_t)ldf; P.xv = S.xv; P.csum = csum;
+            P.hrow = D.hrow; P.hbeg = D.hbeg; P.hcol0 = D.hcol0; P.ent = D.ent; P.sx = D.sx;
+            P.seg_ptr = D.seg_ptr; P.chunk_h = D.chunk_h; P.chunk_ptr = D.chunk_ptr;
+            P.p = D.p; P.q = D.q; P.dvec = D.dvec; P.gprev = D.gprev; P.dprev = D.dprev; P.gpart = D.gpart; P.lsp = D.lsp;
+            P.sc = D.sc; P.hc = hc;
+            P.npeers = npeers[which_factor];
+            for (int q = 0; q < 7; q++)
+                P.peerM[q] = q < P.npeers ? peer[which_factor][q] + S.row_begin * (size_t)ldf : nullptr;
+            const size_t tile_bytes = (size_t)DN_TILE_ROWS * ldf * sizeof(float);
+            const size_t smem_dots = tile_bytes + (size_t)D.H * sizeof(int);
+            const size_t smem_g = 2 * tile_bytes + (size_t)(D.H + DN_GROUPS) * ldf * sizeof(float);
+            CK(ensure_smem((const void*)dense_walk_kernel<0>, smem_dots));
+            CK(ensure_smem((const void*)dense_walk_kernel<1>, smem_dots));
+            CK(ensure_smem((const void*)dense_walk_kernel<2>, smem_g));
+            const int hg = (D.H + 3) / 4;
+            const int gd = (int)std::min<long long>(4 * num_sms, D.T);   // dots passes: four persistent CTAs per SM
+            CK(cudaMemsetAsync(D.tile_counters, 0, 64 * sizeof(int), st));
+            int n_dots = 0;
+            dense_reset_kernel<<<(D.H + 127) / 128, 128, 0, st>>>(P);
             P.tile_counter = D.tile_counters + (n_dots++ & 63);
-            dense_walk_kernel<1><<<gd, DnWalk<1>::threads, smem_dots, st>>>(P);
-            dense_ls_kernel<<<D.nchunks, 256, 0, st>>>(P, 1);
-            dense_choose_kernel<<<hg, 128, 0, st>>>(P);
-            g_launches.fetch_add(5, std::memory_order_relaxed);
-            if ((it & 7) == 7 && it + 1 < maxiter) {
-                // long iteration budgets (factors_multiple's cg): stop enqueueing once every row is done
-                std::vector<DenseScal> hs(D.H);
-                CK(cudaMemcpyAsync(hs.data(), D.sc, (size_t)D.H * sizeof(DenseScal), cudaMemcpyDeviceToHost, st));
-                CK(cudaStreamSynchronize(st));
-                bool any = false;
-                for (auto& q : hs) any = any || q.active;
-                if (!any) break;
+            dense_walk_kernel<0><<<gd, DnWalk<0>::threads, smem_dots, st>>>(P);
+            dense_ls_kernel<<<D.nchunks, 256, 0, st>>>(P, 0);
+            dense_init_kernel<<<hg, 128, 0, st>>>(P);
+            g_launches.fetch_add(4, std::memory_order_relaxed);
+            const long long maxiter = hc.maxupd <= 0 ? (1LL << 40) : hc.maxupd;
+            for (long long it = 0; it < maxiter; it++) {
+                dense_walk_kernel<2><<<D.G, DnWalk<2>::threads, smem_g, st>>>(P);
+                dense_k_kernel<<<D.H, 256, 0, st>>>(P);
+                if ((n_dots & 63) == 0) CK(cudaMemsetAsync(D.tile_counters, 0, 64 * sizeof(int), st));   // all 64 used up
+                P.tile_counter = D.tile_counters + (n_dots++ & 63);
+                dense_walk_kernel<1><<<gd, DnWalk<1>::threads, smem_dots, st>>>(P);
+                dense_ls_kernel<<<D.nchunks, 256, 0, st>>>(P, 1);
+                dense_choose_kernel<<<hg, 128, 0, st>>>(P);
+                g_launches.fetch_add(5, std::memory_order_relaxed);
+                if ((it & 7) == 7 && it + 1 < maxiter) {
+                    // long iteration budgets (factors_multiple's cg): stop enqueueing once every row is done
+                    std::vector<DenseScal> hs(D.H);
+                    CK(cudaMemcpyAsync(hs.data(), D.sc, (size_t)D.H * sizeof(DenseScal), cudaMemcpyDeviceToHost, st));
+                    CK(cudaStreamSynchronize(st));
+                    bool any = false;
+                    for (auto& q : hs) any = any || q.active;
+                    if (!any) break;
+                }
             }
+            CK(cudaGetLastError());
+            return 0;
         }
-        CK(cudaGetLastError());
-        return 0;
-    }
-    int run_dense_impl(Side<double>&, double*, const double*, const HalfSweepConsts<double>&, int, cudaStream_t)
-    {
-        return fail("lock-step path is float32 only");
     }
 
-    // Register-tile kernels (regtile.cuh) take the rows of up to 512 non-zeros when the fit is float32 in
-    // fast numerics with w_mult == 1 and k <= 64: pg, and cg with limit_step and the cached line search.
-    bool regtile_ok(const pmf_b200_params& p) const
+    // the planner's inputs for the parameters of a half-sweep (row_plan.h)
+    PlanMode plan_mode(const pmf_b200_params& p) const
     {
-        if (!std::is_same<real, float>::value || (p.flags & PMF_FLAG_STRICT) || (real)p.w_mult != (real)1) return false;
-        if (ldf > 64 || getenv("POISMF_B200_NO_REGTILE")) return false;
-        if (p.method == PMF_PG) return true;
-        return p.method == PMF_CG && p.limit_step && !(p.flags & PMF_FLAG_NO_CACHED);
+        PlanMode m;
+        m.real_size = sizeof(real); m.ldf = ldf; m.kp = kp;
+        m.method = p.method;
+        m.strict = (p.flags & PMF_FLAG_STRICT) != 0;
+        // register-tile kernels (regtile.cuh) take the rows of up to 512 non-zeros when the fit is float32 in
+        // fast numerics with w_mult == 1 and k <= 64: pg, and cg with limit_step and the cached line search
+        m.regtile = std::is_same<real, float>::value && !m.strict && (real)p.w_mult == (real)1 && ldf <= 64 &&
+                    (p.method == PMF_PG || (p.method == PMF_CG && p.limit_step && !(p.flags & PMF_FLAG_NO_CACHED)));
+        m.lockstep = !(p.flags & PMF_FLAG_NO_LOCKSTEP);
+        if (const char* e = getenv("POISMF_B200_DENSE_MIN")) m.dense_min = std::max(1LL, atoll(e));
+        if (const char* e = getenv("POISMF_B200_DENSE_MIN_TOTAL")) m.dense_min_total = atoll(e);
+        return m;
     }
     // row lists are uploaded on `st`; kernels that read them must be ordered after it
     int plan(Side<real>& S, const pmf_b200_params& p, cudaStream_t st)
     {
-        const int method = p.method;
-        const bool strict = (p.flags & PMF_FLAG_STRICT) != 0;
-        const bool rt = regtile_ok(p);
-        const int key = method * 8 + (strict ? 1 : 0) + (rt ? 2 : 0) + ((p.flags & PMF_FLAG_NO_LOCKSTEP) ? 4 : 0);
+        const PlanMode m = plan_mode(p);
+        const int key = m.method * 8 + (m.strict ? 1 : 0) + (m.regtile ? 2 : 0) + (m.lockstep ? 0 : 4);
         if (S.planned_method == key) return 0;
         if (S.planned_method >= 0) {    // re-planning for another method: the old lists may be in use
             if (sync_all()) return 1;
             S.free_plan();
         }
-        const int nvec = method == PMF_PG ? 3 : (method == PMF_CG ? 7 : TN_NUM_VECS);
-        std::vector<Bin> bins;
-        // (sub-)warp-per-row bins: {lanes per row, tile capacity}; sub-warps in fast numerics only
-        // {lanes per row, tile capacity}.  Rows in flight per SM are bounded by shared memory
-        // (tile + solver state per row), so capacities are graded finely; a full warp per row
-        // gives the shortest per-row latency, which is what bounds throughput at that occupancy.
-        // (64 = a two-warp CTA per row: from ~64 non-zeros on, shared memory leaves fewer than 16 rows
-        // in flight per SM and one warp per row no longer hides the latencies; measured on B200)
-        int wdef[12][2] = {{16, 16}, {32, 24}, {32, 32}, {32, 40}, {32, 48}, {64, 64}, {64, 80}, {64, 96},
-                           {64, 128}, {0, 0}, {0, 0}, {0, 0}};
-        if (strict) for (int c = 5; c < 9; c++) wdef[c][0] = 32;   // strict: warp and 256-thread CTA teams only
-        int nw = 9;
-        if (const char* e = getenv("POISMF_B200_WIDTHS")) {   // tuning knob: "w:cap,w:cap,..." (up to 12)
-            nw = 0;
-            const char* q = e;
-            while (*q && nw < 12) {
-                int w = 0, c = 0, used = 0;
-                if (sscanf(q, "%d:%d%n", &w, &c, &used) != 2) break;
-                wdef[nw][0] = w; wdef[nw][1] = c; nw++;
-                q += used;
-                if (*q == ',') q++;
-            }
-        }
-        if (rt) {
-            // register-tile bins: {warps per row, tile rows per lane}; capacity 8 x warps x tile rows
-            static const int rdef[11][2] = {{1, 2}, {1, 3}, {1, 4}, {2, 3}, {2, 4}, {4, 3}, {4, 4}, {8, 3}, {8, 4}, {16, 3}, {16, 4}};
-            for (int c = 0; c < 11; c++) {
-                Bin b;
-                b.block = true; b.rt_nw = rdef[c][0]; b.rt_tpl = rdef[c][1]; b.rt_nc = ldf <= 32 ? 2 : 4;
-                b.cap = 8 * b.rt_nw * b.rt_tpl; b.threads = 32 * b.rt_nw;
-                b.width = b.threads;
-                bins.push_back(b);
-            }
-            nw = 0;     // the shared-memory (sub-)warp teams are not used
-        }
-        for (int c = 0; c < nw; c++) {
-            const int width = wdef[c][0];
-            if (c > 0 && wdef[c][1] <= wdef[c - 1][1]) continue;
-            if (width == 64 || width == 128) {
-                // a small CTA (2 or 4 warps) per row: for capacities where shared memory leaves so few
-                // rows in flight per SM that one warp per row cannot hide latency
-                Bin b;
-                b.block = true; b.cap = wdef[c][1]; b.threads = width;
-                b.slice = slice_bytes(width, nvec, b.cap);
-                b.smem = b.slice;
-                if (b.smem > SMEM_CTA_MAX) continue;
-                bins.push_back(b);
-                continue;
-            }
-            if (width != 8 && width != 16 && width != 32) continue;
-            Bin b;
-            b.block = false; b.cap = wdef[c][1]; b.width = width;
-            b.slice = slice_bytes(width, nvec, b.cap);
-            // teams per CTA: whatever keeps the most rows in flight per SM under the shared-memory
-            // (228 KB / SM, 1 KB reserved per CTA) and register (80 per thread) budgets
-            int best_teams = 0, best_rows = 0;
-            for (int teams = 256 / width; teams >= 1; teams >>= 1) {
-                const size_t smem = b.slice * teams;
-                if (smem > SMEM_CTA_MAX) continue;
-                const int by_smem = (int)(SMEM_PER_SM / (smem + SMEM_CTA_RESERVED));
-                const int by_regs = 65536 / (teams * width * WARP_KERNEL_REGS);
-                const int by_thr = 2048 / std::max(teams * width, 32);
-                const int ctas = std::min(std::min(by_smem, by_regs), std::min(by_thr, 32));
-                if (ctas * teams > best_rows) { best_rows = ctas * teams; best_teams = teams; }
-            }
-            if (best_teams == 0) continue;
-            b.threads = std::max(best_teams * width, 32);
-            b.smem = b.slice * (b.threads / width);
-            bins.push_back(b);
-        }
-        // CTA-per-row bins: largest capacity with 4, 2, 1 resident CTAs per SM.  The one-per-SM
-        // bins (and the clusters below) run 512 threads per CTA: their rows are long enough to
-        // feed them, and per-row latency is what bounds these bins.
-        const int ctas[3] = {4, 2, 1};
-        int last_cap = bins.empty() ? 0 : bins.back().cap;
-        for (int c = 0; c < 3; c++) {
-            const int thr = (ctas[c] == 1 && !strict) ? 512 : 256;
-            const size_t budget = std::min(SMEM_CTA_MAX, SMEM_PER_SM / ctas[c] - SMEM_CTA_RESERVED);
-            const size_t fixed = slice_bytes(thr, nvec, 0) + 16;
-            if (budget <= fixed) continue;
-            int cap = (int)((budget - fixed) / ((size_t)(kp + 4) * sizeof(real)));
-            cap = cap / 4 * 4;
-            if (cap <= last_cap) continue;
-            Bin b;
-            b.block = true; b.cap = cap; b.threads = thr;
-            b.slice = slice_bytes(thr, nvec, cap);
-            b.smem = b.slice;
-            bins.push_back(b);
-            last_cap = cap;
-        }
-        if (!strict) {
-            // cluster-per-row bins: G CTAs stage G slices of the tile (fast numerics only)
-            const int thr = 512;
-            const size_t fixed = slice_bytes(thr, nvec, 0) + GANG_XBYTES + 16;
-            int gcap = (int)((SMEM_CTA_MAX - fixed) / ((size_t)(kp + 4) * sizeof(real)));
-            gcap = gcap / 4 * 4;
-            const int gs[4] = {2, 4, 8, 16};
-            for (int c = 0; c < 4 && gcap > 0; c++) {
-                Bin b;
-                b.block = true; b.cluster = gs[c]; b.cap = gcap; b.threads = thr;
-                b.slice = slice_bytes(thr, nvec, gcap) + GANG_XBYTES;
-                b.smem = b.slice;
-                bins.push_back(b);
-            }
-            Bin b;     // beyond 16 resident slices: 16 CTAs, each streaming its slice from L2
-            b.block = true; b.cluster = 16; b.cap = 0; b.threads = thr;
-            b.acap = 4096;   // 64 KB (float) of per-non-zero arrays on chip; two such CTAs share an SM
-            b.slice = slice_bytes(thr, nvec, 0) + GANG_XBYTES + (size_t)4 * b.acap * sizeof(real);
-            b.smem = b.slice;
-            bins.push_back(b);
-        } else {   // strict numerics: everything longer stays on one CTA, tile in global memory / L2
-            Bin b;
-            b.block = true; b.cap = 0; b.threads = 256;
-            b.slice = slice_bytes(256, nvec, 0);
-            b.smem = b.slice;
-            bins.push_back(b);
-        }
-        // the heaviest rows go to the lock-step path (dense_rows.cuh): cg under the register-tile conditions
-        std::vector<char> is_dense;
-        if (rt && method == PMF_CG && !(p.flags & PMF_FLAG_NO_LOCKSTEP) && !getenv("POISMF_B200_NO_DENSE")) {
-            long long dmin = 4096;
-            if (const char* e = getenv("POISMF_B200_DENSE_MIN")) dmin = std::max(1LL, atoll(e));
-            // shared memory of the gaxpy pass: two tiles of 256 rows + one accumulator row per heavy row
-            // (+ the per-group edge slots)
-            const size_t hmax = std::min<size_t>(1024, (SMEM_CTA_MAX - 1024) / ((size_t)ldf * sizeof(real)) - 2 * DN_TILE_ROWS - DN_GROUPS);
-            std::vector<std::pair<long long, int>> cand;
-            for (size_t r = 0; r < S.n_rows; r++) {
-                const long long n = S.h_ptr[r + 1] - S.h_ptr[r];
-                if (n >= dmin) cand.push_back({-n, (int)r});
-            }
-            std::sort(cand.begin(), cand.end());          // heaviest first, ties by row id
-            if (cand.size() > hmax) cand.resize(hmax);
-            // the lock-step phase costs ~30 launches per half-sweep whatever its size: below ~250k non-zeros the
-            // per-row cluster teams are cheaper (small shards of a multi-GPU fit, the user side of config #2)
-            long long dense_nnz = 0, dense_min_total = 250000;
-            for (auto& c : cand) dense_nnz -= c.first;
-            if (const char* e = getenv("POISMF_B200_DENSE_MIN_TOTAL")) dense_min_total = atoll(e);
-            if (dense_nnz < dense_min_total) cand.clear();
-            if (!cand.empty()) {
-                std::vector<int> hrows;
-                for (auto& c : cand) hrows.push_back(c.second);
-                const size_t other = (&S == &sides[0]) ? dimB : dimA;
-                const int rc = build_dense(S, hrows, other, st);
-                if (rc == 1) return 1;
-                if (rc == 0) {
-                    is_dense.assign(S.n_rows, 0);
-                    for (int r : hrows) is_dense[r] = 1;
-                }
-            }
-        }
-        std::vector<int>& empty = S.h_empty;
-        empty.clear();
-        for (size_t r = 0; r < S.n_rows; r++) {
-            const long long n = S.h_ptr[r + 1] - S.h_ptr[r];
-            if (n == 0) { empty.push_back((int)r); continue; }
-            if (!is_dense.empty() && is_dense[r]) continue;
-            size_t bi = 0;
-            while (bi + 1 < bins.size() && n > (long long)bins[bi].cap * bins[bi].cluster) bi++;
-            bins[bi].rows.push_back((int)r);
-            bins[bi].max_nnz = std::max(bins[bi].max_nnz, n);
-            bins[bi].nnz += (unsigned long long)n;
-        }
-        size_t total = empty.size();
-        for (auto& b : bins) {
-            // longest first; counting sort (row lengths inside a bin span a small range)
-            if (b.rows.size() > 1) {
-                const long long mx = b.max_nnz;
-                if (mx <= (1 << 22)) {
-                    std::vector<int> cnt((size_t)mx + 2, 0);
-                    for (int r : b.rows) cnt[(size_t)(mx - (S.h_ptr[r + 1] - S.h_ptr[r])) + 1]++;
-                    for (size_t i = 1; i < cnt.size(); i++) cnt[i] += cnt[i - 1];
-                    std::vector<int> sorted(b.rows.size());
-                    for (int r : b.rows) sorted[(size_t)cnt[(size_t)(mx - (S.h_ptr[r + 1] - S.h_ptr[r]))]++] = r;
-                    b.rows.swap(sorted);
-                } else {
-                    std::stable_sort(b.rows.begin(), b.rows.end(), [&](int a, int c) {
-                        return (S.h_ptr[a + 1] - S.h_ptr[a]) > (S.h_ptr[c + 1] - S.h_ptr[c]);
-                    });
-                }
-            }
-            total += b.rows.size();
-        }
+        const size_t other = (&S == &sides[0]) ? dimB : dimA;
+        RowPlan rp = plan_rows(m, S.h_ptr.data(), S.n_rows, other);
+        if (!rp.lockstep.empty() && build_dense(S, rp.lockstep, other, st)) return 1;
+        size_t total = rp.empty.size();
+        for (auto& b : rp.bins) total += b.rows.size();
         CK(dmalloc(&S.d_all_rows, std::max<size_t>(total, 1) * sizeof(int)));
         size_t off = 0;
-        for (auto& b : bins) {
+        std::vector<Bin> bins;
+        for (auto& pb : rp.bins) {
+            Bin b{std::move(pb)};
             b.d_rows = S.d_all_rows + off;
             if (!b.rows.empty())
                 CK(cudaMemcpyAsync(b.d_rows, b.rows.data(), b.rows.size() * sizeof(int), cudaMemcpyHostToDevice, st));
             off += b.rows.size();
+            bins.push_back(std::move(b));
         }
         S.d_empty = S.d_all_rows + off;
-        S.n_empty = (int)empty.size();
-        if (!empty.empty())
-            CK(cudaMemcpyAsync(S.d_empty, empty.data(), empty.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+        S.n_empty = (int)rp.empty.size();
+        if (S.n_empty)
+            CK(cudaMemcpyAsync(S.d_empty, rp.empty.data(), rp.empty.size() * sizeof(int), cudaMemcpyHostToDevice, st));
         const Bin& gb = bins.back();
         if (!gb.rows.empty()) {
             // per-CTA scratch for the three per-non-zero arrays of rows that are not staged
-            const long long per_cta = (gb.max_nnz + gb.cluster - 1) / gb.cluster;
+            const long long per_cta = (gb.max_nnz + gb.shape.cluster - 1) / gb.shape.cluster;
             S.gs_stride = (long long)round_up_sz((size_t)per_cta + 4, 4);
             // streaming clusters are compiled for two CTAs per SM: scratch for 2 x SMs CTAs
-            S.gs_ctas = gb.cluster > 1 ? 2 * num_sms
-                                       : (int)std::min<size_t>(gb.rows.size(), (size_t)num_sms);
+            S.gs_ctas = gb.shape.cluster > 1 ? 2 * num_sms
+                                             : (int)std::min<size_t>(gb.rows.size(), (size_t)num_sms);
             CK(dmalloc(&S.gscratch, (size_t)S.gs_ctas * 3 * S.gs_stride * sizeof(real)));
         }
         S.bins.swap(bins);      // the row lists' host copies stay alive in S.bins until the next plan
@@ -894,12 +681,6 @@ template <class real> struct HandleT : pmf_b200_handle {
     {
         return launch_column_sums(F, nrow, k, ldf, fin, strict, partial, n_partial, csum, stream);
     }
-
-    static cudaError_t launch_regtile(const LaunchCfg& cfg, const SideParams<float>& P)
-    {
-        return P.hc.method == M_PG ? launch_regtile_pg(cfg, P) : launch_regtile_cg(cfg, P);
-    }
-    static cudaError_t launch_regtile(const LaunchCfg&, const SideParams<double>&) { return cudaErrorInvalidConfiguration; }
 
     // ---- one half-sweep ----------------------------------------------------------
     // side CSC: update local rows of B with A fixed (src/poismf.c:510-557)
@@ -972,7 +753,7 @@ template <class real> struct HandleT : pmf_b200_handle {
         CK(cudaMemsetAsync(counters, 0, 64 * sizeof(int), stream));
         if (hc.early_stop) CK(cudaMemsetAsync(d_unchanged, 0, sizeof(unsigned long long), stream));
 
-        const bool overlap = !profiling && !getenv("POISMF_B200_SERIAL_BINS");
+        const bool overlap = !profiling;      // profiled bins run one after another, each timed on its own
         if (overlap) CK(cudaEventRecord(ev_fork, stream));
         int n_launched = 0;
         bool used[NAUX] = {};
@@ -988,17 +769,13 @@ template <class real> struct HandleT : pmf_b200_handle {
             if (profiling) { CK(cudaEventRecord(ev1, stream)); S.dense.ev.push_back(ev0); S.dense.ev.push_back(ev1); }
         }
         for (int bi = (int)S.bins.size() - 1; bi >= 0; bi--) {    // heaviest rows first
-            const Bin& b = S.bins[bi];
-            if (b.rows.empty()) continue;
+            const Bin& bin = S.bins[bi];
+            const BinShape& b = bin.shape;
+            if (bin.rows.empty()) continue;
             cudaStream_t ls = stream;
             if (overlap) {
-                static const int n_streams = []() {   // debugging: POISMF_B200_STREAMS=1..6 side streams
-                    const char* e = getenv("POISMF_B200_STREAMS");
-                    const int v = e ? atoi(e) : NAUX;
-                    return v < 1 ? 1 : (v > NAUX ? NAUX : v);
-                }();
                 // (the lock-step chain keeps aux[0] to itself: a bin queued behind it would start when it ends)
-                const int si = (S.dense.H > 0 && n_streams > 1) ? 1 + (n_launched - 1) % (n_streams - 1) : n_launched % n_streams;
+                const int si = S.dense.H > 0 ? 1 + (n_launched - 1) % (NAUX - 1) : n_launched % NAUX;
                 ls = aux[si];
                 if (!used[si]) { CK(cudaStreamWaitEvent(ls, ev_fork, 0)); used[si] = true; }
             }
@@ -1006,10 +783,10 @@ template <class real> struct HandleT : pmf_b200_handle {
             SideParams<real> P;
             P.M = M + S.row_begin * (size_t)ldf;
             P.F = F; P.xv = S.xv; P.ptr = S.ptr; P.ind = S.ind; P.csum = csum;
-            P.rows = b.d_rows; P.nrows = (int)b.rows.size();
+            P.rows = bin.d_rows; P.nrows = (int)bin.rows.size();
             P.counter = counters + bi;
             P.k = k; P.kp = kp; P.ldf = ldf; P.cap = b.cap; P.slice_bytes = (int)b.slice;
-            P.acap = b.acap < 0 ? b.cap : b.acap;
+            P.acap = b.acap;
             P.hc = hc;
             P.gscratch = b.cap == 0 ? S.gscratch : nullptr;   // rows beyond acap per CTA fall back to global arrays
             P.gs_stride = S.gs_stride;
@@ -1017,44 +794,48 @@ template <class real> struct HandleT : pmf_b200_handle {
             const int wm = updA ? 0 : 1;
             P.npeers = npeers[wm];
             for (int q = 0; q < 7; q++) P.peerM[q] = q < npeers[wm] ? peer[wm][q] + S.row_begin * (size_t)ldf : nullptr;
-            LaunchCfg cfg;
-            cfg.block_team = b.block;
-            cfg.cached = !strict && !(p.flags & PMF_FLAG_NO_CACHED);
-            cfg.threads = b.threads;
-            cfg.smem_bytes = b.smem;
-            cfg.stream = ls;
-            const int teams = b.threads / b.width;
-            cfg.needed = b.block ? P.nrows : (P.nrows + teams - 1) / teams;
-            cfg.team_width = b.width;
-            cfg.max_grid = b.cap == 0 ? S.gs_ctas / b.cluster : (1 << 30);
-            cfg.num_sms = num_sms;
-            cfg.cluster = b.cluster;
-            cfg.rt_nw = b.rt_nw; cfg.rt_tpl = b.rt_tpl; cfg.rt_nc = b.rt_nc;
-            cudaError_t e;
+            LaunchArgs la;
+            la.stream = ls;
+            const int teams = b.kind == BinKind::Warp ? b.threads / b.lanes : 1;
+            la.needed = (P.nrows + teams - 1) / teams;
+            la.max_grid = b.cap == 0 ? S.gs_ctas / b.cluster : (1 << 30);
+            la.num_sms = num_sms;
+            la.cached = !strict && !(p.flags & PMF_FLAG_NO_CACHED);
             cudaEvent_t ev0 = nullptr, ev1 = nullptr;
             if (profiling) {
                 CK(cudaEventCreate(&ev0)); CK(cudaEventCreate(&ev1));
                 CK(cudaEventRecord(ev0, stream));
             }
+            static const char* const kind_name[] = {"regtile", "warp", "cta", "cluster", "streaming"};
             {
                 char nm[96];
-                snprintf(nm, sizeof nm, "bin %s cap %d rows %d", b.rt_nw > 0 ? "regtile" : (b.cluster > 1 ? "cluster" : (b.block ? "cta" : "warp")),
-                         b.cap, P.nrows);
+                snprintf(nm, sizeof nm, "bin %s cap %d rows %d", kind_name[(int)b.kind], b.cap, P.nrows);
                 nvtxRangePushA(nm);
             }
-            if (b.rt_nw > 0)
-                e = launch_regtile(cfg, P);
-            else if (b.cluster > 1)
-                e = p.method == PMF_TNCG ? launch_gang_tn_fast<real>(cfg, P) : launch_gang_pgcg_fast<real>(cfg, P);
-            else if (p.method == PMF_TNCG)
-                e = strict ? launch_rows_tn_strict<real>(cfg, P) : launch_rows_tn_fast<real>(cfg, P);
-            else
-                e = strict ? launch_rows_pgcg_strict<real>(cfg, P) : launch_rows_pgcg_fast<real>(cfg, P);
+            cudaError_t e = cudaErrorInvalidConfiguration;
+            switch (b.kind) {
+            case BinKind::RegTile:
+                if constexpr (std::is_same<real, float>::value)
+                    e = p.method == PMF_PG ? launch_regtile_pg(b, la, P) : launch_regtile_cg(b, la, P);
+                break;
+            case BinKind::Cluster:
+            case BinKind::Streaming:
+                e = p.method == PMF_TNCG ? launch_gang_tn_fast<real>(b, la, P) : launch_gang_pgcg_fast<real>(b, la, P);
+                break;
+            case BinKind::Warp:
+            case BinKind::Cta:
+                if (p.method == PMF_TNCG)
+                    e = strict ? launch_rows_tn_strict<real>(b, la, P) : launch_rows_tn_fast<real>(b, la, P);
+                else
+                    e = strict ? launch_rows_pgcg_strict<real>(b, la, P) : launch_rows_pgcg_fast<real>(b, la, P);
+                break;
+            }
             LAUNCHED();
             nvtxRangePop();
             if (e != cudaSuccess)
-                return fail("row kernel launch failed at side %d bin %d (block %d cluster %d cap %d threads %d smem %zu): %s",
-                            side, bi, (int)b.block, b.cluster, b.cap, b.threads, b.smem, cudaGetErrorString(e));
+                return fail("row kernel launch failed at side %d bin %d (%s, lanes %d cluster %d cap %d threads %d smem %zu): %s",
+                            side, bi, kind_name[(int)b.kind], b.lanes, b.cluster, b.cap, b.threads, b.smem,
+                            cudaGetErrorString(e));
             if (profiling) {
                 CK(cudaEventRecord(ev1, stream));
                 S.bins[bi].ev.push_back(ev0); S.bins[bi].ev.push_back(ev1);
@@ -1174,8 +955,8 @@ template <class real> struct HandleT : pmf_b200_handle {
             for (auto& b : sides[sd].bins) {
                 if (b.rows.empty() || n >= max_entries) continue;
                 pmf_b200_bin_profile& o = out[n++];
-                o.side = sd; o.block_team = b.rt_nw > 0 ? 100 + b.rt_nw : (b.block ? b.cluster : -b.width);
-                o.cap = b.cap; o.nrows = (int)b.rows.size();
+                o.side = sd; o.block_team = profile_code(b.shape);
+                o.cap = b.shape.cap; o.nrows = (int)b.rows.size();
                 o.nnz = b.nnz; o.launches = b.ev.size() / 2; o.ms = 0;
                 for (size_t i = 0; i + 1 < b.ev.size(); i += 2) {
                     float ms = 0;

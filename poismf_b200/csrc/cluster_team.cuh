@@ -17,11 +17,10 @@
 #pragma once
 #include <cooperative_groups.h>
 #include "common.cuh"
+#include "sweep_consts.h"
 
 namespace pmf {
 namespace cg = cooperative_groups;
-
-constexpr int GANG_XSLOTS = 272;   // reals per exchange buffer (>= kp of any supported k, >= 16)
 
 struct ClusterTeam : BlockOps {
     double* xbuf;       // 2 * GANG_XSLOTS doubles, viewed as `real`

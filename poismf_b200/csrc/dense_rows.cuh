@@ -30,11 +30,11 @@
 // summation order over a row's non-zeros is fixed by the sort, so results are reproducible run to run.
 #pragma once
 #include "rowops.cuh"
+#include "sweep_consts.h"
 
 namespace pmf {
 
 constexpr int DN_TRIALS = 20;       // line-search trials evaluated per pass: ALL of them (max_ls of nonnegcg.c)
-constexpr int DN_TILE_ROWS = 256;   // rows of the fixed matrix per tile
 constexpr int DN_LS_CHUNK = 2048;   // non-zeros per CTA of the line-search kernel
 constexpr int DN_MAX_LS = 20, DN_MAX_NFEVAL = 150;
 
@@ -121,7 +121,7 @@ template <int MODE> struct DnWalk {
     static constexpr int nbuf = MODE == 2 ? 2 : 1;             // dots: four CTAs per SM hide each other's tile copies
     static constexpr int min_ctas = MODE == 2 ? 1 : 4;
 };
-constexpr int DN_GROUPS = DnWalk<2>::groups;
+static_assert(DnWalk<2>::groups == DN_GROUPS, "the planner sizes the gaxpy pass with DN_GROUPS");
 
 template <int MODE>
 __global__ void __launch_bounds__(DnWalk<MODE>::threads, DnWalk<MODE>::min_ctas) dense_walk_kernel(const DenseParams P)

@@ -3,24 +3,16 @@
 //
 // Replaces the OpenMP `parallel for schedule(dynamic)` row loops of the reference
 // (/root/reference/src/poismf.c:159-187 pg, :296-321 cg, :352-397 tncg).
-// Rows are binned by non-zero count on the host (HandleT::plan in api.cu); each bin is one
+// Rows are binned by non-zero count on the host (plan_rows in row_plan.h); each bin is one
 // launch of a persistent grid whose teams fetch rows from a list sorted by decreasing
 // length (longest-processing-time-first) through an atomic counter.
 #pragma once
 #include "cluster_team.cuh"
 #include "solver_pg_cg.cuh"
 #include "solver_tn.cuh"
-
-// minimum resident CTAs the (sub-)warp kernels are compiled for: caps registers at 80/thread
-// so that three 256-thread CTAs fit an SM when their shared-memory slices allow it
-#ifndef PMF_WARP_KERNEL_MIN_CTAS
-#define PMF_WARP_KERNEL_MIN_CTAS 3
-#endif
+#include "sweep_consts.h"
 
 namespace pmf {
-
-// registers per thread the (sub-)warp kernels are compiled for (see __launch_bounds__ below)
-constexpr int WARP_KERNEL_REGS = (65536 / (256 * PMF_WARP_KERNEL_MIN_CTAS)) / 8 * 8;
 
 template <class real> struct SideParams {
     real* M;               // factors being updated  [dim   x ldf]
@@ -53,7 +45,6 @@ PMF_DEVINL int num_vecs(int method)
 // Shared-memory slice of one team:
 //   [team scratch 640 B][cluster exchange 2*272*8 B (gangs only)][gscr team*16 B][vectors NV*kp]
 //   [xv,pa,pb,pc: 4*cap][tile cap*kp]
-constexpr int GANG_XBYTES = 2 * GANG_XSLOTS * 8;
 template <class real> struct Slice {
     void* team_scratch;
     void* xchg;
@@ -144,7 +135,7 @@ PMF_DEVINL void process_row(const Team& tm, const SideParams<real>& P, const Sli
     tm.sync();
 }
 
-// W lanes per row (W = 32: a warp per row; W = 8, 16: several short rows side by side in one
+// W lanes per row (W = 32: a warp per row; W = 16: two short rows side by side in one
 // warp).  Each team owns one slice of the CTA's dynamic shared memory and fetches rows from
 // the bin's list through an atomic counter.
 template <class real, int METHOD, bool STRICT, bool CACHED, int W>

@@ -20,10 +20,10 @@
 // members take every branch together.
 #pragma once
 #include "rowops.cuh"
+#include "sweep_consts.h"
 
 namespace pmf {
 
-constexpr int TN_NUM_VECS = 24;
 enum { TV_X = 0, TV_CSUM, TV_XSCALE, TV_XOFFSET, TV_OLDG, TV_G, TV_TMP, TV_DIAGB, TV_PK, TV_SK,
        TV_YK, TV_SR, TV_YR, TV_R, TV_V, TV_ZK, TV_EMAT, TV_GV, TV_W0, TV_W1, TV_W2, TV_GFULL,
        TV_PREV, TV_PIVOT };

@@ -4,164 +4,68 @@
 // kernels build in parallel with the pg/cg ones.
 //   PMF_INST_STRICT : 0/1      PMF_INST_TN : 0 (pg + cg) / 1 (tncg)
 #pragma once
-#include <map>
-#include <mutex>
-#include <tuple>
 #include "kernels.cuh"
 #include "launch.h"
 
 namespace pmf {
 
-// Persistent grid: as many CTAs as can be resident (SMs x occupancy), never more
-// than there are rows to hand out.
-// occupancy queries (and the attribute calls that go with them) are cached per
-// (kernel, block size, shared bytes, cluster size): they cost far more than a launch
-// Function attributes and occupancy are PER DEVICE: both caches carry the current device id (a
-// process may hold handles on several GPUs: pmf_b200_create(device), POISMF_B200_DEVICE).
-static std::mutex g_occ_mutex;
-static std::map<std::tuple<int, const void*, int, size_t, int>, int> g_occ_cache;
-static inline int current_device()
-{
-    int d = 0;
-    cudaGetDevice(&d);
-    return d;
-}
-
-template <class K> static int persistent_grid(K kern, const LaunchCfg& cfg)
-{
-    int occ = 1;
-    {
-        std::lock_guard<std::mutex> lk(g_occ_mutex);
-        auto key = std::make_tuple(current_device(), (const void*)kern, cfg.threads, cfg.smem_bytes, 1);
-        auto it = g_occ_cache.find(key);
-        if (it != g_occ_cache.end()) occ = it->second;
-        else {
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, cfg.threads, cfg.smem_bytes) != cudaSuccess || occ < 1)
-                occ = 1;
-            g_occ_cache[key] = occ;
-        }
-    }
-    long long g = (long long)cfg.num_sms * occ;
-    if (g > cfg.needed) g = cfg.needed;
-    if (g > cfg.max_grid) g = cfg.max_grid;
-    return g < 1 ? 1 : (int)g;
-}
-
-// cudaFuncSetAttribute(MaxDynamicSharedMemorySize): the attribute is a per-kernel maximum, so
-// it is only ever raised (bins of different tile capacity share one kernel)
-template <class K> static cudaError_t ensure_smem(K kern, size_t bytes)
-{
-    static std::map<std::pair<int, const void*>, size_t> current;
-    std::lock_guard<std::mutex> lk(g_occ_mutex);
-    const auto key = std::make_pair(current_device(), (const void*)kern);
-    auto it = current.find(key);
-    if (it != current.end() && it->second >= bytes) return cudaSuccess;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    if (e == cudaSuccess) current[key] = bytes;
-    return e;
-}
-
+// the kernel a (sub-)warp or CTA bin names; strict numerics compile 32-lane and 256-thread teams only
 template <class real, int METHOD, bool STRICT, bool CACHED>
-static cudaError_t launch_one(const LaunchCfg& cfg, const SideParams<real>& P)
+static cudaError_t launch_one(const BinShape& b, const LaunchArgs& a, const SideParams<real>& P)
 {
-    cudaError_t e;
-    if (cfg.block_team && cfg.threads == 512 && !STRICT) {
-        auto kern = rows_block_kernel<real, METHOD, STRICT, CACHED, STRICT ? 256 : 512>;
-        e = ensure_smem(kern, cfg.smem_bytes);
-        if (e != cudaSuccess) return e;
-        kern<<<persistent_grid(kern, cfg), cfg.threads, cfg.smem_bytes, cfg.stream>>>(P);
-    } else if (cfg.block_team) {
-        auto kern = rows_block_kernel<real, METHOD, STRICT, CACHED, 256>;
-        e = ensure_smem(kern, cfg.smem_bytes);
-        if (e != cudaSuccess) return e;
-        kern<<<persistent_grid(kern, cfg), cfg.threads, cfg.smem_bytes, cfg.stream>>>(P);
-    } else if (!STRICT && cfg.team_width == 8) {
-        auto kern = rows_warp_kernel<real, METHOD, STRICT, CACHED, STRICT ? 32 : 8>;
-        e = ensure_smem(kern, cfg.smem_bytes);
-        if (e != cudaSuccess) return e;
-        kern<<<persistent_grid(kern, cfg), cfg.threads, cfg.smem_bytes, cfg.stream>>>(P);
-    } else if (!STRICT && cfg.team_width == 16) {
-        auto kern = rows_warp_kernel<real, METHOD, STRICT, CACHED, STRICT ? 32 : 16>;
-        e = ensure_smem(kern, cfg.smem_bytes);
-        if (e != cudaSuccess) return e;
-        kern<<<persistent_grid(kern, cfg), cfg.threads, cfg.smem_bytes, cfg.stream>>>(P);
-    } else {
-        auto kern = rows_warp_kernel<real, METHOD, STRICT, CACHED, 32>;
-        e = ensure_smem(kern, cfg.smem_bytes);
-        if (e != cudaSuccess) return e;
-        kern<<<persistent_grid(kern, cfg), cfg.threads, cfg.smem_bytes, cfg.stream>>>(P);
+    if (b.kind == BinKind::Cta) {
+        if constexpr (!STRICT)
+            if (b.threads == 512) return launch_persistent(rows_block_kernel<real, METHOD, STRICT, CACHED, 512>, b, a, P);
+        return launch_persistent(rows_block_kernel<real, METHOD, STRICT, CACHED, 256>, b, a, P);
     }
-    return cudaGetLastError();
+    if (b.lanes == 16) {
+        if constexpr (STRICT) return cudaErrorInvalidConfiguration;
+        else return launch_persistent(rows_warp_kernel<real, METHOD, STRICT, CACHED, 16>, b, a, P);
+    }
+    return launch_persistent(rows_warp_kernel<real, METHOD, STRICT, CACHED, 32>, b, a, P);
 }
 
 #if !PMF_INST_STRICT
 // ---- cluster-per-row launch (cudaLaunchKernelEx with a cluster dimension) ----
-template <class real, int METHOD, bool CACHED, int MINB>
-static cudaError_t launch_gang_thr(const LaunchCfg& cfg, const SideParams<real>& P);
-
 template <class real, int METHOD, bool CACHED>
-static cudaError_t launch_gang_one(const LaunchCfg& cfg, const SideParams<real>& P)
+static cudaError_t launch_gang_one(const BinShape& b, const LaunchArgs& a, const SideParams<real>& P)
 {
-    // streaming (cap 0) bins are compiled for 2 CTAs per SM (64 registers) so that they can share
-    // an SM with the short-row kernels while they wait on L2
-    if (P.cap == 0) return launch_gang_thr<real, METHOD, CACHED, 2>(cfg, P);
-    return launch_gang_thr<real, METHOD, CACHED, 1>(cfg, P);
-}
-
-template <class real, int METHOD, bool CACHED, int MINB>
-static cudaError_t launch_gang_thr(const LaunchCfg& cfg, const SideParams<real>& P)
-{
-    auto kern = rows_cluster_kernel<real, METHOD, CACHED, MINB>;
-    cudaError_t e = ensure_smem(kern, cfg.smem_bytes);
+    // streaming bins are compiled for 2 CTAs per SM (64 registers) so that they can share an SM with the
+    // short-row kernels while they wait on L2
+    auto kern = b.kind == BinKind::Streaming ? rows_cluster_kernel<real, METHOD, CACHED, 2>
+                                             : rows_cluster_kernel<real, METHOD, CACHED, 1>;
+    int nclusters = 1;
+    cudaError_t e = ensure_smem((const void*)kern, b.smem);
+    if (e == cudaSuccess) e = resident(&nclusters, (const void*)kern, b.threads, b.smem, b.cluster, a.num_sms);
     if (e != cudaSuccess) return e;
+    nclusters = std::min({nclusters, a.needed, a.max_grid});
     cudaLaunchConfig_t lc = {};
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = cfg.cluster; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    at[0].val.clusterDim.x = b.cluster; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     lc.attrs = at; lc.numAttrs = 1;
-    lc.blockDim = dim3(cfg.threads); lc.dynamicSmemBytes = cfg.smem_bytes; lc.stream = cfg.stream;
-    int nclusters = 0;
-    {
-        std::lock_guard<std::mutex> lk(g_occ_mutex);
-        auto key = std::make_tuple(current_device(), (const void*)kern, cfg.threads, cfg.smem_bytes, cfg.cluster);
-        auto it = g_occ_cache.find(key);
-        if (it != g_occ_cache.end()) nclusters = it->second;
-        else {
-            if (cfg.cluster > 8) {
-                e = cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-                if (e != cudaSuccess) return e;
-            }
-            lc.gridDim = dim3(cfg.cluster);   // placeholder for the occupancy query
-            e = cudaOccupancyMaxActiveClusters(&nclusters, kern, &lc);
-            if (e != cudaSuccess || nclusters < 1) {
-                cudaGetLastError();
-                nclusters = cfg.num_sms / cfg.cluster / 2;
-                if (nclusters < 1) nclusters = 1;
-            }
-            g_occ_cache[key] = nclusters;
-        }
-    }
-    if (nclusters > cfg.needed) nclusters = cfg.needed;
-    if (nclusters > cfg.max_grid) nclusters = cfg.max_grid;
-    lc.gridDim = dim3((unsigned)(nclusters * cfg.cluster));
+    lc.gridDim = dim3((unsigned)(nclusters * b.cluster));
+    lc.blockDim = dim3(b.threads); lc.dynamicSmemBytes = b.smem; lc.stream = a.stream;
     return cudaLaunchKernelEx(&lc, kern, P);
 }
 #if PMF_INST_TN
-template <class real> cudaError_t launch_gang_tn_fast(const LaunchCfg& cfg, const SideParams<real>& P)
+template <class real>
+cudaError_t launch_gang_tn_fast(const BinShape& b, const LaunchArgs& a, const SideParams<real>& P)
 {
-    return launch_gang_one<real, M_TNCG, false>(cfg, P);
+    return launch_gang_one<real, M_TNCG, false>(b, a, P);
 }
-template cudaError_t launch_gang_tn_fast<float>(const LaunchCfg&, const SideParams<float>&);
-template cudaError_t launch_gang_tn_fast<double>(const LaunchCfg&, const SideParams<double>&);
+template cudaError_t launch_gang_tn_fast<float>(const BinShape&, const LaunchArgs&, const SideParams<float>&);
+template cudaError_t launch_gang_tn_fast<double>(const BinShape&, const LaunchArgs&, const SideParams<double>&);
 #else
-template <class real> cudaError_t launch_gang_pgcg_fast(const LaunchCfg& cfg, const SideParams<real>& P)
+template <class real>
+cudaError_t launch_gang_pgcg_fast(const BinShape& b, const LaunchArgs& a, const SideParams<real>& P)
 {
-    if (P.hc.method == M_PG) return launch_gang_one<real, M_PG, false>(cfg, P);
-    if (cfg.cached) return launch_gang_one<real, M_CG, true>(cfg, P);
-    return launch_gang_one<real, M_CG, false>(cfg, P);
+    if (P.hc.method == M_PG) return launch_gang_one<real, M_PG, false>(b, a, P);
+    if (a.cached) return launch_gang_one<real, M_CG, true>(b, a, P);
+    return launch_gang_one<real, M_CG, false>(b, a, P);
 }
-template cudaError_t launch_gang_pgcg_fast<float>(const LaunchCfg&, const SideParams<float>&);
-template cudaError_t launch_gang_pgcg_fast<double>(const LaunchCfg&, const SideParams<double>&);
+template cudaError_t launch_gang_pgcg_fast<float>(const BinShape&, const LaunchArgs&, const SideParams<float>&);
+template cudaError_t launch_gang_pgcg_fast<double>(const BinShape&, const LaunchArgs&, const SideParams<double>&);
 #endif
 #endif
 
@@ -177,18 +81,18 @@ template cudaError_t launch_gang_pgcg_fast<double>(const LaunchCfg&, const SideP
 #endif
 
 template <class real>
-cudaError_t PMF_LAUNCH_NAME(const LaunchCfg& cfg, const SideParams<real>& P)
+cudaError_t PMF_LAUNCH_NAME(const BinShape& b, const LaunchArgs& a, const SideParams<real>& P)
 {
     constexpr bool S = PMF_INST_STRICT != 0;
 #if PMF_INST_TN
-    return launch_one<real, M_TNCG, S, false>(cfg, P);
+    return launch_one<real, M_TNCG, S, false>(b, a, P);
 #else
-    if (P.hc.method == M_PG) return launch_one<real, M_PG, S, false>(cfg, P);
-    if (!S && cfg.cached) return launch_one<real, M_CG, S, true>(cfg, P);
-    return launch_one<real, M_CG, S, false>(cfg, P);
+    if (P.hc.method == M_PG) return launch_one<real, M_PG, S, false>(b, a, P);
+    if (!S && a.cached) return launch_one<real, M_CG, S, true>(b, a, P);
+    return launch_one<real, M_CG, S, false>(b, a, P);
 #endif
 }
-template cudaError_t PMF_LAUNCH_NAME<float>(const LaunchCfg&, const SideParams<float>&);
-template cudaError_t PMF_LAUNCH_NAME<double>(const LaunchCfg&, const SideParams<double>&);
+template cudaError_t PMF_LAUNCH_NAME<float>(const BinShape&, const LaunchArgs&, const SideParams<float>&);
+template cudaError_t PMF_LAUNCH_NAME<double>(const BinShape&, const LaunchArgs&, const SideParams<double>&);
 
 }  // namespace pmf

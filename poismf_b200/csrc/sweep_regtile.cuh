@@ -1,64 +1,34 @@
-// poismf_b200 — instantiation of the register-tile row kernels (regtile.cuh) for one method.
+// poismf_b200 — instantiation of the register-tile row kernels (regtile.cuh) for one method: one kernel per
+// entry of REGTILE_SHAPES (row_plan.h) and chunk count.
 //   PMF_RT_METHOD : M_PG or M_CG
 #pragma once
-#include <map>
-#include <mutex>
-#include <tuple>
+#include <utility>
 #include "regtile.cuh"
 #include "launch.h"
 
 namespace pmf {
 
-static std::mutex g_rt_mutex;
-static std::map<std::tuple<int, const void*>, int> g_rt_occ;   // (device, kernel) -> resident CTAs per SM
-
-template <int NC, int TPL, int NW, int METHOD>
-static cudaError_t rt_launch_one(const LaunchCfg& cfg, const SideParams<float>& P)
+template <int NC, int METHOD, size_t... I>
+static cudaError_t rt_launch_nc(const BinShape& b, const LaunchArgs& a, const SideParams<float>& P,
+                                std::index_sequence<I...>)
 {
-    auto kern = rows_regtile_kernel<NC, TPL, NW, METHOD>;
-    int occ = 1;
-    {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        std::lock_guard<std::mutex> lk(g_rt_mutex);
-        auto key = std::make_tuple(dev, (const void*)kern);
-        auto it = g_rt_occ.find(key);
-        if (it != g_rt_occ.end()) occ = it->second;
-        else {
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 32 * NW, 0) != cudaSuccess || occ < 1) occ = 1;
-            g_rt_occ[key] = occ;
-        }
-    }
-    long long g = (long long)cfg.num_sms * occ;
-    if (g > cfg.needed) g = cfg.needed;
-    if (g < 1) g = 1;
-    kern<<<(unsigned)g, 32 * NW, 0, cfg.stream>>>(P);
-    return cudaGetLastError();
-}
-
-template <int NC, int METHOD>
-static cudaError_t rt_launch_nc(const LaunchCfg& cfg, const SideParams<float>& P)
-{
-#define PMF_RT_CASE(NW_, TPL_) \
-    if (cfg.rt_nw == NW_ && cfg.rt_tpl == TPL_) return rt_launch_one<NC, TPL_, NW_, METHOD>(cfg, P);
-    PMF_RT_CASE(1, 2) PMF_RT_CASE(1, 3) PMF_RT_CASE(1, 4)
-    PMF_RT_CASE(2, 3) PMF_RT_CASE(2, 4)
-    PMF_RT_CASE(4, 3) PMF_RT_CASE(4, 4)
-    PMF_RT_CASE(8, 3) PMF_RT_CASE(8, 4)
-    PMF_RT_CASE(16, 3) PMF_RT_CASE(16, 4)
-#undef PMF_RT_CASE
-    return cudaErrorInvalidConfiguration;
+    cudaError_t e = cudaErrorInvalidConfiguration;
+    ((b.rt_nw == REGTILE_SHAPES[I].nw && b.rt_tpl == REGTILE_SHAPES[I].tpl &&
+      (e = launch_persistent(rows_regtile_kernel<NC, REGTILE_SHAPES[I].tpl, REGTILE_SHAPES[I].nw, METHOD>, b, a, P),
+       true)) || ...);
+    return e;
 }
 
 #if PMF_RT_METHOD == 3
-cudaError_t launch_regtile_pg(const LaunchCfg& cfg, const SideParams<float>& P)
+cudaError_t launch_regtile_pg(const BinShape& b, const LaunchArgs& a, const SideParams<float>& P)
 #else
-cudaError_t launch_regtile_cg(const LaunchCfg& cfg, const SideParams<float>& P)
+cudaError_t launch_regtile_cg(const BinShape& b, const LaunchArgs& a, const SideParams<float>& P)
 #endif
 {
     constexpr int METHOD = PMF_RT_METHOD;
-    if (cfg.rt_nc == 2) return rt_launch_nc<2, METHOD>(cfg, P);
-    if (cfg.rt_nc == 4) return rt_launch_nc<4, METHOD>(cfg, P);
+    constexpr auto shapes = std::make_index_sequence<sizeof(REGTILE_SHAPES) / sizeof(REGTILE_SHAPES[0])>();
+    if (b.rt_nc == 2) return rt_launch_nc<2, METHOD>(b, a, P, shapes);
+    if (b.rt_nc == 4) return rt_launch_nc<4, METHOD>(b, a, P, shapes);
     return cudaErrorInvalidConfiguration;
 }
 

@@ -1,11 +1,11 @@
-"""Register-tile kernels vs the shared-memory teams on one config: device time of the sweep, per-bin
+"""Register-tile kernels with and without the lock-step path on one config: device time of the sweep, per-bin
 times (serialised), log-likelihood after 1 and 3 sweeps, max factor difference.
     python scripts/dev_regtile.py [config] [method]"""
 import os, sys
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from bench import CONFIGS, make_problem, team_name
-from poismf_b200 import make_params
+from poismf_b200 import FLAG_NO_LOCKSTEP, make_params
 from poismf_b200.device import DeviceFit
 from oracle.oracle import Restatement
 
@@ -17,16 +17,11 @@ csr, csc, A0, B0 = make_problem(cfg)
 nnz = csr[0].shape[0]
 orc = Restatement(np.float32)
 res = {}
-modes = os.environ.get("MODES", "regtile,nodense,smem").split(",")
+modes = os.environ.get("MODES", "regtile,nodense").split(",")
 for mode in modes:
-    os.environ.pop("POISMF_B200_NO_REGTILE", None); os.environ.pop("POISMF_B200_NO_DENSE", None)
-    if mode == "smem":
-        os.environ["POISMF_B200_NO_REGTILE"] = "1"
-    elif mode == "nodense":
-        os.environ["POISMF_B200_NO_DENSE"] = "1"
     fit = DeviceFit(cfg["dimA"], cfg["dimB"], cfg["k"], np.float32)
     st = torch.cuda.Stream(); fit.set_stream(st.cuda_stream); fit.set_csr_csc(csr, csc)
-    p = make_params(cfg["method"], numiter=1, **cfg["hp"])
+    p = make_params(cfg["method"], numiter=1, flags=FLAG_NO_LOCKSTEP if mode == "nodense" else 0, **cfg["hp"])
     ts = []
     for rep in range(5):
         fit.set_factors(A0, B0); torch.cuda.synchronize()

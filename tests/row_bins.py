@@ -1,6 +1,6 @@
 """Shared pieces of the per-bin half-sweep tests (tests/test_gpu_row_bins.py, tests/test_host_row_bins.py).
 
-The device's planner (HandleT::plan, poismf_b200/csrc/api.cu) sends every row of the updated side to a kernel
+The device's planner (plan_rows, poismf_b200/csrc/row_plan.h) sends every row of the updated side to a kernel
 chosen by its non-zero count.  These helpers build count matrices whose rows have exactly the requested
 lengths, run the plain-C restatement's one-sided half-sweep (oracle_half_sweep) on the same inputs, and gate
 a result per bin against the float64 truth.

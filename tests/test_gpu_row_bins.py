@@ -1,6 +1,6 @@
 """Every row-kernel bin of the half-sweep against a float64 reference, bin by bin.
 
-The planner (HandleT::plan, poismf_b200/csrc/api.cu) sends each row of the updated side to a kernel chosen by
+The planner (plan_rows, poismf_b200/csrc/row_plan.h) sends each row of the updated side to a kernel chosen by
 its non-zero count: register-tile bins (float32 fast pg / cached cg with limit_step, k <= 64), (sub-)warp and
 CTA teams, clusters of 2..16 CTAs, the streaming cluster bin and the lock-step path for the heaviest rows.
 Whole-fit gates (log-likelihood, objective statistics over a matrix) do not see a kernel that is wrong on the
@@ -31,7 +31,7 @@ from test_gpu_headline import _dump
 pytestmark = pytest.mark.gpu
 
 LMAX = 40000
-ACAP = 4096          # per-CTA on-chip non-zeros of the streaming bin (plan(): b.acap); longer rows use global scratch
+ACAP = 4096          # per-CTA on-chip non-zeros of the streaming bin (bin_ladder(): b.acap); longer rows use global scratch
 DENSE_MIN = 600      # lock-step cases: rows of >= 600 non-zeros take the lock-step path
 
 
