@@ -30,6 +30,7 @@ UNITS = {
     "api.cu": [],
     "sweep_fast_pgcg.cu": [],
     "sweep_fast_tn.cu": [],
+    "sweep_lockstep.cu": [],
     "sweep_regtile_cg.cu": [],
     "sweep_regtile_pg.cu": [],
     "sweep_strict_pgcg.cu": ["--fmad=false"],

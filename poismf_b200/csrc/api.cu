@@ -31,8 +31,8 @@
 #include "staged_copy.h"
 #include <chrono>
 #include "kernels.cuh"
-#include "dense_rows.cuh"
 #include "launch.h"
+#include "lockstep.h"
 #include "topn_tc.cuh"
 #include "topn_include.cuh"
 
@@ -149,35 +149,11 @@ static int launch_column_sums(const real* M, size_t nrow, int k, int ldf, const 
 // ---------------------------------------------------------------------------
 struct Bin : PlannedBin {
     int* d_rows = nullptr;         // device copy of `rows`
-    std::vector<cudaEvent_t> ev;   // profiling: start/stop pairs of this bin's launches
-};
-
-// the heaviest rows of a side, solved in lock-step by the whole GPU (dense_rows.cuh)
-struct DensePlan {
-    int H = 0, T = 0, nnzH = 0, nchunks = 0, G = 0;
-    unsigned long long nnz = 0;
-    std::vector<int> rows;                 // local row ids, heaviest first
-    void* blocks[20] = {};                 // every device allocation below, for release
-    int nblocks = 0;
-    int *hrow = nullptr, *hcol0 = nullptr, *seg_ptr = nullptr, *chunk_h = nullptr, *chunk_ptr = nullptr;
-    long long* hbeg = nullptr;
-    uint2* ent = nullptr;
-    float* sx = nullptr;
-    float *p = nullptr, *q = nullptr, *dvec = nullptr, *gprev = nullptr, *dprev = nullptr, *gpart = nullptr, *lsp = nullptr;
-    DenseScal* sc = nullptr;
-    int* tile_counters = nullptr;          // one per dots launch of a half-sweep
-    std::vector<cudaEvent_t> ev;
-    void release()
-    {
-        for (auto e : ev) cudaEventDestroy(e);
-        ev.clear();
-        for (int i = 0; i < nblocks; i++) dfree(blocks[i]);
-        nblocks = 0; H = 0; nnzH = 0; rows.clear(); nnz = 0;
-    }
+    Timings timings;
 };
 
 template <class real> struct Side {
-    DensePlan dense;
+    LockstepPlan lockstep;         // the heaviest rows (lockstep.h)
     real* xv = nullptr;
     long long* ptr = nullptr;
     int* ind = nullptr;
@@ -194,8 +170,8 @@ template <class real> struct Side {
     // callers synchronise the streams that used these buffers first (devpool.h)
     void free_plan()
     {
-        for (auto& b : bins) for (auto e : b.ev) cudaEventDestroy(e);
-        dense.release();
+        for (auto& b : bins) b.timings.clear();
+        lockstep.release();
         if (d_all_rows) dfree(d_all_rows);
         if (gscratch) dfree(gscratch);
         d_all_rows = nullptr; gscratch = nullptr; d_empty = nullptr;
@@ -475,146 +451,6 @@ template <class real> struct HandleT : pmf_b200_handle {
     }
     void* factor_ptr(int which) override { return which == 0 ? (void*)A : (void*)B; }
 
-    // ---- lock-step path for the heaviest rows (dense_rows.cuh) ------------------------------------
-    int build_dense(Side<real>& S, const std::vector<int>& hrows, size_t other, cudaStream_t st)
-    {
-        DensePlan& D = S.dense;
-        D.release();
-        const int H = (int)hrows.size();
-        const int U = DN_TILE_ROWS;
-        const long long T = ((long long)other + U - 1) / U;
-        long long nnzH = 0;
-        for (int r : hrows) nnzH += S.h_ptr[r + 1] - S.h_ptr[r];
-        D.H = H; D.T = (int)T; D.nnzH = (int)nnzH; D.nnz = (unsigned long long)nnzH; D.rows = hrows;
-        D.G = (int)std::min<long long>(num_sms, T);         // persistent CTAs of the gaxpy pass
-        // host tables: [hrow H][hcol0 H+1][chunk_ptr H+1][chunk_h nchunks]
-        std::vector<long long> hbeg(H);
-        std::vector<int> hcol0(H + 1, 0), chunk_ptr(H + 1, 0);
-        for (int h = 0; h < H; h++) {
-            const long long n = S.h_ptr[hrows[h] + 1] - S.h_ptr[hrows[h]];
-            hbeg[h] = S.h_ptr[hrows[h]];
-            hcol0[h + 1] = hcol0[h] + (int)n;
-            chunk_ptr[h + 1] = chunk_ptr[h] + (int)((n + DN_LS_CHUNK - 1) / DN_LS_CHUNK);
-        }
-        D.nchunks = chunk_ptr[H];
-        std::vector<int> i32(hrows);
-        i32.insert(i32.end(), hcol0.begin(), hcol0.end());
-        i32.insert(i32.end(), chunk_ptr.begin(), chunk_ptr.end());
-        for (int h = 0; h < H; h++)
-            for (int c = chunk_ptr[h]; c < chunk_ptr[h + 1]; c++) i32.push_back(h);
-        auto grab = [&](auto** ptr, size_t bytes) -> int {
-            CK(dmalloc(ptr, std::max<size_t>(bytes, 16)));
-            D.blocks[D.nblocks++] = (void*)*ptr;
-            return 0;
-        };
-        int* tables = nullptr;
-        if (grab(&tables, i32.size() * sizeof(int))) return 1;
-        D.hrow = tables; D.hcol0 = tables + H; D.chunk_ptr = D.hcol0 + H + 1; D.chunk_h = D.chunk_ptr + H + 1;
-        if (grab(&D.hbeg, (size_t)H * sizeof(long long))) return 1;
-        if (grab(&D.ent, (size_t)nnzH * sizeof(uint2))) return 1;
-        if (grab(&D.sx, (size_t)nnzH * sizeof(float))) return 1;
-        if (grab(&D.seg_ptr, ((size_t)T * H + 1) * sizeof(int))) return 1;
-        if (grab(&D.p, (size_t)nnzH * sizeof(float))) return 1;
-        if (grab(&D.q, (size_t)nnzH * sizeof(float))) return 1;
-        if (grab(&D.dvec, (size_t)H * ldf * sizeof(float))) return 1;
-        if (grab(&D.gprev, (size_t)H * 64 * sizeof(float))) return 1;
-        if (grab(&D.dprev, (size_t)H * 64 * sizeof(float))) return 1;
-        if (grab(&D.gpart, (size_t)D.G * H * ldf * sizeof(float))) return 1;
-        if (grab(&D.lsp, (size_t)D.nchunks * DN_TRIALS * sizeof(float))) return 1;
-        if (grab(&D.sc, (size_t)H * sizeof(DenseScal))) return 1;
-        if (grab(&D.tile_counters, 64 * sizeof(int))) return 1;
-        CK(cudaMemcpyAsync(tables, i32.data(), i32.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(D.hbeg, hbeg.data(), (size_t)H * sizeof(long long), cudaMemcpyHostToDevice, st));
-        CK(cudaMemsetAsync(D.q, 0, (size_t)nnzH * sizeof(float), st));
-        // sort the heavy rows' non-zeros by (tile of the fixed matrix, heavy row); stable: ascending position inside
-        int *slot = nullptr, *pos = nullptr, *spos = nullptr;
-        unsigned *k1 = nullptr, *k2 = nullptr;
-        void* tmp = nullptr;
-        CK(dmalloc(&slot, (size_t)nnzH * sizeof(int))); deferred.push_back(slot);
-        CK(dmalloc(&pos, (size_t)nnzH * sizeof(int))); deferred.push_back(pos);
-        CK(dmalloc(&spos, (size_t)nnzH * sizeof(int))); deferred.push_back(spos);
-        CK(dmalloc(&k1, (size_t)nnzH * sizeof(unsigned))); deferred.push_back(k1);
-        CK(dmalloc(&k2, (size_t)nnzH * sizeof(unsigned))); deferred.push_back(k2);
-        int bits = 1;
-        while (bits < 32 && (1LL << bits) < T * H) bits++;
-        size_t tb = 0;
-        CK(cub::DeviceRadixSort::SortPairs(nullptr, tb, k1, k2, pos, spos, (int)nnzH, 0, bits, st));
-        CK(dmalloc(&tmp, std::max<size_t>(tb, 16))); deferred.push_back(tmp);
-        const int grid = num_sms * 8;
-        dense_fill_slot_kernel<<<dim3(8, H), 256, 0, st>>>(D.hcol0, H, slot);
-        LAUNCHED();
-        dense_keys_kernel<<<grid, 256, 0, st>>>(S.ind, slot, D.hbeg, D.hcol0, (int)nnzH, H, U, k1, pos);
-        LAUNCHED();
-        CK(cub::DeviceRadixSort::SortPairs(tmp, tb, k1, k2, pos, spos, (int)nnzH, 0, bits, st));
-        LAUNCHED();
-        dense_unpack_kernel<<<grid, 256, 0, st>>>(k2, spos, S.ind, (const float*)S.xv, D.hbeg, D.hcol0, (int)nnzH, H, U, ldf, D.ent, D.sx);
-        LAUNCHED();
-        dense_segments_kernel<<<grid, 256, 0, st>>>(k2, (int)nnzH, (int)(T * H), D.seg_ptr);
-        LAUNCHED();
-        CK(cudaGetLastError());
-        return 0;
-    }
-
-    // one half-sweep of the heavy rows: ~5 launches per cg iteration, all on `st`
-    int run_dense(Side<real>& S, real* M, const real* F, const HalfSweepConsts<real>& hc, int which_factor, cudaStream_t st)
-    {
-        if constexpr (!std::is_same<real, float>::value) {
-            return fail("lock-step path is float32 only");
-        } else {
-            DensePlan& D = S.dense;
-            DenseParams P;
-            P.H = D.H; P.T = D.T; P.U = DN_TILE_ROWS; P.ldf = ldf; P.k = k; P.L = ldf / 4;
-            P.nnzH = D.nnzH; P.nchunks = D.nchunks; P.G = D.G;
-            P.R = (int)(which_factor == 0 ? dimB : dimA);
-            P.F = F; P.M = M + S.row_begin * (size_t)ldf; P.xv = S.xv; P.csum = csum;
-            P.hrow = D.hrow; P.hbeg = D.hbeg; P.hcol0 = D.hcol0; P.ent = D.ent; P.sx = D.sx;
-            P.seg_ptr = D.seg_ptr; P.chunk_h = D.chunk_h; P.chunk_ptr = D.chunk_ptr;
-            P.p = D.p; P.q = D.q; P.dvec = D.dvec; P.gprev = D.gprev; P.dprev = D.dprev; P.gpart = D.gpart; P.lsp = D.lsp;
-            P.sc = D.sc; P.hc = hc;
-            P.npeers = npeers[which_factor];
-            for (int q = 0; q < 7; q++)
-                P.peerM[q] = q < P.npeers ? peer[which_factor][q] + S.row_begin * (size_t)ldf : nullptr;
-            const size_t tile_bytes = (size_t)DN_TILE_ROWS * ldf * sizeof(float);
-            const size_t smem_dots = tile_bytes + (size_t)D.H * sizeof(int);
-            const size_t smem_g = 2 * tile_bytes + (size_t)(D.H + DN_GROUPS) * ldf * sizeof(float);
-            CK(ensure_smem((const void*)dense_walk_kernel<0>, smem_dots));
-            CK(ensure_smem((const void*)dense_walk_kernel<1>, smem_dots));
-            CK(ensure_smem((const void*)dense_walk_kernel<2>, smem_g));
-            const int hg = (D.H + 3) / 4;
-            const int gd = (int)std::min<long long>(4 * num_sms, D.T);   // dots passes: four persistent CTAs per SM
-            CK(cudaMemsetAsync(D.tile_counters, 0, 64 * sizeof(int), st));
-            int n_dots = 0;
-            dense_reset_kernel<<<(D.H + 127) / 128, 128, 0, st>>>(P);
-            P.tile_counter = D.tile_counters + (n_dots++ & 63);
-            dense_walk_kernel<0><<<gd, DnWalk<0>::threads, smem_dots, st>>>(P);
-            dense_ls_kernel<<<D.nchunks, 256, 0, st>>>(P, 0);
-            dense_init_kernel<<<hg, 128, 0, st>>>(P);
-            g_launches.fetch_add(4, std::memory_order_relaxed);
-            const long long maxiter = hc.maxupd <= 0 ? (1LL << 40) : hc.maxupd;
-            for (long long it = 0; it < maxiter; it++) {
-                dense_walk_kernel<2><<<D.G, DnWalk<2>::threads, smem_g, st>>>(P);
-                dense_k_kernel<<<D.H, 256, 0, st>>>(P);
-                if ((n_dots & 63) == 0) CK(cudaMemsetAsync(D.tile_counters, 0, 64 * sizeof(int), st));   // all 64 used up
-                P.tile_counter = D.tile_counters + (n_dots++ & 63);
-                dense_walk_kernel<1><<<gd, DnWalk<1>::threads, smem_dots, st>>>(P);
-                dense_ls_kernel<<<D.nchunks, 256, 0, st>>>(P, 1);
-                dense_choose_kernel<<<hg, 128, 0, st>>>(P);
-                g_launches.fetch_add(5, std::memory_order_relaxed);
-                if ((it & 7) == 7 && it + 1 < maxiter) {
-                    // long iteration budgets (factors_multiple's cg): stop enqueueing once every row is done
-                    std::vector<DenseScal> hs(D.H);
-                    CK(cudaMemcpyAsync(hs.data(), D.sc, (size_t)D.H * sizeof(DenseScal), cudaMemcpyDeviceToHost, st));
-                    CK(cudaStreamSynchronize(st));
-                    bool any = false;
-                    for (auto& q : hs) any = any || q.active;
-                    if (!any) break;
-                }
-            }
-            CK(cudaGetLastError());
-            return 0;
-        }
-    }
-
     // the planner's inputs for the parameters of a half-sweep (row_plan.h)
     PlanMode plan_mode(const pmf_b200_params& p) const
     {
@@ -641,9 +477,23 @@ template <class real> struct HandleT : pmf_b200_handle {
             if (sync_all()) return 1;
             S.free_plan();
         }
+        if (build_plan(S, m, st)) {     // release what a part-way plan holds
+            sync_all();
+            S.free_plan();
+            return 1;
+        }
+        S.planned_method = key;
+        return 0;
+    }
+    int build_plan(Side<real>& S, const PlanMode& m, cudaStream_t st)
+    {
         const size_t other = (&S == &sides[0]) ? dimB : dimA;
         RowPlan rp = plan_rows(m, S.h_ptr.data(), S.n_rows, other);
-        if (!rp.lockstep.empty() && build_dense(S, rp.lockstep, other, st)) return 1;
+        if (!rp.lockstep.empty()) {
+            const cudaError_t e = S.lockstep.build(rp.lockstep, S.h_ptr.data(), S.ind, (const float*)S.xv, other, k, ldf,
+                                                   num_sms, deferred, st, g_launches);
+            if (e != cudaSuccess) return fail("lock-step plan: %s", cudaGetErrorString(e));
+        }
         size_t total = rp.empty.size();
         for (auto& b : rp.bins) total += b.rows.size();
         CK(dmalloc(&S.d_all_rows, std::max<size_t>(total, 1) * sizeof(int)));
@@ -672,7 +522,6 @@ template <class real> struct HandleT : pmf_b200_handle {
             CK(dmalloc(&S.gscratch, (size_t)S.gs_ctas * 3 * S.gs_stride * sizeof(real)));
         }
         S.bins.swap(bins);      // the row lists' host copies stay alive in S.bins until the next plan
-        S.planned_method = key;
         return 0;
     }
 
@@ -757,16 +606,17 @@ template <class real> struct HandleT : pmf_b200_handle {
         if (overlap) CK(cudaEventRecord(ev_fork, stream));
         int n_launched = 0;
         bool used[NAUX] = {};
-        if (S.dense.H > 0) {                                      // the heaviest rows: lock-step path, own stream
+        if (S.lockstep.rows() > 0) {                              // the heaviest rows: lock-step path, own stream
             cudaStream_t ls = stream;
             if (overlap) { ls = aux[0]; CK(cudaStreamWaitEvent(ls, ev_fork, 0)); used[0] = true; n_launched = 1; }
-            cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-            if (profiling) { CK(cudaEventCreate(&ev0)); CK(cudaEventCreate(&ev1)); CK(cudaEventRecord(ev0, stream)); }
+            if (profiling) CK(S.lockstep.timings.start(stream));
+            cudaError_t e = cudaErrorInvalidValue;   // float32 only (row_plan.h)
             nvtxRangePushA("lock-step rows");
-            const int rc_dense = run_dense(S, M, F, hc, updA ? 0 : 1, ls);
+            if constexpr (std::is_same<real, float>::value)
+                e = S.lockstep.run(M, peer[updA ? 0 : 1], npeers[updA ? 0 : 1], S.row_begin, F, csum, hc, ls, g_launches);
             nvtxRangePop();
-            if (rc_dense) return 1;
-            if (profiling) { CK(cudaEventRecord(ev1, stream)); S.dense.ev.push_back(ev0); S.dense.ev.push_back(ev1); }
+            if (e != cudaSuccess) return fail("lock-step rows of side %d: %s", side, cudaGetErrorString(e));
+            if (profiling) CK(S.lockstep.timings.stop(stream));
         }
         for (int bi = (int)S.bins.size() - 1; bi >= 0; bi--) {    // heaviest rows first
             const Bin& bin = S.bins[bi];
@@ -775,7 +625,7 @@ template <class real> struct HandleT : pmf_b200_handle {
             cudaStream_t ls = stream;
             if (overlap) {
                 // (the lock-step chain keeps aux[0] to itself: a bin queued behind it would start when it ends)
-                const int si = S.dense.H > 0 ? 1 + (n_launched - 1) % (NAUX - 1) : n_launched % NAUX;
+                const int si = S.lockstep.rows() > 0 ? 1 + (n_launched - 1) % (NAUX - 1) : n_launched % NAUX;
                 ls = aux[si];
                 if (!used[si]) { CK(cudaStreamWaitEvent(ls, ev_fork, 0)); used[si] = true; }
             }
@@ -801,11 +651,7 @@ template <class real> struct HandleT : pmf_b200_handle {
             la.max_grid = b.cap == 0 ? S.gs_ctas / b.cluster : (1 << 30);
             la.num_sms = num_sms;
             la.cached = !strict && !(p.flags & PMF_FLAG_NO_CACHED);
-            cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-            if (profiling) {
-                CK(cudaEventCreate(&ev0)); CK(cudaEventCreate(&ev1));
-                CK(cudaEventRecord(ev0, stream));
-            }
+            if (profiling) CK(S.bins[bi].timings.start(stream));
             static const char* const kind_name[] = {"regtile", "warp", "cta", "cluster", "streaming"};
             {
                 char nm[96];
@@ -836,10 +682,7 @@ template <class real> struct HandleT : pmf_b200_handle {
                 return fail("row kernel launch failed at side %d bin %d (%s, lanes %d cluster %d cap %d threads %d smem %zu): %s",
                             side, bi, kind_name[(int)b.kind], b.lanes, b.cluster, b.cap, b.threads, b.smem,
                             cudaGetErrorString(e));
-            if (profiling) {
-                CK(cudaEventRecord(ev1, stream));
-                S.bins[bi].ev.push_back(ev0); S.bins[bi].ev.push_back(ev1);
-            }
+            if (profiling) CK(S.bins[bi].timings.stop(stream));
         }
         if (overlap)
             for (int si = 0; si < NAUX; si++)
@@ -926,43 +769,30 @@ template <class real> struct HandleT : pmf_b200_handle {
 
     void clear_profile() override
     {
-        for (int sd = 0; sd < 2; sd++) {
-            for (auto& b : sides[sd].bins) {
-                for (auto e : b.ev) cudaEventDestroy(e);
-                b.ev.clear();
-            }
-            for (auto e : sides[sd].dense.ev) cudaEventDestroy(e);
-            sides[sd].dense.ev.clear();
+        for (Side<real>& S : sides) {
+            S.lockstep.timings.clear();
+            for (Bin& b : S.bins) b.timings.clear();
         }
     }
+    // the lock-step path of side 0, then of side 1, then the bins of side 0 and of side 1
     int get_profile(pmf_b200_bin_profile* out, int max_entries) override
     {
         cudaSetDevice(device);
         cudaStreamSynchronize(stream);
         int n = 0;
+        auto put = [&](int sd, int code, int cap, int nrows, unsigned long long nnz, const Timings& t) {
+            if (n >= max_entries) return;
+            pmf_b200_bin_profile& o = out[n++];
+            o.side = sd; o.block_team = code; o.cap = cap; o.nrows = nrows; o.nnz = nnz;
+            o.launches = t.launches(); o.ms = t.ms();
+        };
         for (int sd = 0; sd < 2; sd++) {
-            DensePlan& D = sides[sd].dense;
-            if (D.H > 0 && n < max_entries) {
-                pmf_b200_bin_profile& o = out[n++];
-                o.side = sd; o.block_team = 200; o.cap = 0; o.nrows = D.H; o.nnz = D.nnz; o.launches = D.ev.size() / 2; o.ms = 0;
-                for (size_t i = 0; i + 1 < D.ev.size(); i += 2) {
-                    float ms = 0;
-                    if (cudaEventElapsedTime(&ms, D.ev[i], D.ev[i + 1]) == cudaSuccess) o.ms += ms;
-                }
-            }
+            const LockstepPlan& L = sides[sd].lockstep;
+            if (L.rows() > 0) put(sd, LOCKSTEP_PROFILE_CODE, 0, L.rows(), L.nnz(), L.timings);
         }
         for (int sd = 0; sd < 2; sd++)
-            for (auto& b : sides[sd].bins) {
-                if (b.rows.empty() || n >= max_entries) continue;
-                pmf_b200_bin_profile& o = out[n++];
-                o.side = sd; o.block_team = profile_code(b.shape);
-                o.cap = b.shape.cap; o.nrows = (int)b.rows.size();
-                o.nnz = b.nnz; o.launches = b.ev.size() / 2; o.ms = 0;
-                for (size_t i = 0; i + 1 < b.ev.size(); i += 2) {
-                    float ms = 0;
-                    if (cudaEventElapsedTime(&ms, b.ev[i], b.ev[i + 1]) == cudaSuccess) o.ms += ms;
-                }
-            }
+            for (const Bin& b : sides[sd].bins)
+                if (!b.rows.empty()) put(sd, profile_code(b.shape), b.shape.cap, (int)b.rows.size(), b.nnz, b.timings);
         return n;
     }
 

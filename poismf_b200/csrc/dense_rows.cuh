@@ -34,8 +34,6 @@
 
 namespace pmf {
 
-constexpr int DN_TRIALS = 20;       // line-search trials evaluated per pass: ALL of them (max_ls of nonnegcg.c)
-constexpr int DN_LS_CHUNK = 2048;   // non-zeros per CTA of the line-search kernel
 constexpr int DN_MAX_LS = 20, DN_MAX_NFEVAL = 150;
 
 // ---- TMA bulk copy (cp.async.bulk, global -> shared, completion on an mbarrier) ---------------------

@@ -6,9 +6,40 @@
 #include <mutex>
 #include <tuple>
 #include <utility>
+#include <vector>
 #include "row_plan.h"
 
 namespace pmf {
+
+// profiling: a start/stop event pair around each launch of a bin (or of the lock-step path)
+struct Timings {
+    std::vector<cudaEvent_t> ev;
+    cudaError_t start(cudaStream_t st)
+    {
+        cudaEvent_t a = nullptr, b = nullptr;
+        cudaError_t e = cudaEventCreate(&a);
+        if (e == cudaSuccess && (e = cudaEventCreate(&b)) != cudaSuccess) cudaEventDestroy(a);
+        if (e != cudaSuccess) return e;
+        ev.push_back(a); ev.push_back(b);
+        return cudaEventRecord(a, st);
+    }
+    cudaError_t stop(cudaStream_t st) { return cudaEventRecord(ev.back(), st); }
+    int launches() const { return (int)(ev.size() / 2); }
+    double ms() const
+    {
+        double sum = 0;
+        for (size_t i = 0; i + 1 < ev.size(); i += 2) {
+            float ms = 0;
+            if (cudaEventElapsedTime(&ms, ev[i], ev[i + 1]) == cudaSuccess) sum += ms;
+        }
+        return sum;
+    }
+    void clear()
+    {
+        for (auto e : ev) cudaEventDestroy(e);
+        ev.clear();
+    }
+};
 
 template <class real> struct SideParams;
 

@@ -2,10 +2,11 @@
 //
 // Host-only arithmetic, no CUDA call: HandleT::plan (api.cu) uploads what plan_rows decides, half_sweep
 // launches one kernel per bin, and the launchers (sweep_inst.cuh, sweep_regtile.cuh) instantiate the kernel
-// a BinShape names.
+// a BinShape names.  The lock-step rows go to LockstepPlan (lockstep.h), which uploads lockstep_tables.
 #pragma once
 #include <algorithm>
 #include <cstddef>
+#include <cstdint>
 #include <utility>
 #include <vector>
 
@@ -47,7 +48,8 @@ struct PlanMode {
 };
 
 // pmf_b200_bin_profile::block_team: -lanes for a (sub-)warp team, CTAs per row for CTA and cluster teams,
-// 100 + warps per row for register tiles (200 is the lock-step path)
+// 100 + warps per row for register tiles, LOCKSTEP_PROFILE_CODE for the lock-step path
+constexpr int LOCKSTEP_PROFILE_CODE = 200;
 inline int profile_code(const BinShape& b)
 {
     switch (b.kind) {
@@ -212,9 +214,10 @@ inline RowPlan plan_rows(const PlanMode& m, const long long* ptr, size_t n_rows,
         // per-row cluster teams are cheaper (small shards of a multi-GPU fit, the user side of config #2)
         long long nnzH = 0;
         for (auto& c : cand) nnzH -= c.first;
-        // the lock-step tables index non-zeros and (tile, heavy row) segments with 32-bit integers
+        // the lock-step tables index non-zeros and the T x H + 1 bounds of the (tile, heavy row) segments with
+        // 32-bit integers
         const long long T = ((long long)other_dim + DN_TILE_ROWS - 1) / DN_TILE_ROWS;
-        const bool fits = nnzH < (1LL << 31) && T * (long long)cand.size() < (1LL << 32) && ptr[n_rows] < (1LL << 31);
+        const bool fits = nnzH < (1LL << 31) && T * (long long)cand.size() + 1 <= INT32_MAX && ptr[n_rows] < (1LL << 31);
         if (nnzH >= m.dense_min_total && fits)
             for (auto& c : cand) plan.lockstep.push_back(c.second);
     }
@@ -248,6 +251,56 @@ inline RowPlan plan_rows(const PlanMode& m, const long long* ptr, size_t n_rows,
         }
     }
     return plan;
+}
+
+// The host side of a lock-step plan (sweep_lockstep.cu): the tables every lock-step kernel indexes and the element
+// count of every device array, for the lock-step rows `rows` of a side with row pointers ptr, a fixed matrix of
+// other_dim rows of ldf reals and num_sms SMs.  plan_rows keeps T x H + 1, the non-zeros and the side's non-zeros
+// below 2^31; ldf <= 64 and H <= 65535 are the path's own bounds (lockstep.h).
+struct LockstepTables {
+    int H = 0;          // heavy rows
+    int T = 0;          // tiles of DN_TILE_ROWS rows of the fixed matrix
+    int G = 0;          // persistent CTAs of the gaxpy pass
+    int nnzH = 0;       // non-zeros of the heavy rows
+    int nchunks = 0;    // line-search chunks of DN_LS_CHUNK non-zeros, none across two rows
+    std::vector<int> i32;          // one block: hrow [H] | hcol0 [H+1] | chunk_ptr [H+1] | chunk_h [nchunks]
+    std::vector<long long> hbeg;   // [H] first non-zero of each heavy row in the side's arrays
+    // device arrays: hbeg and the per-row scalars hold H entries; ent, sx, p, q and the sort's temporaries nnzH
+    size_t n_seg = 0;       // seg_ptr: T x H + 1
+    size_t n_dvec = 0;      // dvec: H x ldf
+    size_t n_hist = 0;      // gprev, dprev: H x 64
+    size_t n_gpart = 0;     // gpart: G x H x ldf
+    size_t n_lsp = 0;       // lsp: nchunks x DN_TRIALS
+};
+
+inline LockstepTables lockstep_tables(const long long* ptr, const std::vector<int>& rows, size_t other_dim,
+                                      int num_sms, int ldf)
+{
+    LockstepTables t;
+    const int H = t.H = (int)rows.size();
+    const long long T = ((long long)other_dim + DN_TILE_ROWS - 1) / DN_TILE_ROWS;
+    t.T = (int)T;
+    t.G = (int)std::min<long long>(num_sms, T);
+    t.hbeg.resize(H);
+    std::vector<int> hcol0(H + 1, 0), chunk_ptr(H + 1, 0);
+    for (int h = 0; h < H; h++) {
+        const long long n = ptr[rows[h] + 1] - ptr[rows[h]];
+        t.hbeg[h] = ptr[rows[h]];
+        hcol0[h + 1] = hcol0[h] + (int)n;
+        chunk_ptr[h + 1] = chunk_ptr[h] + (int)((n + DN_LS_CHUNK - 1) / DN_LS_CHUNK);
+    }
+    t.nnzH = hcol0[H];
+    t.nchunks = chunk_ptr[H];
+    t.i32 = rows;
+    t.i32.insert(t.i32.end(), hcol0.begin(), hcol0.end());
+    t.i32.insert(t.i32.end(), chunk_ptr.begin(), chunk_ptr.end());
+    for (int h = 0; h < H; h++) t.i32.insert(t.i32.end(), (size_t)(chunk_ptr[h + 1] - chunk_ptr[h]), h);
+    t.n_seg = (size_t)T * H + 1;
+    t.n_dvec = (size_t)H * ldf;
+    t.n_hist = (size_t)H * 64;
+    t.n_gpart = (size_t)t.G * H * ldf;
+    t.n_lsp = (size_t)t.nchunks * DN_TRIALS;
+    return t;
 }
 
 }  // namespace pmf

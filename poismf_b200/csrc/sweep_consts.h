@@ -25,5 +25,8 @@ constexpr int TN_NUM_VECS = 24;                  // k-vectors of the tncg solver
 
 constexpr int DN_TILE_ROWS = 256;   // lock-step path: rows of the fixed matrix per tile
 constexpr int DN_GROUPS = 1024 / 16;  // lock-step gaxpy pass: groups of 16 lanes of its 1024-thread CTA
+constexpr int DN_LS_CHUNK = 2048;   // lock-step line search: non-zeros per CTA
+constexpr int DN_TRIALS = 20;       // lock-step line search: trials evaluated per pass, ALL of them (max_ls of nonnegcg.c)
+constexpr int DN_TILE_COUNTERS = 64;  // lock-step dots passes: ring of tile counters, one per pass of a half-sweep
 
 }  // namespace pmf

@@ -1,5 +1,5 @@
 """CPU checks of the half-sweep's row planner (poismf_b200/csrc/row_plan.h): the bin ladder of every mode, where each
-row length goes, the order of the row lists, the lock-step rows and the profile codes.  A small driver over the
+row length goes, the order of the row lists, the lock-step rows and their host tables, and the profile codes.  A small driver over the
 header is compiled with the host C++ compiler; no CUDA call is made."""
 import os
 import shutil
@@ -49,6 +49,24 @@ int main(int argc, char** argv)
                                    b.cluster, b.smem);
                         printf("\n");
                     }
+        return 0;
+    }
+    if (!strcmp(argv[1], "tables")) {
+        // tables <other_dim> <num_sms> <ldf>; stdin: n, n row lengths, then the lock-step rows
+        std::vector<long long> ptr(1, 0);
+        long long n = 0, v;
+        if (scanf("%lld", &n) != 1) return 1;
+        for (long long i = 0; i < n && scanf("%lld", &v) == 1; i++) ptr.push_back(ptr.back() + v);
+        std::vector<int> rows;
+        while (scanf("%lld", &v) == 1) rows.push_back((int)v);
+        const LockstepTables t = lockstep_tables(ptr.data(), rows, (size_t)strtoull(argv[2], nullptr, 10), atoi(argv[3]),
+                                                 atoi(argv[4]));
+        printf("%d %d %d %d %d %zu %zu %zu %zu %zu\n", t.H, t.T, t.G, t.nnzH, t.nchunks, t.n_seg, t.n_dvec, t.n_hist,
+               t.n_gpart, t.n_lsp);
+        for (int x : t.i32) printf(" %d", x);
+        printf("\n");
+        for (long long x : t.hbeg) printf(" %lld", x);
+        printf("\n");
         return 0;
     }
     // plan <real size> <k> <method> <strict> <regtile> <lockstep> <dense_min> <dense_min_total> <other_dim>,
@@ -214,14 +232,76 @@ def test_no_lockstep_rows(driver):
     assert _plan(driver, lengths, **dict(on, lockstep=False), dense_min_total=0)["lockstep"] == []
     assert _plan(driver, lengths, **dict(on, regtile=False), dense_min_total=0)["lockstep"] == []
     assert _plan(driver, lengths, **dict(on, method=PG), dense_min_total=0)["lockstep"] == []
-    # tiles of the fixed matrix x heavy rows >= 2^32 (328 heavy rows at k = 64)
-    tiles = -(-2**32 // 328)
-    assert _plan(driver, lengths, **on, dense_min_total=0, other=256 * (tiles - 1))["lockstep"]
-    assert _plan(driver, lengths, **on, dense_min_total=0, other=256 * tiles)["lockstep"] == []
+    # the T x H + 1 bounds of the (tile of the fixed matrix, heavy row) segments must fit an int32: T x H <= 2^31 - 2
+    # (328 heavy rows at k = 64)
+    tiles = (2**31 - 2) // 328
+    assert _plan(driver, lengths, **on, dense_min_total=0, other=256 * tiles)["lockstep"]
+    assert _plan(driver, lengths, **on, dense_min_total=0, other=256 * (tiles + 1))["lockstep"] == []
+    one = np.zeros(100, dtype=np.int64)
+    one[7] = 5000
+    assert _plan(driver, one, **on, dense_min_total=0, other=256 * (2**31 - 2))["lockstep"] == [7]
+    assert _plan(driver, one, **on, dense_min_total=0, other=256 * (2**31 - 2) + 1)["lockstep"] == []
     # the side's non-zeros >= 2^31 while the heavy rows' are not
     big = np.full(2400, 1_000_000)
     assert _plan(driver, big[:2000], **on, dense_min_total=0)["lockstep"]
     assert _plan(driver, big, **on, dense_min_total=0)["lockstep"] == []
+
+
+def _tables(driver, lengths, rows, other, sms, ldf):
+    out = subprocess.run([driver, "tables", str(other), str(sms), str(ldf)],
+                         input=" ".join(str(int(v)) for v in [len(lengths), *lengths, *rows]),
+                         capture_output=True, text=True, check=True).stdout.split("\n")
+    return [int(v) for v in out[0].split()], [int(v) for v in out[1].split()], [int(v) for v in out[2].split()]
+
+
+def _tables_ref(lengths, rows, other, sms, ldf):
+    """numpy restatement of lockstep_tables: sizes, the int32 block hrow | hcol0 | chunk_ptr | chunk_h, hbeg, and the
+    element counts of seg_ptr, dvec, gprev / dprev, gpart and lsp."""
+    lengths, rows = np.asarray(lengths, dtype=np.int64), np.asarray(rows, dtype=np.int64)
+    ptr = np.concatenate([[0], np.cumsum(lengths)])
+    n = lengths[rows]
+    H, T = len(rows), -(-other // 256)
+    G = min(sms, T)
+    hcol0 = np.concatenate([[0], np.cumsum(n)])
+    chunks = -(-n // 2048)
+    chunk_ptr = np.concatenate([[0], np.cumsum(chunks)])
+    nchunks = int(chunk_ptr[-1])
+    sizes = [H, T, G, int(hcol0[-1]), nchunks, T * H + 1, H * ldf, H * 64, G * H * ldf, nchunks * 20]
+    i32 = np.concatenate([rows, hcol0, chunk_ptr, np.repeat(np.arange(H), chunks)])
+    return sizes, i32.tolist(), ptr[rows].tolist()
+
+
+@pytest.mark.parametrize("case", ["one_row", "many_rows", "chunk_edges", "odd_tiles", "few_tiles"])
+def test_lockstep_tables(driver, case):
+    """lockstep_tables gives the numpy restatement's tables and device array sizes: one heavy row, many rows, row
+    lengths at multiples of the line-search chunk and one either side, fixed sides of no whole number of tiles, and
+    fewer tiles than SMs (the gaxpy pass then runs one CTA per tile)."""
+    rng = np.random.default_rng(len(case))
+    lengths = rng.integers(0, 3000, 5000)
+    other, sms, ldf = 160_000, 148, 52
+    if case == "one_row":
+        lengths[123] = 300_000
+        rows = [123]
+    elif case == "many_rows":
+        lengths[rng.choice(5000, 400, replace=False)] = rng.integers(4096, 60_000, 400)
+        rows = np.argsort(-lengths, kind="stable")[:400]
+    elif case == "chunk_edges":
+        edges = [m * 2048 + d for m in (1, 2, 3, 7) for d in (-1, 0, 1)] + [1, 2048 * 16]
+        rows = rng.choice(5000, len(edges), replace=False)
+        lengths[rows] = edges
+    elif case == "odd_tiles":
+        rows = np.argsort(-lengths, kind="stable")[:50]
+        other, ldf = 100_001, 64
+    else:
+        rows = np.argsort(-lengths, kind="stable")[:30]
+        other, ldf = 255 + 256 * 20, 16
+    got = _tables(driver, lengths, rows, other, sms, ldf)
+    want = _tables_ref(lengths, rows, other, sms, ldf)
+    assert got == want
+    if case == "few_tiles":
+        assert got[0][2] == got[0][1] == 21
+    if case == "chunk_edges":
+        assert got[0][4] == sum(-(-e // 2048) for e in edges)
 
 
 @pytest.mark.parametrize("rs,k,method,strict,regtile", [
