@@ -166,6 +166,15 @@ int pmf_b200_fit_coo(int dtype, int index_bytes, void* A, void* B, const void* r
 int pmf_b200_coo_to_csr_csc(int dtype, int index_bytes, const void* rows, const void* cols, const void* vals,
                             size_t n_entries, size_t dimA, size_t dimB, void* Xr, void* Xr_indptr,
                             void* Xr_indices, void* Xc, void* Xc_indptr, void* Xc_indices, size_t* nnz_out);
+/* The same conversion into a fit handle (PoisMF._process_data for a resident fit): the CSR and CSC of the triplets
+ * (the structure pmf_b200_coo_to_csr_csc gives: duplicates summed, ids ascending) replace the matrix the handle
+ * held and stay on the device; the row plans are rebuilt by the next sweep, the factors are untouched.  Ids lie in
+ * [0, dimA) / [0, dimB) of the handle.  Returns 0; 2 when n_entries is 0 or > 2^31-1, index_bytes is not 4 or 8,
+ * or the handle has imported peer mappings (part of a sharded fit): the handle is then unchanged; 2 when an id is
+ * outside [0, dim): the handle then holds NO matrix (factors untouched; set a matrix before sweeping, until then
+ * a sweep fails with 1); 1 on a CUDA failure (the matrix is then unspecified). */
+int pmf_b200_set_coo(pmf_b200_handle* h, const void* rows, const void* cols, const void* vals, size_t n_entries,
+                     int index_bytes);
 
 /* Replaces factors_single, src/pred.c:201-304 (prototype src/poismf.h:281-289): factors of ONE new row
  * (nnz counts X at item ids X_ind) by tncg, with B and Bsum (old l1 already added) fixed; l1_new - l1_old
@@ -179,6 +188,17 @@ int pmf_b200_factors_single(int dtype, int index_bytes, void* out, size_t k, con
 int pmf_b200_predict_multiple(int dtype, int index_bytes, void* out, const void* A, const void* B,
                               const void* ixA, const void* ixB, size_t n, int k,
                               size_t dimA, size_t dimB);
+/* The same scores against the factors RESIDENT in a fit handle: out[i] = <A[ixA[i]], B[ixB[i]]> for the handle's
+ * A [dimA x k] and B [dimB x k], bitwise what pmf_b200_predict_multiple gives for the factors pmf_b200_get_factors
+ * reads back (the reference's left-to-right sum over components 0..k-1, no contraction).  Only the ids (index_bytes
+ * each) go up and the n scores (real_t) come down; the ids travel in fixed-size chunks whose
+ * uploads overlap the scoring of the previous chunk.  Waits like pmf_b200_topN_fitted first; synchronous: `out`
+ * is filled on return.  The handle's factors, matrices, plans and profiling counters are left untouched.  Device
+ * memory of the call: n scores plus two chunks of ids.  Returns 0 (also for n == 0); 2, before any byte of `out`
+ * is written, when index_bytes is not 4 or 8 or an id is >= dimA / >= dimB (or a negative 4-byte id); 1 on a CUDA
+ * failure, when the handle holds no factors, or when n scores exceed a quarter of the free device memory. */
+int pmf_b200_predict_fitted(pmf_b200_handle* h, int index_bytes, const void* ixA, const void* ixB, size_t n,
+                            void* out);
 
 /* Replaces topN, src/topN.c:112-284 (prototype src/poismf.h:240-247) for ONE user. */
 int pmf_b200_topN(int dtype, int index_bytes, const void* a_vec, const void* B, int k,

@@ -29,6 +29,7 @@ SYMBOLS = [
     "pmf_b200_topN_batch_include", "pmf_b200_topN_fitted_include",
     "pmf_b200_topN_new_batch", "pmf_b200_topN_new_fitted", "pmf_b200_fit_stats",
     "pmf_b200_release_cache", "pmf_b200_fit_coo", "pmf_b200_coo_to_csr_csc",
+    "pmf_b200_predict_fitted", "pmf_b200_set_coo",
 ]
 
 
@@ -96,6 +97,8 @@ def lib():
     L.pmf_b200_topN_stats.restype = None
     L.pmf_b200_fit_coo.argtypes = [i, i] + [vp] * 5 + [sz, sz, sz, sz, d, d, d, d, i, i, sz, sz, i, i, i]
     L.pmf_b200_coo_to_csr_csc.argtypes = [i, i, vp, vp, vp, sz, sz, sz] + [vp] * 6 + [C.POINTER(C.c_size_t)]
+    L.pmf_b200_predict_fitted.argtypes = [vp, i, vp, vp, sz, vp]
+    L.pmf_b200_set_coo.argtypes = [vp, vp, vp, vp, sz, i]
     L.pmf_b200_release_cache.argtypes = []
     L.pmf_b200_release_cache.restype = C.c_size_t
     _lib = L

@@ -218,6 +218,7 @@ struct pmf_b200_handle {
     virtual int ipc_export(int which, void* out) = 0;
     virtual int ipc_import(int which, const void* handles, int n_ranks, int self_rank) = 0;
     virtual int exchange_status() = 0;
+    virtual bool has_peers() const = 0;        // peer replicas or epoch slots imported: part of a sharded fit
     virtual int get_profile(pmf_b200_bin_profile* out, int max_entries) = 0;
     virtual void clear_profile() = 0;
     bool profiling = false;
@@ -709,6 +710,7 @@ template <class real> struct HandleT : pmf_b200_handle {
         cudaMemcpy(&v, sig_status, sizeof v, cudaMemcpyDeviceToHost);
         return v;
     }
+    bool has_peers() const override { return npeers[0] || npeers[1] || n_sig_opened; }
 
     int ipc_export(int which, void* out) override
     {
@@ -1342,6 +1344,19 @@ extern "C" int pmf_b200_coo_to_csr_csc(int dtype, int index_bytes, const void* r
     pmf_b200_destroy(h);
     return rc;
 }
+// The conversion into a fit handle: both orientations replace the handle's matrix and stay on the device.
+extern "C" int pmf_b200_set_coo(pmf_b200_handle* h, const void* rows, const void* cols, const void* vals,
+                                size_t n_entries, int index_bytes)
+{
+    if (!h) return fail("set_coo: null handle");
+    const char* bad = n_entries == 0 ? "set_coo: no entries"
+                    : n_entries > (size_t)INT32_MAX ? "set_coo: more than 2^31-1 triplets"
+                    : (index_bytes != 4 && index_bytes != 8) ? "set_coo: index_bytes must be 4 or 8"
+                    : h->has_peers() ? "set_coo: the handle is part of a sharded fit (set each rank's shard instead)"
+                    : nullptr;
+    if (bad) { g_err = bad; return 2; }
+    return h->ingest_coo(rows, cols, vals, n_entries, index_bytes);
+}
 
 // ---- factors_single drop-in (src/pred.c:201-304, prototype src/poismf.h:281-289) --------------------
 // One new row by tncg == factors_multiple on a one-row matrix.  The reference passes no row count
@@ -1492,6 +1507,109 @@ extern "C" int pmf_b200_predict_multiple(int dtype, int index_bytes, void* out, 
     return with_types(dtype, index_bytes, "predict_multiple: bad dtype/index width", [&](auto r, auto i) {
         using real = decltype(r); using IX = decltype(i);
         return predict_impl((real*)out, (const real*)A, (const real*)B, (const IX*)ixA, (const IX*)ixB, n, k, dimA, dimB);
+    });
+}
+
+// ---- predict_multiple against the factors resident in a handle ------------------------------------------------
+// Pairs per upload chunk: 8-byte ids travel in 16 MB blocks (4-byte ids in 8 MB), large enough for the threaded
+// staging of pageable arrays (staged_copy.h) and for the launch between chunks to be hidden behind the copies.
+static constexpr size_t PREDICT_CHUNK = (size_t)1 << 21;
+
+// the upload stream of one pipelined call and the events of its two chunk slots, released when the call returns
+// (a stream or event destroyed with work pending is released once that work completes)
+struct UploadRing {
+    cudaStream_t up = nullptr;
+    cudaEvent_t loaded[2] = {}, consumed[2] = {};
+    cudaError_t init()
+    {
+        cudaError_t e = cudaStreamCreateWithFlags(&up, cudaStreamNonBlocking);
+        for (int s = 0; s < 2 && e == cudaSuccess; s++) {
+            e = cudaEventCreateWithFlags(&loaded[s], cudaEventDisableTiming);
+            if (e == cudaSuccess) e = cudaEventCreateWithFlags(&consumed[s], cudaEventDisableTiming);
+        }
+        return e;
+    }
+    ~UploadRing()
+    {
+        for (int s = 0; s < 2; s++) {
+            if (loaded[s]) cudaEventDestroy(loaded[s]);
+            if (consumed[s]) cudaEventDestroy(consumed[s]);
+        }
+        if (up) cudaStreamDestroy(up);
+    }
+};
+
+// Chunk c's ids go up on the ring's stream into slot c % 2 (once chunk c - 2's kernel has read that slot) while chunk
+// c - 1 is scored on `st`.  The scores of every chunk stay on the device until the last kernel has run; they are
+// copied to `out` only if no pair was out of range, so a 2 leaves `out` untouched.
+template <class real, class IX>
+static int predict_fitted_impl(const real* dA, const real* dB, size_t dimA, size_t dimB, int k, int ldf, int num_sms,
+                               cudaStream_t st, const IX* ixA, const IX* ixB, size_t n, real* out)
+{
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    if (n > free_b / 4 / sizeof(real))
+        return fail("predict_fitted: %zu scores exceed a quarter of the free device memory (%zu MB); pass fewer pairs "
+                    "per call", n, free_b >> 20);
+    const size_t chunk = std::min(n, PREDICT_CHUNK);
+    const int nslots = n > chunk ? 2 : 1;
+    DeviceBlocks mem;
+    real* d_out = nullptr;
+    int* d_bad = nullptr;
+    IX* d_ix[2][2] = {};
+    CK(mem.alloc(&d_out, n * sizeof(real)));
+    CK(mem.alloc(&d_bad, sizeof(int)));
+    for (int s = 0; s < nslots; s++)
+        for (int w = 0; w < 2; w++) CK(mem.alloc(&d_ix[s][w], chunk * sizeof(IX)));
+    UploadRing ring;               // a single chunk goes up on `st` itself: no stream or events to create
+    if (nslots > 1) CK(ring.init());
+    cudaStream_t up = nslots > 1 ? ring.up : st;
+    CK(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
+    for (size_t off = 0, c = 0; off < n; off += chunk, c++) {
+        const size_t m = std::min(chunk, n - off);
+        const int s = (int)(c & 1);
+        if (c >= 2) CK(cudaStreamWaitEvent(up, ring.consumed[s], 0));
+        CK(Stager::get().h2d(d_ix[s][0], ixA + off, m * sizeof(IX), up));
+        CK(Stager::get().h2d(d_ix[s][1], ixB + off, m * sizeof(IX), up));
+        if (nslots > 1) {
+            CK(cudaEventRecord(ring.loaded[s], up));
+            CK(cudaStreamWaitEvent(st, ring.loaded[s], 0));
+        }
+        const int grid = (int)std::min<size_t>((m + 255) / 256, (size_t)num_sms * 16);
+        predict_resident_kernel<real, IX><<<grid, 256, 0, st>>>(dA, dB, d_ix[s][0], d_ix[s][1], m, dimA, dimB, k, ldf,
+                                                                d_out + off, d_bad);
+        LAUNCHED();
+        CK(cudaGetLastError());
+        if (nslots > 1) CK(cudaEventRecord(ring.consumed[s], st));
+    }
+    int bad = 0;
+    CK(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (bad) {
+        mem.settled = true;
+        g_err = "predict_fitted: an id is outside [0, dimA) / [0, dimB)";
+        return 2;
+    }
+    CK(Stager::get().d2h(out, d_out, n * sizeof(real), st));
+    CK(cudaStreamSynchronize(st));
+    mem.settled = true;
+    return 0;
+}
+
+extern "C" int pmf_b200_predict_fitted(pmf_b200_handle* h, int index_bytes, const void* ixA, const void* ixB, size_t n,
+                                       void* out)
+{
+    if (!h) return fail("predict_fitted: null handle");
+    if (pmf_b200_sync(h)) return 1;             // every row of the last half-sweep (own and peers') has landed
+    const void* A = h->factor_ptr(0);
+    const void* B = h->factor_ptr(1);
+    if (!A || !B) return fail("predict_fitted: the handle holds no factors");
+    if (index_bytes != 4 && index_bytes != 8) { g_err = "predict_fitted: index_bytes must be 4 or 8"; return 2; }
+    if (n == 0) return 0;
+    return with_types(h->dtype, index_bytes, "predict_fitted: bad dtype", [&](auto r, auto i) {
+        using real = decltype(r); using IX = decltype(i);
+        return predict_fitted_impl<real, IX>((const real*)A, (const real*)B, h->dimA, h->dimB, h->k, h->ldf, h->num_sms,
+                                             h->stream, (const IX*)ixA, (const IX*)ixB, n, (real*)out);
     });
 }
 

@@ -1,7 +1,7 @@
 // poismf_b200 — small streaming kernels around the row solvers:
 // index narrowing on upload, column sums (the "all items" term of the gradient,
 // /root/reference/src/poismf.c:77-83,512-514,562-564), empty-row zeroing
-// (:166-169,:308-311,:367-370) and predict_multiple (src/pred.c:42-64).
+// (:166-169,:308-311,:367-370) and predict_multiple (src/pred.c:42-64), on uploaded or resident factors.
 #pragma once
 #include "common.cuh"
 
@@ -177,6 +177,43 @@ __global__ void predict_pairs_kernel(const real* __restrict__ A, const real* __r
         for (int c = 0; c < k; c++) acc = add_rn(acc, mul_rn(a[c], b[c]));
         out[i] = acc;
     }
+}
+
+// The same sums over the RESIDENT factors of a fit handle, whose rows are ldf reals, 16-byte aligned with zero
+// pads: each row is read as whole 16-byte vectors, and only components 0..k-1 are added (a pad is never summed).
+// ids are range-checked here: a pair with ixA >= dimA or ixB >= dimB (a negative int id converts to a huge size_t)
+// sets *bad and is skipped, its output left unwritten; no out-of-range row is ever read.
+template <class real, class IX>
+__global__ void __launch_bounds__(256) predict_resident_kernel(const real* __restrict__ A, const real* __restrict__ B,
+                                                               const IX* __restrict__ ixA, const IX* __restrict__ ixB,
+                                                               size_t n, size_t dimA, size_t dimB, int k, int ldf,
+                                                               real* __restrict__ out, int* __restrict__ bad)
+{
+    constexpr int V = RealTraits<real>::V;
+    struct alignas(16) Vec { real e[V]; };
+    const int full = k / V, rest = k - full * V;
+    int any = 0;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t a = (size_t)ixA[i], b = (size_t)ixB[i];
+        if (a >= dimA || b >= dimB) { any = 1; continue; }
+        const Vec* pa = reinterpret_cast<const Vec*>(A + a * ldf);
+        const Vec* pb = reinterpret_cast<const Vec*>(B + b * ldf);
+        real acc = 0;
+#pragma unroll 4
+        for (int t = 0; t < full; t++) {
+            const Vec x = pa[t], y = pb[t];
+#pragma unroll
+            for (int j = 0; j < V; j++) acc = add_rn(acc, mul_rn(x.e[j], y.e[j]));
+        }
+        if (rest) {
+            const Vec x = pa[full], y = pb[full];
+#pragma unroll
+            for (int j = 0; j < V; j++)
+                if (j < rest) acc = add_rn(acc, mul_rn(x.e[j], y.e[j]));
+        }
+        out[i] = acc;
+    }
+    if (any) atomicOr(bad, 1);
 }
 
 // scores[u, j] = <A[user[u]], B[j]> (same left-to-right sum); excluded items get -inf later.

@@ -46,6 +46,45 @@ class DeviceFit:
         self.set_matrix(_lib.SIDE_CSR, *csr)
         self.set_matrix(_lib.SIDE_CSC, *csc)
 
+    def set_coo(self, rows, cols, vals):
+        """Both orientations of the matrix from COO triplets, built on the device (pmf_b200_set_coo): duplicates
+        are summed, as coo.tocsr() / coo.tocsc() do; the factors are untouched.  ValueError on empty triplets or an
+        id outside the handle's dimensions (the handle then holds no matrix) or on a handle of a sharded fit."""
+        rows, cols, vals = (np.ascontiguousarray(a) for a in (rows, cols, vals))
+        if rows.dtype != cols.dtype:
+            raise ValueError("set_coo: rows and cols must share one index dtype")
+        if vals.dtype != self.dtype:
+            raise TypeError(f"set_coo: vals must be {self.dtype}, got {vals.dtype}")
+        if not rows.ndim == cols.ndim == vals.ndim == 1 or not rows.shape[0] == cols.shape[0] == vals.shape[0]:
+            raise ValueError("set_coo: rows, cols and vals must be 1-D arrays of one length")
+        rc = self.L.pmf_b200_set_coo(self.h, _lib.ptr(rows), _lib.ptr(cols), _lib.ptr(vals), vals.shape[0],
+                                     _lib.index_bytes(rows))
+        if rc == 2:
+            raise ValueError(_lib.last_error())
+        self._ck(rc)
+
+    def predict(self, users, items, out=None):
+        """Scores <A[users[i]], B[items[i]]> of (user, item) pairs against the factors resident in this handle
+        (pmf_b200_predict_fitted: only the ids and the scores cross PCIe).  Bitwise c_funs._predict_multiple on
+        get_factors().  `users` and `items` share one index dtype (int32, int64 or uint64); `out`, when given, is a
+        C-contiguous array of the handle's dtype and length.  ValueError on an id out of range (`out` untouched)."""
+        users, items = np.ascontiguousarray(users), np.ascontiguousarray(items)
+        if users.ndim != 1 or users.shape != items.shape:
+            raise ValueError("predict: users and items must be 1-D arrays of one length")
+        if users.dtype != items.dtype:
+            raise ValueError("predict: users and items must share one index dtype")
+        ib = _lib.index_bytes(users)
+        n = users.shape[0]
+        if out is None:
+            out = np.empty(n, self.dtype)
+        elif out.dtype != self.dtype or out.shape != (n,) or not out.flags.c_contiguous:
+            raise ValueError(f"predict: out must be a C-contiguous {self.dtype} array of length {n}")
+        rc = self.L.pmf_b200_predict_fitted(self.h, ib, _lib.ptr(users), _lib.ptr(items), n, _lib.ptr(out))
+        if rc == 2:
+            raise ValueError(_lib.last_error())
+        self._ck(rc)
+        return out
+
     def set_factors(self, A=None, B=None):
         for M in (A, B):
             assert M is None or (M.dtype == self.dtype and M.flags.c_contiguous)

@@ -292,6 +292,13 @@ class GpuBackend:
         return new_users_sharded((Xr, Xr_indptr, Xr_indices), fold, self.rank, self.world, self.group, excl_ptr,
                                  excl_ix, incl_ptr, incl_ix, gather)
 
+    def predict(self, users, items, gather=True):
+        """DeviceFit.predict with the pairs split across the ranks (predict_sharded): every rank scores its
+        contiguous range of pairs against ITS replicas and the scores are all-gathered; with gather=False a rank
+        returns its own range, user_ranges(n, world)[rank].  An id out of range anywhere raises ValueError on every
+        rank."""
+        return predict_sharded(users, items, self.fit.predict, self.rank, self.world, self.group, gather)
+
     def transform(self, Xr_indptr, Xr_indices, Xr, gather=True, **kw):
         """DeviceFit.transform with the new users split across the ranks; returns their factors."""
         return new_users_sharded((Xr, Xr_indptr, Xr_indices),
@@ -333,6 +340,36 @@ def new_users_sharded(csr, fold, rank=0, world=1, group=None, excl_ptr=None, exc
     parts = [None] * world
     dist.all_gather_object(parts, out, group=group)
     return tuple(np.concatenate([p[j] for p in parts], axis=0) for j in range(len(out)))
+
+
+def predict_sharded(users, items, predictor, rank=0, world=1, group=None, gather=True):
+    """Scores of (users[i], items[i]) pairs split across ranks that all hold full replicas of the factors: rank r
+    scores the contiguous range user_ranges(n, world)[r] with `predictor(users_slice, items_slice) -> scores`
+    (GpuBackend.predict passes the resident handle's; the CPU tests inject a stand-in), and the scores are
+    all-gathered in pair order; with gather=False a rank returns its own range only.  Every rank joins one
+    all-gather of its status (and, with gather=True, its scores) whether or not its range failed, so an error on
+    any rank (ValueError for an id out of range) is raised on every rank and none is left waiting."""
+    users, items = np.asarray(users), np.asarray(items)
+    if users.ndim != 1 or users.shape != items.shape:
+        raise ValueError("predict: users and items must be 1-D arrays of one length")
+    lo, hi = user_ranges(users.shape[0], world)[rank]
+    err, mine = None, None
+    try:
+        mine = predictor(np.ascontiguousarray(users[lo:hi]), np.ascontiguousarray(items[lo:hi]))
+    except Exception as e:      # raised below, on every rank
+        if world == 1:
+            raise
+        err = e
+    if world == 1:
+        return mine
+    import torch.distributed as dist
+    parts = [None] * world
+    dist.all_gather_object(parts, (err, mine if gather and err is None else None), group=group)
+    for r, (e, _) in enumerate(parts):
+        if e is not None:
+            kind = type(e) if type(e) in (ValueError, TypeError, MemoryError) else RuntimeError
+            raise kind(f"predict on rank {r}: {e}")
+    return np.concatenate([p[1] for p in parts]) if gather else mine
 
 
 def topn_sharded(A, B, top_n, users=None, excl_ptr=None, excl_ix=None, output_score=False, rank=0, world=1,
